@@ -73,7 +73,29 @@ def parse():
                     help="seconds after which the line is printed without the unfinished part of `secondary`")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: --nt samples per GPU (default, the contract); strong: --nt samples in total")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (the PCG iterate x) as "
+                         "DIR/<name>.npy in float64, so that two builds can be compared on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every array as ``out_dir/<name>.npy`` in float64."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    # x has 3 entries per observed pixel of the fixed 1000 x 500 patch: at most 12 MB
+    assert total <= DUMP_LIMIT_BYTES, "outputs of %d bytes exceed the %d-byte dump limit" % (total, DUMP_LIMIT_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -384,6 +406,12 @@ def main():
     value = world * nt * args.steps / (ms * 1e-3)
     t_a_ms = float(np.mean([e0.elapsed_time(e1) for e0, e1 in a_events]))
     assert bool(torch.isfinite(solver.x).all().item()), "PCG state is not finite"
+    x_last = None
+    if args.dump_outputs:
+        # the last timed step's iterate, copied on the device now (the steps below overwrite the solver state) and
+        # written to disk once the headline measurements are done.  ||r|| after the step is not dumped: M_BD A = I makes it
+        # rounding noise that differs from run to run.
+        x_last = solver.gather_x() if sharded else solver.x.clone()
 
     # keep the GPU under the same load for ~1.5 s so that nvidia-smi sees the clocks of this loop.  Every
     # rank runs the SAME number of extra steps (each one contains a peer exchange: a per-rank wall-clock
@@ -503,6 +531,8 @@ def main():
                 "host_cores_available": os.cpu_count()}
     else:
         line = None
+    if x_last is not None and rank == 0:
+        dump_outputs(args.dump_outputs, {"x": dv.to_host(x_last)})
     failed_primary = world > 1 and ((sharded and solver.failed()) or (getattr(A, "_p2p", None) is not None and A._p2p.error() != 0))
     if not args.no_secondary and not failed_primary:
         # the other configurations, on the same GPUs, after the headline measurement.  A watchdog prints the line
