@@ -92,6 +92,8 @@ SIGNATURES = {
     "cm2_enable_peer_access": (_int, [_int]),
     "cm2_allreduce_p2p_set_timeout": (_f64, [_f64]),
     "cm2_pcg_bd_iter_refuse": (_int, [_int]),
+    "cm2_pcg_bd_iter_max_npix": (_i64, [_int]),
+    "cm2_pcg_bd_tail_strided": (_int, [_int]),
     "cm2_pcg_sharded_signal_bytes": (_i64, []),
     "cm2_pcg_sharded_work_doubles": (_i64, []),
     "cm2_pcg_bd_sharded": (_int, [_int, _int, _int, _int, _int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
@@ -103,7 +105,8 @@ _NOT_STATUS = {"cm2_version", "cm2_last_error", "cm2_launch_count", "cm2_scan_sc
                "cm2_toeplitz_scratch_bytes", "cm2_defl_work_doubles", "cm2_allreduce_p2p_signal_bytes",
                "cm2_toeplitz_fft_points", "cm2_toeplitz_fft_scratch_bytes", "cm2_filter_poly_max_order", "cm2_filter_poly_set_tma",
                "cm2_amatvec_filter_poly_max_order", "cm2_amatvec_toeplitz_max_band",
-               "cm2_allreduce_p2p_set_timeout", "cm2_pcg_bd_iter_refuse",
+               "cm2_allreduce_p2p_set_timeout", "cm2_pcg_bd_iter_refuse", "cm2_pcg_bd_iter_max_npix",
+               "cm2_pcg_bd_tail_strided",
                "cm2_pcg_sharded_signal_bytes", "cm2_pcg_sharded_work_doubles", "cm2_dense_gram_work_doubles"}
 
 

@@ -303,7 +303,11 @@ int cm2_pcg_update_xr(const double *p, const double *q, double *x, double *r, in
  *   bd_update  : pq ; alpha ; x += alpha p ; r -= alpha q ; z = M r ; rho' ; beta' ; |r|^2 ; flags
  *   bd_iter    : bd_update followed by the NEXT iteration's p = z + beta' p, all in ONE cooperative
  *                launch (two grid barriers); with it an iteration is  q = A p ; bd_iter.  bd_reset's
- *                p0, when non-NULL, receives the first search direction p = z. */
+ *                p0, when non-NULL, receives the first search direction p = z.
+ * z is scratch of the M_BD path: bd_iter, and bd_reset with b, x and p0 all non-NULL, keep it on chip
+ * and may leave the buffer unwritten; bd_update writes it for bd_update_p.  bd_iter holds its
+ * pixels' p on chip between its grid barriers up to cm2_pcg_bd_iter_max_npix(pol) pixels and runs a
+ * one-thread-per-pixel kernel above that, or when p, q, x or r is not 16-byte aligned. */
 int cm2_pcg_bd_reset(const double *bd_inv, int64_t npix, int pol, double *r, double *z,
                      double *scal, double atol, double rtol, const double *b, double *x, double *p0,
                      cm2_stream_t stream);
@@ -316,6 +320,11 @@ int cm2_pcg_bd_iter(const double *bd_inv, int64_t npix, int pol, double *p, cons
 /* test hook: on != 0 makes cm2_pcg_bd_iter ask for more CTAs than can be co-resident, so that the
  * cooperative launch is refused like on a GPU that does not grant them; returns the previous value */
 int cm2_pcg_bd_iter_refuse(int on);
+/* the largest npix for which cm2_pcg_bd_iter runs its on-chip (tiled) kernel on the current device */
+int64_t cm2_pcg_bd_iter_max_npix(int pol);
+/* development/test hook: on != 0 makes cm2_pcg_bd_reset and cm2_pcg_bd_iter run the
+ * one-thread-per-pixel kernels at every npix (the large-npix path); returns the previous value */
+int cm2_pcg_bd_tail_strided(int on);
 
 /* ---- (f) next rows: the other time-domain filters and the map output step ----------------------
  * Subscan filter of polynomial order 0..cm2_filter_poly_max_order(), one CTA per subscan with the
