@@ -16,6 +16,7 @@
 // warp with a segmented shuffle scan, (3) one fp64 RED per (run, Stokes component) goes to L2.
 // Random pointing degenerates gracefully to one RED per sample and component.
 #include <cstdint>
+#include <type_traits>
 
 #include "cm2_common.cuh"
 
@@ -53,8 +54,6 @@ __device__ __forceinline__ int64_t block_of(const BlockW &bw, int64_t t) {
     }
     return lo;
 }
-
-__device__ __forceinline__ void load_f64(const double *__restrict__ a, int64_t t0, int64_t nt, double (&c)[K]);
 
 // weights of the K samples starting at t0 (one lookup when the chunk sits inside one block)
 __device__ __forceinline__ void chunk_weights(const BlockW &bw, int64_t t0, int64_t nt, double (&w)[K]) {
@@ -116,27 +115,42 @@ static TileOrder make_order(int64_t nt, int64_t nstreams) {
     return o;
 }
 
+// Cache policy of the TOD loads.  STREAM: L2 evict-first, for data read once.  KEEP: default L2 priority, for the
+// per-subscan kernels whose CTA reads the same samples again in a second pass.
+enum Cache { STREAM, KEEP };
+
+template <Cache CP = STREAM>
 __device__ __forceinline__ void load_pix(const int32_t *__restrict__ pix, int64_t t0, int64_t nt, int (&p)[K]) {
     if (t0 + K <= nt) {
-        I8 v = ld_stream_i8(pix + t0);
+        I8 v = CP == KEEP ? ld_keep_i8(pix + t0) : ld_stream_i8(pix + t0);
 #pragma unroll
         for (int j = 0; j < K; ++j) p[j] = v.v[j];
     } else {
 #pragma unroll
-        for (int j = 0; j < K; ++j) p[j] = (t0 + j < nt) ? ld_stream_i1(pix + t0 + j) : -1;
+        for (int j = 0; j < K; ++j) p[j] = (t0 + j < nt) ? (CP == KEEP ? pix[t0 + j] : ld_stream_i1(pix + t0 + j)) : -1;
     }
 }
 
+template <Cache CP = STREAM>
 __device__ __forceinline__ void load_f64(const double *__restrict__ a, int64_t t0, int64_t nt, double (&c)[K]) {
     if (t0 + K <= nt) {
-        D4 v0 = ld_stream_d4(a + t0);
-        D4 v1 = ld_stream_d4(a + t0 + 4);
+        D4 v0 = CP == KEEP ? ld_keep_d4(a + t0) : ld_stream_d4(a + t0);
+        D4 v1 = CP == KEEP ? ld_keep_d4(a + t0 + 4) : ld_stream_d4(a + t0 + 4);
 #pragma unroll
         for (int j = 0; j < 4; ++j) { c[j] = v0.v[j]; c[4 + j] = v1.v[j]; }
     } else {
 #pragma unroll
-        for (int j = 0; j < K; ++j) c[j] = (t0 + j < nt) ? ld_stream_d1(a + t0 + j) : 0.0;
+        for (int j = 0; j < K; ++j) c[j] = (t0 + j < nt) ? (CP == KEEP ? a[t0 + j] : ld_stream_d1(a + t0 + j)) : 0.0;
     }
+}
+
+// pixels and, for POL > 1, cos / sin of the K samples starting at t0
+template <int POL, Cache CP = STREAM>
+__device__ __forceinline__ void load_tod(const int32_t *__restrict__ pix, const double *__restrict__ cs,
+                                         const double *__restrict__ sn, int64_t t0, int64_t nt, int (&p)[K],
+                                         double (&c)[K], double (&s)[K]) {
+    load_pix<CP>(pix, t0, nt, p);
+    if (POL > 1) { load_f64<CP>(cs, t0, nt, c); load_f64<CP>(sn, t0, nt, s); }
 }
 
 // x values of the K samples; one gather per run start, copied along the run
@@ -169,6 +183,22 @@ __device__ __forceinline__ double project(const double (&xv)[POL], double c, dou
     else return fma(xv[2], s, fma(xv[1], c, xv[0]));
 }
 
+// (P x) of sample j of the chunk (c, s are not read for POL = 1)
+template <int POL>
+__device__ __forceinline__ double project(const double (&xv)[K][POL], const double (&c)[K], const double (&s)[K], int j) {
+    return project<POL>(xv[j], POL > 1 ? c[j] : 0.0, POL > 1 ? s[j] : 0.0);
+}
+
+// P^T contribution of sample j of the chunk with TOD value v[j]: the contrib functor of run_compress / run_scatter
+template <int POL>
+__device__ __forceinline__ auto pt_contrib(const double (&v)[K], const double (&c)[K], const double (&s)[K]) {
+    return [&v, &c, &s](int j, double (&o)[POL]) {
+        if constexpr (POL == 1) { o[0] = v[j]; }
+        else if constexpr (POL == 2) { o[0] = v[j] * c[j]; o[1] = v[j] * s[j]; }
+        else { o[0] = v[j]; o[1] = v[j] * c[j]; o[2] = v[j] * s[j]; }
+    };
+}
+
 template <int NV, int STRIDE>
 __device__ __forceinline__ void emit(double *__restrict__ y, int pix, const double (&v)[NV]) {
     if (pix >= 0) {
@@ -190,6 +220,16 @@ struct RunState {
     double head[NV];   // partial of the lane's first run (when the lane holds more than one run)
     int ph, pt;        // pixel of the first / last run
     bool single;
+
+    // the state before the first tile: run_merge emits nothing for it
+    __device__ __forceinline__ static RunState empty() {
+        RunState rs;
+        rs.ph = rs.pt = -1;
+        rs.single = true;
+#pragma unroll
+        for (int k = 0; k < NV; ++k) rs.acc[k] = rs.head[k] = 0.0;
+        return rs;
+    }
 };
 
 template <int NV, int STRIDE, class F>
@@ -283,11 +323,10 @@ __global__ void __launch_bounds__(BLOCK) k_pointing_apply(const int32_t *__restr
         if (t0 >= nt) continue;
         int p[K];
         double c[K], s[K], xv[K][POL], out[K];
-        load_pix(pix, t0, nt, p);
-        if (POL > 1) { load_f64(cs, t0, nt, c); load_f64(sn, t0, nt, s); }
+        load_tod<POL>(pix, cs, sn, t0, nt, p, c, s);
         gather_x<POL>(x, p, xv);
 #pragma unroll
-        for (int j = 0; j < K; ++j) out[j] = p[j] >= 0 ? project<POL>(xv[j], POL > 1 ? c[j] : 0.0, POL > 1 ? s[j] : 0.0) : 0.0;
+        for (int j = 0; j < K; ++j) out[j] = p[j] >= 0 ? project<POL>(xv, c, s, j) : 0.0;
         if (t0 + K <= nt) {
             D4 a, b;
 #pragma unroll
@@ -315,11 +354,7 @@ __global__ void __launch_bounds__(BLOCK) k_pointing_apply_t(const int32_t *__res
         load_pix(pix, t0, nt, p);
         load_f64(d, t0, nt, v);
         if (POL > 1) { load_f64(cs, t0, nt, c); load_f64(sn, t0, nt, s); }
-        run_scatter<POL, POL>(y, p, [&](int j, double (&o)[POL]) {
-            if constexpr (POL == 1) { o[0] = v[j]; }
-            else if constexpr (POL == 2) { o[0] = v[j] * c[j]; o[1] = v[j] * s[j]; }
-            else { o[0] = v[j]; o[1] = v[j] * c[j]; o[2] = v[j] * s[j]; }
-        });
+        run_scatter<POL, POL>(y, p, pt_contrib<POL>(v, c, s));
     }
 }
 
@@ -338,11 +373,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_white(const int32_t *__restri
     // (the loop-carried state is rs, 15 registers, not the 40 registers of p/c/s: the first version
     // carried p/c/s across the back edge and spent 79 register moves per tile on it).
     // ILV = false: time order (the instantiation measured on configs[1]); true: detector-interleaved (TileOrder).
-    RunState<POL> rs;
-    rs.ph = rs.pt = -1;
-    rs.single = true;
-#pragma unroll
-    for (int k = 0; k < POL; ++k) rs.acc[k] = rs.head[k] = 0.0;
+    RunState<POL> rs = RunState<POL>::empty();
     const int64_t nv = ILV ? ord.count() : ntiles;
     for (int64_t vt = (int64_t)blockIdx.x * (BLOCK / 32) + (threadIdx.x >> 5); vt < nv; vt += nwarps) {
         int64_t tile = vt;
@@ -353,20 +384,15 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_white(const int32_t *__restri
         const int64_t t0 = tile * TILE + (int64_t)lane * K;
         int p[K];
         double c[K], s[K];
-        load_pix(pix, t0, nt, p);
-        if (POL > 1) { load_f64(cs, t0, nt, c); load_f64(sn, t0, nt, s); }
+        load_tod<POL>(pix, cs, sn, t0, nt, p, c, s);
         run_merge<POL, POL>(y, rs);             // previous tile (the empty state on the first trip emits nothing)
         double w[K], xv[K][POL], v[K];
         if constexpr (WS) load_f64(bw.w, t0, nt, w);
         gather_x<POL>(x, p, xv);
         if constexpr (!WS) chunk_weights(bw, t0 < nt ? t0 : nt - 1, nt, w);
 #pragma unroll
-        for (int j = 0; j < K; ++j) v[j] = w[j] * project<POL>(xv[j], POL > 1 ? c[j] : 0.0, POL > 1 ? s[j] : 0.0);
-        run_compress<POL, POL>(y, p, [&](int j, double (&o)[POL]) {
-            if constexpr (POL == 1) { o[0] = v[j]; }
-            else if constexpr (POL == 2) { o[0] = v[j] * c[j]; o[1] = v[j] * s[j]; }
-            else { o[0] = v[j]; o[1] = v[j] * c[j]; o[2] = v[j] * s[j]; }
-        }, rs);
+        for (int j = 0; j < K; ++j) v[j] = w[j] * project<POL>(xv, c, s, j);
+        run_compress<POL, POL>(y, p, pt_contrib<POL>(v, c, s), rs);
     }
     run_merge<POL, POL>(y, rs);
 }
@@ -413,15 +439,14 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_white_staged(const int32_t *_
         const int64_t t0 = tile * TILE + (int64_t)lane * K;
         int p[K];
         double c[K], s[K];
-        load_pix(pix, t0, nt, p);
-        if (POL > 1) { load_f64(cs, t0, nt, c); load_f64(sn, t0, nt, s); }
+        load_tod<POL>(pix, cs, sn, t0, nt, p, c, s);
         if (len_prev) stage_flush<POL>(sm, y, base_prev, len_prev);   // previous tile, after this tile's loads were issued
         len_prev = 0;
         double w[K], xv[K][POL], v[K];
         gather_x<POL>(x, p, xv);
         chunk_weights(bw, t0 < nt ? t0 : nt - 1, nt, w);
 #pragma unroll
-        for (int j = 0; j < K; ++j) v[j] = w[j] * project<POL>(xv[j], POL > 1 ? c[j] : 0.0, POL > 1 ? s[j] : 0.0);
+        for (int j = 0; j < K; ++j) v[j] = w[j] * project<POL>(xv, c, s, j);
         int lo = INT32_MAX, hi = INT32_MIN;
 #pragma unroll
         for (int j = 0; j < K; ++j) {
@@ -430,11 +455,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_white_staged(const int32_t *_
         lo = __reduce_min_sync(FULL, lo);
         hi = __reduce_max_sync(FULL, hi);
         if (hi < lo) continue;                                    // every sample of the tile is flagged
-        auto contrib = [&](int j, double (&o)[POL]) {
-            if constexpr (POL == 1) { o[0] = v[j]; }
-            else if constexpr (POL == 2) { o[0] = v[j] * c[j]; o[1] = v[j] * s[j]; }
-            else { o[0] = v[j]; o[1] = v[j] * c[j]; o[2] = v[j] * s[j]; }
-        };
+        auto contrib = pt_contrib<POL>(v, c, s);
         if ((int64_t)hi - lo < wpix) {                            // warp-uniform
             double acc[POL];
             int cur = p[0];
@@ -499,18 +520,13 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_toeplitz(const int32_t *__res
     const int lane = threadIdx.x & 31;
     const int64_t nwarps = (int64_t)gridDim.x * (BLOCK / 32);
     const int64_t ntiles = (nt + VAL - 1) / VAL;
-    RunState<POL> rs;
-    rs.ph = rs.pt = -1;
-    rs.single = true;
-#pragma unroll
-    for (int k = 0; k < POL; ++k) rs.acc[k] = rs.head[k] = 0.0;
+    RunState<POL> rs = RunState<POL>::empty();
     for (int64_t tile = (int64_t)blockIdx.x * (BLOCK / 32) + (threadIdx.x >> 5); tile < ntiles; tile += nwarps) {
         const int64_t t0 = tile * VAL - HL * K + (int64_t)lane * K;   // multiple of 8: the 256-bit loads stay aligned
         int p[K];
         double c[K], s[K];
         if (t0 >= 0) {
-            load_pix(pix, t0, nt, p);
-            if (POL > 1) { load_f64(cs, t0, nt, c); load_f64(sn, t0, nt, s); }
+            load_tod<POL>(pix, cs, sn, t0, nt, p, c, s);
         } else {
 #pragma unroll
             for (int j = 0; j < K; ++j) { p[j] = -1; c[j] = 0.0; s[j] = 0.0; }
@@ -521,7 +537,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_toeplitz(const int32_t *__res
             double xv[K][POL];
             gather_x<POL>(x, p, xv);
 #pragma unroll
-            for (int j = 0; j < K; ++j) v[j] = p[j] >= 0 ? project<POL>(xv[j], POL > 1 ? c[j] : 0.0, POL > 1 ? s[j] : 0.0) : 0.0;
+            for (int j = 0; j < K; ++j) v[j] = p[j] >= 0 ? project<POL>(xv, c, s, j) : 0.0;
         }
 #pragma unroll
         for (int j = 0; j < K; ++j) sv[32 * j + lane] = v[j];
@@ -583,11 +599,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_toeplitz(const int32_t *__res
             for (int j = 0; j < K; ++j) { out[j] = 0.0; p[j] = -1; }
         }
         __syncwarp();                          // all reads of sv done before the next tile overwrites it
-        run_compress<POL, POL>(y, p, [&](int j, double (&o)[POL]) {
-            if constexpr (POL == 1) { o[0] = out[j]; }
-            else if constexpr (POL == 2) { o[0] = out[j] * c[j]; o[1] = out[j] * s[j]; }
-            else { o[0] = out[j]; o[1] = out[j] * c[j]; o[2] = out[j] * s[j]; }
-        }, rs);
+        run_compress<POL, POL>(y, p, pt_contrib<POL>(out, c, s), rs);
     }
     run_merge<POL, POL>(y, rs);
 }
@@ -624,8 +636,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_mu(const int32_t *__re
     double m0;
     {
         const int64_t t0 = tile * TILE + (int64_t)lane * K;
-        load_pix(pix, t0, nt, p);
-        if (POL > 1) { load_f64(cs, t0, nt, c); load_f64(sn, t0, nt, s); }
+        load_tod<POL>(pix, cs, sn, t0, nt, p, c, s);
         flag = __ldg(sg.tile_flag + tile);
         k0 = __ldg(sg.tile_seg + tile);
         if (tile2 >= 0) { flag2 = __ldg(sg.tile_flag + tile2); k02 = __ldg(sg.tile_seg + tile2); }
@@ -671,19 +682,14 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_mu(const int32_t *__re
             double xv[K][POL], vv[K];
             gather_x<POL>(x, p, xv);
 #pragma unroll
-            for (int j = 0; j < K; ++j) vv[j] = project<POL>(xv[j], POL > 1 ? c[j] : 0.0, POL > 1 ? s[j] : 0.0) - mu[j];
-            run_compress<POL, POL>(y, p, [&](int j, double (&o)[POL]) {
-                if constexpr (POL == 1) { o[0] = vv[j]; }
-                else if constexpr (POL == 2) { o[0] = vv[j] * c[j]; o[1] = vv[j] * s[j]; }
-                else { o[0] = vv[j]; o[1] = vv[j] * c[j]; o[2] = vv[j] * s[j]; }
-            }, rs);
+            for (int j = 0; j < K; ++j) vv[j] = project<POL>(xv, c, s, j) - mu[j];
+            run_compress<POL, POL>(y, p, pt_contrib<POL>(vv, c, s), rs);
         }
         int64_t tile3 = -1, v3 = v2;
         int flag3 = 0, k03 = 0;
         if (tile2 >= 0) {     // warp-uniform: the next tile's TOD loads and mean, the lookup of the tile after it
             const int64_t t1 = tile2 * TILE + (int64_t)lane * K;
-            load_pix(pix, t1, nt, p);
-            if (POL > 1) { load_f64(cs, t1, nt, c); load_f64(sn, t1, nt, s); }
+            load_tod<POL>(pix, cs, sn, t1, nt, p, c, s);
             m0 = flag2 == 1 ? __ldg(sg.mu + k02) : 0.0;
             v3 = ord.next(v2 + nwarps, nwarps, ntiles, tile3);
             if (tile3 >= 0) { flag3 = __ldg(sg.tile_flag + tile3); k03 = __ldg(sg.tile_seg + tile3); }
@@ -722,11 +728,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_poly_mu(const int32_t 
     const int lane = threadIdx.x & 31;
     const int64_t nwarps = (int64_t)gridDim.x * (BLOCK / 32);
     const int64_t ntiles = (nt + TILE - 1) / TILE;
-    RunState<POL> rs;
-    rs.ph = rs.pt = -1;
-    rs.single = true;
-#pragma unroll
-    for (int k = 0; k < POL; ++k) rs.acc[k] = rs.head[k] = 0.0;
+    RunState<POL> rs = RunState<POL>::empty();
     const int64_t nv = ord.count();
     for (int64_t vt = (int64_t)blockIdx.x * (BLOCK / 32) + (threadIdx.x >> 5); vt < nv; vt += nwarps) {
         const int64_t tile = ord.tile(vt);
@@ -734,8 +736,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_poly_mu(const int32_t 
         const int64_t t0 = tile * TILE + (int64_t)lane * K;
         int p[K];
         double c[K], s[K];
-        load_pix(pix, t0, nt, p);
-        if (POL > 1) { load_f64(cs, t0, nt, c); load_f64(sn, t0, nt, s); }
+        load_tod<POL>(pix, cs, sn, t0, nt, p, c, s);
         const int flag = __ldg(sg.tile_flag + tile);
         const int k0 = __ldg(sg.tile_seg + tile);
         run_merge<POL, POL>(y, rs);            // previous tile, after this tile's loads have been issued
@@ -782,12 +783,8 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_poly_mu(const int32_t 
         double xv[K][POL], v[K];
         gather_x<POL>(x, p, xv);
 #pragma unroll
-        for (int j = 0; j < K; ++j) v[j] = project<POL>(xv[j], POL > 1 ? c[j] : 0.0, POL > 1 ? s[j] : 0.0) - pv[j];
-        run_compress<POL, POL>(y, p, [&](int j, double (&o)[POL]) {
-            if constexpr (POL == 1) { o[0] = v[j]; }
-            else if constexpr (POL == 2) { o[0] = v[j] * c[j]; o[1] = v[j] * s[j]; }
-            else { o[0] = v[j]; o[1] = v[j] * c[j]; o[2] = v[j] * s[j]; }
-        }, rs);
+        for (int j = 0; j < K; ++j) v[j] = project<POL>(xv, c, s, j) - pv[j];
+        run_compress<POL, POL>(y, p, pt_contrib<POL>(v, c, s), rs);
     }
     run_merge<POL, POL>(y, rs);
 }
@@ -821,8 +818,7 @@ __global__ void __launch_bounds__(BLOCK) k_pointing_filter_mu(const int32_t *__r
             int p[K];
             double c[K], s[K], mu[K], xv[K][POL], out[K];
             bool in[K];
-            load_pix(pix, t0, nt, p);
-            if (POL > 1) { load_f64(cs, t0, nt, c); load_f64(sn, t0, nt, s); }
+            load_tod<POL>(pix, cs, sn, t0, nt, p, c, s);
             if (flag == 1) {
 #pragma unroll
                 for (int j = 0; j < K; ++j) { mu[j] = m0; in[j] = true; }
@@ -851,8 +847,7 @@ __global__ void __launch_bounds__(BLOCK) k_pointing_filter_mu(const int32_t *__r
             for (int j = 0; j < K; ++j) if (!in[j]) p[j] = -1;
             gather_x<POL>(x, p, xv);
 #pragma unroll
-            for (int j = 0; j < K; ++j)
-                out[j] = in[j] ? (p[j] >= 0 ? project<POL>(xv[j], POL > 1 ? c[j] : 0.0, POL > 1 ? s[j] : 0.0) : 0.0) - mu[j] : 0.0;
+            for (int j = 0; j < K; ++j) out[j] = in[j] ? (p[j] >= 0 ? project<POL>(xv, c, s, j) : 0.0) - mu[j] : 0.0;
             if (t0 + K <= nt) {
                 D4 a, b;
 #pragma unroll
@@ -882,8 +877,7 @@ __global__ void __launch_bounds__(BLOCK) k_moments(const int32_t *__restrict__ p
         const int64_t t0 = tile * TILE + (int64_t)lane * K;
         int p[K];
         double c[K], s[K], w[K];
-        load_pix(pix, t0, nt, p);
-        if (POL > 1) { load_f64(cs, t0, nt, c); load_f64(sn, t0, nt, s); }
+        load_tod<POL>(pix, cs, sn, t0, nt, p, c, s);
         if (wsamp) load_f64(wsamp, t0, nt, w);
         else chunk_weights(bw, t0 < nt ? t0 : nt - 1, nt, w);
         double *base = mom + (POL == 2 ? 3 : 0);
@@ -934,28 +928,6 @@ __global__ void __launch_bounds__(BLOCK) k_hits(const int32_t *__restrict__ pix,
 // aligned; samples of a tile outside [a, b) are treated as flagged.
 constexpr int SEG_SMEM = 12288;  // d_t values kept on chip per segment (96 kB dynamic smem, 2 CTAs/SM); longer -> recompute
 
-__device__ __forceinline__ void load_pix_keep(const int32_t *__restrict__ pix, int64_t t0, int64_t nt, int (&p)[K]) {
-    if (t0 + K <= nt) {
-        I8 v = ld_keep_i8(pix + t0);
-#pragma unroll
-        for (int j = 0; j < K; ++j) p[j] = v.v[j];
-    } else {
-#pragma unroll
-        for (int j = 0; j < K; ++j) p[j] = (t0 + j < nt) ? pix[t0 + j] : -1;
-    }
-}
-__device__ __forceinline__ void load_f64_keep(const double *__restrict__ a, int64_t t0, int64_t nt, double (&c)[K]) {
-    if (t0 + K <= nt) {
-        D4 v0 = ld_keep_d4(a + t0);
-        D4 v1 = ld_keep_d4(a + t0 + 4);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { c[j] = v0.v[j]; c[4 + j] = v1.v[j]; }
-    } else {
-#pragma unroll
-        for (int j = 0; j < K; ++j) c[j] = (t0 + j < nt) ? a[t0 + j] : 0.0;
-    }
-}
-
 template <int POL>
 __global__ void __launch_bounds__(BLOCK) k_amatvec_filter(const int32_t *__restrict__ pix, const double *__restrict__ cs,
                                                           const double *__restrict__ sn, int64_t nt,
@@ -978,14 +950,14 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter(const int32_t *__restr
             const int tb = (int)(tile * TILE - base);   // bank-conflict-free tile layout: (lane, j) at tb + 32 j + lane
             int p[K];
             double c[K], s[K], xv[K][POL];
-            load_pix_keep(pix, t0, nt, p);
+            load_pix<KEEP>(pix, t0, nt, p);
 #pragma unroll
             for (int j = 0; j < K; ++j) if (t0 + j < a || t0 + j >= b) p[j] = -1;
-            if (POL > 1) { load_f64_keep(cs, t0, nt, c); load_f64_keep(sn, t0, nt, s); }
+            if (POL > 1) { load_f64<KEEP>(cs, t0, nt, c); load_f64<KEEP>(sn, t0, nt, s); }
             gather_x<POL>(x, p, xv);
 #pragma unroll
             for (int j = 0; j < K; ++j) {
-                const double dv = p[j] >= 0 ? project<POL>(xv[j], POL > 1 ? c[j] : 0.0, POL > 1 ? s[j] : 0.0) : 0.0;
+                const double dv = p[j] >= 0 ? project<POL>(xv, c, s, j) : 0.0;
                 if (p[j] >= 0) { sum += dv; cnt += 1.0; }
                 if (fits) sd[tb + j * 32 + lane] = dv;
             }
@@ -1015,14 +987,9 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter(const int32_t *__restr
                     double xv[K][POL];
                     gather_x<POL>(x, p, xv);
 #pragma unroll
-                    for (int j = 0; j < K; ++j)
-                        v[j] = project<POL>(xv[j], POL > 1 ? c[j] : 0.0, POL > 1 ? s[j] : 0.0) - mu;
+                    for (int j = 0; j < K; ++j) v[j] = project<POL>(xv, c, s, j) - mu;
                 }
-                run_scatter<POL, POL>(y, p, [&](int j, double (&o)[POL]) {
-                    if constexpr (POL == 1) { o[0] = v[j]; }
-                    else if constexpr (POL == 2) { o[0] = v[j] * c[j]; o[1] = v[j] * s[j]; }
-                    else { o[0] = v[j]; o[1] = v[j] * c[j]; o[2] = v[j] * s[j]; }
-                });
+                run_scatter<POL, POL>(y, p, pt_contrib<POL>(v, c, s));
             }
         }
         __syncthreads();
@@ -1075,8 +1042,7 @@ __global__ void __launch_bounds__(BLOCK, 2) k_amatvec_filter_poly(const int32_t 
             const double jb = (double)(int)(t0 - a);
             int p[K];
             double c[K], s[K], xv[K][POL];
-            load_pix_keep(pix, t0, nt, p);
-            if (POL > 1) { load_f64_keep(cs, t0, nt, c); load_f64_keep(sn, t0, nt, s); }
+            load_tod<POL, KEEP>(pix, cs, sn, t0, nt, p, c, s);
 #pragma unroll
             for (int j = 0; j < K; ++j) {
                 if (t0 + j < a || t0 + j >= b || p[j] < 0) p[j] = -1;
@@ -1091,7 +1057,7 @@ __global__ void __launch_bounds__(BLOCK, 2) k_amatvec_filter_poly(const int32_t 
                     ++cnt;
                     jmin = min(jmin, jj);
                     jmax = max(jmax, jj);
-                    dv = project<POL>(xv[j], POL > 1 ? c[j] : 0.0, POL > 1 ? s[j] : 0.0);
+                    dv = project<POL>(xv, c, s, j);
                     double L[NK];
                     legendre<NK>(fma(jb + (double)j, step_f, -1.0), L);
                     int q = NK;
@@ -1220,46 +1186,52 @@ __global__ void __launch_bounds__(BLOCK, 2) k_amatvec_filter_poly(const int32_t 
                     for (int r = 0; r < NK; ++r) pj = fma(cf[r], L[r], pj);
                     v[j] = sd[tb + j * 32 + lane] - pj;
                 }
-                run_scatter<POL, POL>(y, p, [&](int j, double (&o)[POL]) {
-                    if constexpr (POL == 1) { o[0] = v[j]; }
-                    else if constexpr (POL == 2) { o[0] = v[j] * c[j]; o[1] = v[j] * s[j]; }
-                    else { o[0] = v[j]; o[1] = v[j] * c[j]; o[2] = v[j] * s[j]; }
-                });
+                run_scatter<POL, POL>(y, p, pt_contrib<POL>(v, c, s));
             }
         }
         __syncthreads();
     }
 }
 
-template <int POL, int NK>
-static int launch_amatvec_filter_poly(const int32_t *pix, const double *c, const double *s, int64_t nt,
-                                      const int64_t *seg_start, const int64_t *seg_end, int64_t nseg, const double *x,
-                                      double *y, int cap, cudaStream_t st) {
-    const size_t smem = (size_t)cap * 12;
-    auto kern = k_amatvec_filter_poly<POL, NK>;
-    CM2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<persistent_grid(kern, BLOCK, smem, nseg), BLOCK, smem, st>>>(pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap);
+// f(std::integral_constant<int, P>{}) for P = pol (check_tod has limited pol to 1..3)
+template <class F>
+static int with_pol(int pol, F f) {
+    if (pol == 1) return f(std::integral_constant<int, 1>{});
+    if (pol == 2) return f(std::integral_constant<int, 2>{});
+    return f(std::integral_constant<int, 3>{});
+}
+
+// CTAs of BLOCK / 32 warp tiles that cover nt samples, `tile` of them per warp tile
+static int64_t tod_blocks(int64_t nt, int64_t tile = TILE) {
+    const int64_t ntiles = (nt + tile - 1) / tile;
+    return (ntiles + (BLOCK / 32) - 1) / (BLOCK / 32);
+}
+
+// launch of a persistent kernel over `blocks` CTAs of work; a dynamic shared-memory size is also set as its limit
+template <class... Params, class... Args>
+static int launch_tod(void (*kern)(Params...), int64_t blocks, size_t smem, cudaStream_t st, Args... args) {
+    if (smem > 0) CM2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<persistent_grid(kern, BLOCK, smem, blocks), BLOCK, smem, st>>>(args...);
     CM2_LAUNCHED();
     return CM2_OK;
+}
+
+// zero fill of n entries of nv 8-byte values (the map a scatter-add accumulates into)
+static cudaError_t zero_fill(void *y, int64_t n, int nv, cudaStream_t st) {
+    return n > 0 ? cudaMemsetAsync(y, 0, sizeof(double) * (size_t)n * nv, st) : cudaSuccess;
 }
 
 template <int POL>
 static int dispatch_amatvec_filter_poly(int nk, const int32_t *pix, const double *c, const double *s, int64_t nt,
                                         const int64_t *seg_start, const int64_t *seg_end, int64_t nseg, const double *x,
                                         double *y, int cap, cudaStream_t st) {
+    const size_t smem = (size_t)cap * 12;
     switch (nk) {
-        case 2: return launch_amatvec_filter_poly<POL, 2>(pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap, st);
-        case 3: return launch_amatvec_filter_poly<POL, 3>(pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap, st);
-        case 4: return launch_amatvec_filter_poly<POL, 4>(pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap, st);
-        default: return launch_amatvec_filter_poly<POL, 5>(pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap, st);
+        case 2: return launch_tod(k_amatvec_filter_poly<POL, 2>, nseg, smem, st, pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap);
+        case 3: return launch_tod(k_amatvec_filter_poly<POL, 3>, nseg, smem, st, pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap);
+        case 4: return launch_tod(k_amatvec_filter_poly<POL, 4>, nseg, smem, st, pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap);
+        default: return launch_tod(k_amatvec_filter_poly<POL, 5>, nseg, smem, st, pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap);
     }
-}
-
-template <class Kern>
-static int tod_grid(Kern k, int64_t nt) {
-    int64_t ntiles = (nt + TILE - 1) / TILE;
-    int64_t blocks = (ntiles + (BLOCK / 32) - 1) / (BLOCK / 32);
-    return persistent_grid(k, BLOCK, 0, blocks);
 }
 
 static int check_tod(const void *pix, const void *c, const void *s, int64_t nt, int pol) {
@@ -1283,11 +1255,7 @@ extern "C" int cm2_pointing_apply(const int32_t *pix, const double *c, const dou
     CM2_REQUIRE(aligned(d, 32), "d must be 32-byte aligned");
     if (nt == 0) return CM2_OK;
     cudaStream_t st = as_stream(stream);
-    if (pol == 1) k_pointing_apply<1><<<tod_grid(k_pointing_apply<1>, nt), BLOCK, 0, st>>>(pix, c, s, nt, x, d);
-    else if (pol == 2) k_pointing_apply<2><<<tod_grid(k_pointing_apply<2>, nt), BLOCK, 0, st>>>(pix, c, s, nt, x, d);
-    else k_pointing_apply<3><<<tod_grid(k_pointing_apply<3>, nt), BLOCK, 0, st>>>(pix, c, s, nt, x, d);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return with_pol(pol, [&](auto P) { return launch_tod(k_pointing_apply<P>, tod_blocks(nt), 0, st, pix, c, s, nt, x, d); });
 }
 
 extern "C" int cm2_pointing_apply_t(const int32_t *pix, const double *c, const double *s, int64_t nt, int pol,
@@ -1297,13 +1265,9 @@ extern "C" int cm2_pointing_apply_t(const int32_t *pix, const double *c, const d
     CM2_REQUIRE(aligned(d, 32), "d must be 32-byte aligned");
     CM2_REQUIRE(npix >= 0, "npix < 0");
     cudaStream_t st = as_stream(stream);
-    if (npix > 0) CM2_CUDA(cudaMemsetAsync(y, 0, sizeof(double) * (size_t)npix * pol, st));
+    CM2_CUDA(zero_fill(y, npix, pol, st));
     if (nt == 0 || npix == 0) return CM2_OK;
-    if (pol == 1) k_pointing_apply_t<1><<<tod_grid(k_pointing_apply_t<1>, nt), BLOCK, 0, st>>>(pix, c, s, nt, d, y);
-    else if (pol == 2) k_pointing_apply_t<2><<<tod_grid(k_pointing_apply_t<2>, nt), BLOCK, 0, st>>>(pix, c, s, nt, d, y);
-    else k_pointing_apply_t<3><<<tod_grid(k_pointing_apply_t<3>, nt), BLOCK, 0, st>>>(pix, c, s, nt, d, y);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return with_pol(pol, [&](auto P) { return launch_tod(k_pointing_apply_t<P>, tod_blocks(nt), 0, st, pix, c, s, nt, d, y); });
 }
 
 static int check_blocks(const double *wblk, int64_t nblocks, int64_t blocksize, const int64_t *blk_start) {
@@ -1332,48 +1296,34 @@ extern "C" int cm2_amatvec_white(const int32_t *pix, const double *c, const doub
     if (rc) return rc;
     CM2_REQUIRE(npix >= 0, "npix < 0");
     cudaStream_t st = as_stream(stream);
-    if (npix > 0) CM2_CUDA(cudaMemsetAsync(y, 0, sizeof(double) * (size_t)npix * pol, st));
+    CM2_CUDA(zero_fill(y, npix, pol, st));
     if (nt == 0 || npix == 0) return CM2_OK;
     const BlockW bw = make_blockw(wblk, nblocks, blocksize, blk_start);
     const TileOrder ord = make_order(nt, nstreams);
     if (g_white_stage_wpix > 0) {
         const int wpix = g_white_stage_wpix;
         const size_t smem = sizeof(double) * (size_t)(BLOCK / 32) * pol * wpix;
-#define CM2_STAGED(POL) do { \
-        CM2_CUDA(cudaFuncSetAttribute(k_amatvec_white_staged<POL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        int64_t ntiles_ = (nt + TILE - 1) / TILE, blocks_ = (ntiles_ + (BLOCK / 32) - 1) / (BLOCK / 32); \
-        k_amatvec_white_staged<POL><<<persistent_grid(k_amatvec_white_staged<POL>, BLOCK, smem, blocks_), BLOCK, smem, st>>>(pix, c, s, nt, bw, ord, x, y, wpix); } while (0)
-        if (pol == 1) CM2_STAGED(1); else if (pol == 2) CM2_STAGED(2); else CM2_STAGED(3);
-#undef CM2_STAGED
-        CM2_LAUNCHED();
-        return CM2_OK;
+        return with_pol(pol, [&](auto P) {
+            return launch_tod(k_amatvec_white_staged<P>, tod_blocks(nt), smem, st, pix, c, s, nt, bw, ord, x, y, wpix);
+        });
     }
-#define CM2_WHITE(POL, ILV) k_amatvec_white<POL, ILV><<<tod_grid(k_amatvec_white<POL, ILV>, nt), BLOCK, 0, st>>>(pix, c, s, nt, bw, ord, x, y)
     if (wblk != nullptr && blk_start == nullptr && blocksize == 1) {      // one weight per sample, streamed
         CM2_REQUIRE(nblocks >= nt && aligned(wblk, 32), "per-sample weights: nt values, 32-byte aligned");
-        if (pol == 1) k_amatvec_white<1, false, true><<<tod_grid(k_amatvec_white<1, false, true>, nt), BLOCK, 0, st>>>(pix, c, s, nt, bw, ord, x, y);
-        else if (pol == 2) k_amatvec_white<2, false, true><<<tod_grid(k_amatvec_white<2, false, true>, nt), BLOCK, 0, st>>>(pix, c, s, nt, bw, ord, x, y);
-        else k_amatvec_white<3, false, true><<<tod_grid(k_amatvec_white<3, false, true>, nt), BLOCK, 0, st>>>(pix, c, s, nt, bw, ord, x, y);
-    } else if (ord.S > 1) {
-        if (pol == 1) CM2_WHITE(1, true); else if (pol == 2) CM2_WHITE(2, true); else CM2_WHITE(3, true);
-    } else {
-        if (pol == 1) CM2_WHITE(1, false); else if (pol == 2) CM2_WHITE(2, false); else CM2_WHITE(3, false);
+        return with_pol(pol, [&](auto P) {
+            return launch_tod(k_amatvec_white<P, false, true>, tod_blocks(nt), 0, st, pix, c, s, nt, bw, ord, x, y);
+        });
     }
-#undef CM2_WHITE
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return with_pol(pol, [&](auto P) {
+        return launch_tod(ord.S > 1 ? k_amatvec_white<P, true> : k_amatvec_white<P, false>, tod_blocks(nt), 0, st,
+                          pix, c, s, nt, bw, ord, x, y);
+    });
 }
 
 template <int POL, int NLAG>
 static int launch_amatvec_toeplitz(const int32_t *pix, const double *c, const double *s, int64_t nt, const ToepW &tw,
                                    const double *x, double *y, cudaStream_t st) {
     constexpr int VAL = TILE - 2 * ((NLAG + K - 1) / K) * K;
-    const int64_t ntiles = (nt + VAL - 1) / VAL;
-    const int64_t blocks = (ntiles + (BLOCK / 32) - 1) / (BLOCK / 32);
-    auto kern = k_amatvec_toeplitz<POL, NLAG>;
-    kern<<<persistent_grid(kern, BLOCK, 0, blocks), BLOCK, 0, st>>>(pix, c, s, nt, tw, x, y);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch_tod(k_amatvec_toeplitz<POL, NLAG>, tod_blocks(nt, VAL), 0, st, pix, c, s, nt, tw, x, y);
 }
 
 template <int POL>
@@ -1401,12 +1351,10 @@ extern "C" int cm2_amatvec_toeplitz(const int32_t *pix, const double *c, const d
                          nband, cm2_amatvec_toeplitz_max_band());
     CM2_REQUIRE(npix >= 0, "npix < 0");
     cudaStream_t st = as_stream(stream);
-    if (npix > 0) CM2_CUDA(cudaMemsetAsync(y, 0, sizeof(double) * (size_t)npix * pol, st));
+    CM2_CUDA(zero_fill(y, npix, pol, st));
     if (nt == 0 || npix == 0) return CM2_OK;
     const ToepW tw{band, nband, make_blockw(nullptr, nblocks, blocksize, blk_start)};
-    if (pol == 1) return dispatch_amatvec_toeplitz<1>(pix, c, s, nt, tw, x, y, st);
-    if (pol == 2) return dispatch_amatvec_toeplitz<2>(pix, c, s, nt, tw, x, y, st);
-    return dispatch_amatvec_toeplitz<3>(pix, c, s, nt, tw, x, y, st);
+    return with_pol(pol, [&](auto P) { return dispatch_amatvec_toeplitz<P>(pix, c, s, nt, tw, x, y, st); });
 }
 
 extern "C" int cm2_weights_moments(const int32_t *pix, const double *c, const double *s, const double *w,
@@ -1419,25 +1367,19 @@ extern "C" int cm2_weights_moments(const int32_t *pix, const double *c, const do
     CM2_REQUIRE(aligned(w, 32), "w must be 32-byte aligned");
     CM2_REQUIRE(npix >= 0, "npix < 0");
     cudaStream_t st = as_stream(stream);
-    if (npix > 0) CM2_CUDA(cudaMemsetAsync(mom, 0, sizeof(double) * 6 * (size_t)npix, st));
+    CM2_CUDA(zero_fill(mom, npix, 6, st));
     if (nt == 0 || npix == 0) return CM2_OK;
     const BlockW bw = make_blockw(wblk, nblocks, blocksize, blk_start);
-    if (pol == 1) k_moments<1><<<tod_grid(k_moments<1>, nt), BLOCK, 0, st>>>(pix, c, s, w, bw, nt, mom);
-    else if (pol == 2) k_moments<2><<<tod_grid(k_moments<2>, nt), BLOCK, 0, st>>>(pix, c, s, w, bw, nt, mom);
-    else k_moments<3><<<tod_grid(k_moments<3>, nt), BLOCK, 0, st>>>(pix, c, s, w, bw, nt, mom);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return with_pol(pol, [&](auto P) { return launch_tod(k_moments<P>, tod_blocks(nt), 0, st, pix, c, s, w, bw, nt, mom); });
 }
 
 extern "C" int cm2_hits_i64(const int32_t *pix, int64_t nt, int64_t npix, int64_t *hits, cm2_stream_t stream) {
     CM2_REQUIRE(nt >= 0 && npix >= 0, "negative size");
     CM2_REQUIRE(aligned(pix, 32), "pix must be 32-byte aligned");
     cudaStream_t st = as_stream(stream);
-    if (npix > 0) CM2_CUDA(cudaMemsetAsync(hits, 0, sizeof(int64_t) * (size_t)npix, st));
+    CM2_CUDA(zero_fill(hits, npix, 1, st));
     if (nt == 0 || npix == 0) return CM2_OK;
-    k_hits<<<tod_grid(k_hits, nt), BLOCK, 0, st>>>(pix, nt, reinterpret_cast<unsigned long long *>(hits));
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch_tod(k_hits, tod_blocks(nt), 0, st, pix, nt, reinterpret_cast<unsigned long long *>(hits));
 }
 
 extern "C" int cm2_amatvec_filter(const int32_t *pix, const double *c, const double *s, int64_t nt, int pol,
@@ -1447,21 +1389,12 @@ extern "C" int cm2_amatvec_filter(const int32_t *pix, const double *c, const dou
     if (rc) return rc;
     CM2_REQUIRE(npix >= 0 && nseg >= 0, "negative size");
     cudaStream_t st = as_stream(stream);
-    if (npix > 0) CM2_CUDA(cudaMemsetAsync(y, 0, sizeof(double) * (size_t)npix * pol, st));
+    CM2_CUDA(zero_fill(y, npix, pol, st));
     if (nt == 0 || npix == 0 || nseg == 0) return CM2_OK;
     const size_t smem = sizeof(double) * SEG_SMEM;
-    if (pol == 1) {
-        CM2_CUDA(cudaFuncSetAttribute(k_amatvec_filter<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_amatvec_filter<1><<<persistent_grid(k_amatvec_filter<1>, BLOCK, smem, nseg), BLOCK, smem, st>>>(pix, c, s, nt, seg_start, seg_end, nseg, x, y);
-    } else if (pol == 2) {
-        CM2_CUDA(cudaFuncSetAttribute(k_amatvec_filter<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_amatvec_filter<2><<<persistent_grid(k_amatvec_filter<2>, BLOCK, smem, nseg), BLOCK, smem, st>>>(pix, c, s, nt, seg_start, seg_end, nseg, x, y);
-    } else {
-        CM2_CUDA(cudaFuncSetAttribute(k_amatvec_filter<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_amatvec_filter<3><<<persistent_grid(k_amatvec_filter<3>, BLOCK, smem, nseg), BLOCK, smem, st>>>(pix, c, s, nt, seg_start, seg_end, nseg, x, y);
-    }
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return with_pol(pol, [&](auto P) {
+        return launch_tod(k_amatvec_filter<P>, nseg, smem, st, pix, c, s, nt, seg_start, seg_end, nseg, x, y);
+    });
 }
 
 extern "C" int cm2_amatvec_filter_mu(const int32_t *pix, const double *c, const double *s, int64_t nt, int pol,
@@ -1472,15 +1405,13 @@ extern "C" int cm2_amatvec_filter_mu(const int32_t *pix, const double *c, const 
     if (rc) return rc;
     CM2_REQUIRE(npix >= 0 && nseg >= 0, "negative size");
     cudaStream_t st = as_stream(stream);
-    if (npix > 0) CM2_CUDA(cudaMemsetAsync(y, 0, sizeof(double) * (size_t)npix * pol, st));
+    CM2_CUDA(zero_fill(y, npix, pol, st));
     if (nt == 0 || npix == 0 || nseg == 0) return CM2_OK;
     SegInfo sg{seg_start, seg_end, seg_mu, tile_seg, tile_flag, nseg};
     const TileOrder ord = make_order(nt, nstreams);
-    if (pol == 1) k_amatvec_filter_mu<1><<<tod_grid(k_amatvec_filter_mu<1>, nt), BLOCK, 0, st>>>(pix, c, s, nt, sg, ord, x, y);
-    else if (pol == 2) k_amatvec_filter_mu<2><<<tod_grid(k_amatvec_filter_mu<2>, nt), BLOCK, 0, st>>>(pix, c, s, nt, sg, ord, x, y);
-    else k_amatvec_filter_mu<3><<<tod_grid(k_amatvec_filter_mu<3>, nt), BLOCK, 0, st>>>(pix, c, s, nt, sg, ord, x, y);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return with_pol(pol, [&](auto P) {
+        return launch_tod(k_amatvec_filter_mu<P>, tod_blocks(nt), 0, st, pix, c, s, nt, sg, ord, x, y);
+    });
 }
 
 extern "C" int cm2_pointing_filter_mu(const int32_t *pix, const double *c, const double *s, int64_t nt, int pol,
@@ -1494,30 +1425,23 @@ extern "C" int cm2_pointing_filter_mu(const int32_t *pix, const double *c, const
     if (nt == 0) return CM2_OK;
     cudaStream_t st = as_stream(stream);
     if (nseg == 0) {
-        CM2_CUDA(cudaMemsetAsync(d, 0, sizeof(double) * (size_t)nt, st));
+        CM2_CUDA(zero_fill(d, nt, 1, st));
         return CM2_OK;
     }
     SegInfo sg{seg_start, seg_end, seg_mu, tile_seg, tile_flag, nseg};
-    if (pol == 1) k_pointing_filter_mu<1><<<tod_grid(k_pointing_filter_mu<1>, nt), BLOCK, 0, st>>>(pix, c, s, nt, sg, x, d);
-    else if (pol == 2) k_pointing_filter_mu<2><<<tod_grid(k_pointing_filter_mu<2>, nt), BLOCK, 0, st>>>(pix, c, s, nt, sg, x, d);
-    else k_pointing_filter_mu<3><<<tod_grid(k_pointing_filter_mu<3>, nt), BLOCK, 0, st>>>(pix, c, s, nt, sg, x, d);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return with_pol(pol, [&](auto P) { return launch_tod(k_pointing_filter_mu<P>, tod_blocks(nt), 0, st, pix, c, s, nt, sg, x, d); });
 }
 
 template <int POL>
 static int dispatch_amatvec_filter_poly_mu(int nk, const int32_t *pix, const double *c, const double *s, int64_t nt,
                                            const SegPoly &sg, const TileOrder &ord, const double *x, double *y, cudaStream_t st) {
-#define CM2_POLY_MU(NK) k_amatvec_filter_poly_mu<POL, NK><<<tod_grid(k_amatvec_filter_poly_mu<POL, NK>, nt), BLOCK, 0, st>>>(pix, c, s, nt, sg, ord, x, y)
+    const int64_t blocks = tod_blocks(nt);
     switch (nk) {
-        case 2: CM2_POLY_MU(2); break;
-        case 3: CM2_POLY_MU(3); break;
-        case 4: CM2_POLY_MU(4); break;
-        default: CM2_POLY_MU(5); break;
+        case 2: return launch_tod(k_amatvec_filter_poly_mu<POL, 2>, blocks, 0, st, pix, c, s, nt, sg, ord, x, y);
+        case 3: return launch_tod(k_amatvec_filter_poly_mu<POL, 3>, blocks, 0, st, pix, c, s, nt, sg, ord, x, y);
+        case 4: return launch_tod(k_amatvec_filter_poly_mu<POL, 4>, blocks, 0, st, pix, c, s, nt, sg, ord, x, y);
+        default: return launch_tod(k_amatvec_filter_poly_mu<POL, 5>, blocks, 0, st, pix, c, s, nt, sg, ord, x, y);
     }
-#undef CM2_POLY_MU
-    CM2_LAUNCHED();
-    return CM2_OK;
 }
 
 /* single-TOD-pass P^T F_K P given the per-subscan Legendre coefficients (cm2_filter_poly_seg_coef);
@@ -1533,14 +1457,12 @@ extern "C" int cm2_amatvec_filter_poly_mu(const int32_t *pix, const double *c, c
     if (poly_order < 1 || poly_order > 4)
         return set_error(CM2_ERR_UNSUPPORTED, "run-table Legendre A-matvec: poly_order=%d, orders 1..4 are supported", poly_order);
     cudaStream_t st = as_stream(stream);
-    if (npix > 0 && !accumulate) CM2_CUDA(cudaMemsetAsync(y, 0, sizeof(double) * (size_t)npix * pol, st));
+    if (!accumulate) CM2_CUDA(zero_fill(y, npix, pol, st));
     if (nt == 0 || npix == 0 || nseg == 0) return CM2_OK;
     SegPoly sg{seg_start, seg_end, seg_coef, tile_seg, tile_flag, nseg};
     const int nk = poly_order + 1;
     const TileOrder ord = make_order(nt, nstreams);
-    if (pol == 1) return dispatch_amatvec_filter_poly_mu<1>(nk, pix, c, s, nt, sg, ord, x, y, st);
-    if (pol == 2) return dispatch_amatvec_filter_poly_mu<2>(nk, pix, c, s, nt, sg, ord, x, y, st);
-    return dispatch_amatvec_filter_poly_mu<3>(nk, pix, c, s, nt, sg, ord, x, y, st);
+    return with_pol(pol, [&](auto P) { return dispatch_amatvec_filter_poly_mu<P>(nk, pix, c, s, nt, sg, ord, x, y, st); });
 }
 
 /* fused P^T F_K P, Legendre subscan filter of order 1..4 */
@@ -1561,10 +1483,10 @@ extern "C" int cm2_amatvec_filter_poly(const int32_t *pix, const double *c, cons
         return set_error(CM2_ERR_UNSUPPORTED, "fused Legendre A-matvec: subscan of %lld samples exceeds the shared-memory window",
                          (long long)max_seg_len);
     cudaStream_t st = as_stream(stream);
-    if (npix > 0) CM2_CUDA(cudaMemsetAsync(y, 0, sizeof(double) * (size_t)npix * pol, st));
+    CM2_CUDA(zero_fill(y, npix, pol, st));
     if (nt == 0 || npix == 0 || nseg == 0) return CM2_OK;
     const int nk = poly_order + 1;
-    if (pol == 1) return dispatch_amatvec_filter_poly<1>(nk, pix, c, s, nt, seg_start, seg_end, nseg, x, y, (int)cap, st);
-    if (pol == 2) return dispatch_amatvec_filter_poly<2>(nk, pix, c, s, nt, seg_start, seg_end, nseg, x, y, (int)cap, st);
-    return dispatch_amatvec_filter_poly<3>(nk, pix, c, s, nt, seg_start, seg_end, nseg, x, y, (int)cap, st);
+    return with_pol(pol, [&](auto P) {
+        return dispatch_amatvec_filter_poly<P>(nk, pix, c, s, nt, seg_start, seg_end, nseg, x, y, (int)cap, st);
+    });
 }
