@@ -46,7 +46,8 @@ SIGNATURES = {
     "cm2_toeplitz_fft_scratch_bytes": (_i64, [_i64]),
     "cm2_noise_toeplitz_fft_apply": (_int, [_vp, _int, _i64, _i64, _vp, _vp, _vp, _i64, _vp, _int, _int, _vp]),
     "cm2_filter_offset_apply": (_int, [_vp, _vp, _vp, _i64, _vp, _vp, _i64, _vp]),
-    "cm2_amatvec_white": (_int, [_vp, _vp, _vp, _i64, _int, _vp, _i64, _i64, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "cm2_amatvec_white": (_int, [_vp, _vp, _vp, _vp, _i64, _int, _vp, _i64, _i64, _vp, _vp, _vp, _i64, _i64, _vp]),
+    "cm2_pack_pointing": (_int, [_vp, _i64, _vp, _vp, _vp]),
     "cm2_amatvec_white_set_stage": (_int, [_int]),
     "cm2_amatvec_filter": (_int, [_vp, _vp, _vp, _i64, _int, _vp, _vp, _i64, _vp, _vp, _i64, _vp]),
     "cm2_filter_runs_mark": (_int, [_vp, _vp, _vp, _i64, _i64, _vp, _vp, _vp]),

@@ -144,6 +144,47 @@ __device__ __forceinline__ void load_f64(const double *__restrict__ a, int64_t t
     }
 }
 
+// Packed pixel stream (cm2_pack_pointing): one 64-bit word per lane of K samples, word t0 / K for the samples
+// t0 .. t0 + K - 1, so a warp tile reads 256 contiguous bytes instead of 1 kB of int32 ids.  lo = bits 0..31, signed:
+//   lo >= 0  b0 = lo, b1 = b0 + (int16) bits 32..47, codes = bits 48..63: sample j is (code & 2 ? b1 : b0) + (code & 1),
+//            code = (codes >> 2j) & 3.  A raster sweep crosses each pixel in a run of samples and steps to the next
+//            pixel or, at a row change, jumps by about a row length: two bases cover both.
+//   lo == -1 every sample of the lane is flagged (-1).  The packer leaves bits 32..63 zero, so the decode of the
+//            lo >= 0 case yields -1 for all K samples too.
+//   lo == -2 escape: the lane reads its pixels from the int32 array.  Lanes that mix flagged and unflagged
+//            samples, lanes the two bases do not cover, and a last lane of fewer than K samples escape.
+constexpr int PK_FLAGGED = -1, PK_ESCAPE = -2;
+
+__device__ __forceinline__ uint64_t ld_stream_u64(const uint64_t *p) {
+    // the .L2::evict_first form of ld needs a 256-bit vector; an evict-first access policy does the same for 64 bits
+    uint64_t pol, r;
+    asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
+    asm volatile("ld.global.L1::no_allocate.L2::cache_hint.b64 %0, [%1], %2;" : "=l"(r) : "l"(p), "l"(pol));
+    return r;
+}
+
+// The packed word of the lane at t0, PK_ESCAPE for a lane of fewer than K samples.  The load and the decode are apart
+// (unpack_pix) so that the escape branch, which needs the word, does not hold back the work between them.
+__device__ __forceinline__ uint64_t load_packed(const uint64_t *__restrict__ pk, int64_t t0, int64_t nt) {
+    return t0 + K <= nt ? ld_stream_u64(pk + t0 / K) : (uint64_t)(uint32_t)PK_ESCAPE;
+}
+
+__device__ __forceinline__ void unpack_pix(uint64_t wd, const int32_t *__restrict__ pix, int64_t t0, int64_t nt,
+                                           int (&p)[K]) {
+    const int b0 = (int)(uint32_t)wd;
+    if (b0 == PK_ESCAPE) {
+        load_pix(pix, t0, nt, p);
+        return;
+    }
+    const int b1 = b0 + (int)(int16_t)(uint16_t)(wd >> 32);
+    const unsigned codes = (unsigned)(wd >> 48);
+#pragma unroll
+    for (int j = 0; j < K; ++j) {
+        const unsigned code = (codes >> (2 * j)) & 3u;
+        p[j] = ((code & 2u) ? b1 : b0) + (int)(code & 1u);
+    }
+}
+
 // pixels and, for POL > 1, cos / sin of the K samples starting at t0
 template <int POL, Cache CP = STREAM>
 __device__ __forceinline__ void load_tod(const int32_t *__restrict__ pix, const double *__restrict__ cs,
@@ -151,6 +192,38 @@ __device__ __forceinline__ void load_tod(const int32_t *__restrict__ pix, const 
                                          double (&c)[K], double (&s)[K]) {
     load_pix<CP>(pix, t0, nt, p);
     if (POL > 1) { load_f64<CP>(cs, t0, nt, c); load_f64<CP>(sn, t0, nt, s); }
+}
+
+// the packed word of the K samples q (format above)
+__device__ __forceinline__ uint64_t pack_lane(const int (&q)[K]) {
+    bool all_flagged = true, any_flagged = false;
+    int b0 = q[0];
+#pragma unroll
+    for (int j = 0; j < K; ++j) {
+        all_flagged &= q[j] == -1;
+        any_flagged |= q[j] < 0;
+        b0 = min(b0, q[j]);
+    }
+    if (all_flagged) return (uint32_t)PK_FLAGGED;
+    if (any_flagged) return (uint32_t)PK_ESCAPE;
+    // b0 = the smallest pixel covers {b0, b0 + 1}; b1 = the smallest pixel above those covers {b1, b1 + 1}
+    int b1 = b0;
+#pragma unroll
+    for (int j = 0; j < K; ++j) {
+        if (q[j] - b0 > 1 && (b1 == b0 || q[j] < b1)) b1 = q[j];
+    }
+    if (b1 - b0 > INT16_MAX) return (uint32_t)PK_ESCAPE;
+    uint64_t codes = 0;
+#pragma unroll
+    for (int j = 0; j < K; ++j) {
+        const int d0 = q[j] - b0, d1 = q[j] - b1;
+        unsigned code;
+        if (d0 <= 1) code = (unsigned)d0;
+        else if (d1 <= 1) code = 2u + (unsigned)d1;
+        else return (uint32_t)PK_ESCAPE;
+        codes |= (uint64_t)code << (2 * j);
+    }
+    return (uint64_t)(uint32_t)b0 | ((uint64_t)(uint16_t)(b1 - b0) << 32) | (codes << 48);
 }
 
 // x values of the K samples; one gather per run start, copied along the run
@@ -361,10 +434,12 @@ __global__ void __launch_bounds__(BLOCK) k_pointing_apply_t(const int32_t *__res
 // Fused y = P^T diag(w) P x.  The next tile's pix/cos/sin loads are issued between the compress
 // and the merge phase of the current tile, so their DRAM latency overlaps the shuffles and REDs.
 // WS = true: per-sample weights bw.w[t] (blocks of one sample: the pixel-sorted pointing copy), read as a stream.
-template <int POL, bool ILV, bool WS = false>
+// PK = true: the pixels come from the packed stream pk (8 B per lane instead of 32), int32 pix for escape lanes.
+template <int POL, bool ILV, bool WS = false, bool PK = false>
 __global__ void __launch_bounds__(BLOCK) k_amatvec_white(const int32_t *__restrict__ pix, const double *__restrict__ cs,
                                                          const double *__restrict__ sn, int64_t nt, BlockW bw, TileOrder ord,
-                                                         const double *__restrict__ x, double *__restrict__ y) {
+                                                         const double *__restrict__ x, double *__restrict__ y,
+                                                         const uint64_t *__restrict__ pk) {
     const int lane = threadIdx.x & 31;
     const int64_t nwarps = (int64_t)gridDim.x * (BLOCK / 32);
     const int64_t ntiles = (nt + TILE - 1) / TILE;
@@ -375,7 +450,17 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_white(const int32_t *__restri
     // ILV = false: time order (the instantiation measured on configs[1]); true: detector-interleaved (TileOrder).
     RunState<POL> rs = RunState<POL>::empty();
     const int64_t nv = ILV ? ord.count() : ntiles;
-    for (int64_t vt = (int64_t)blockIdx.x * (BLOCK / 32) + (threadIdx.x >> 5); vt < nv; vt += nwarps) {
+    const int64_t vt0 = (int64_t)blockIdx.x * (BLOCK / 32) + (threadIdx.x >> 5);
+    // PK: the packed word is loaded one trip ahead (2 registers), so the decode and the x gather do not wait for it
+    uint64_t wd_next = 0;
+    if constexpr (PK) wd_next = load_packed(pk, (ILV ? ord.tile(vt0) : vt0) * TILE + (int64_t)lane * K, nt);
+    for (int64_t vt = vt0; vt < nv; vt += nwarps) {
+        uint64_t wd = 0;
+        if constexpr (PK) {
+            wd = wd_next;
+            const int64_t vn = vt + nwarps;
+            wd_next = load_packed(pk, vn < nv ? (ILV ? ord.tile(vn) : vn) * TILE + (int64_t)lane * K : nt, nt);
+        }
         int64_t tile = vt;
         if constexpr (ILV) {
             tile = ord.tile(vt);
@@ -384,8 +469,13 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_white(const int32_t *__restri
         const int64_t t0 = tile * TILE + (int64_t)lane * K;
         int p[K];
         double c[K], s[K];
-        load_tod<POL>(pix, cs, sn, t0, nt, p, c, s);
+        if constexpr (PK) {
+            if (POL > 1) { load_f64(cs, t0, nt, c); load_f64(sn, t0, nt, s); }
+        } else {
+            load_tod<POL>(pix, cs, sn, t0, nt, p, c, s);
+        }
         run_merge<POL, POL>(y, rs);             // previous tile (the empty state on the first trip emits nothing)
+        if constexpr (PK) unpack_pix(wd, pix, t0, nt, p);
         double w[K], xv[K][POL], v[K];
         if constexpr (WS) load_f64(bw.w, t0, nt, w);
         gather_x<POL>(x, p, xv);
@@ -395,6 +485,24 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_white(const int32_t *__restri
         run_compress<POL, POL>(y, p, pt_contrib<POL>(v, c, s), rs);
     }
     run_merge<POL, POL>(y, rs);
+}
+
+// packed[l] = the packed word of lane l (samples 8 l .. 8 l + 7), one thread per lane; *nescape += escape lanes
+__global__ void __launch_bounds__(BLOCK) k_pack_pointing(const int32_t *__restrict__ pix, int64_t nt,
+                                                         uint64_t *__restrict__ packed, unsigned long long *__restrict__ nescape) {
+    const int64_t nlanes = (nt + K - 1) / K;
+    unsigned nesc = 0;
+    for (int64_t l = (int64_t)blockIdx.x * BLOCK + threadIdx.x; l < nlanes; l += (int64_t)gridDim.x * BLOCK) {
+        uint64_t wd = (uint32_t)PK_ESCAPE;
+        if (l * K + K <= nt) {
+            const I8 v = ld_stream_i8(pix + l * K);
+            wd = pack_lane(v.v);
+        }
+        nesc += (int)(uint32_t)wd == PK_ESCAPE;
+        packed[l] = wd;
+    }
+    nesc = __reduce_add_sync(FULL, nesc);
+    if ((threadIdx.x & 31) == 0 && nesc) atomicAdd(nescape, (unsigned long long)nesc);
 }
 
 // Variant of k_amatvec_white with the scatter STAGED through shared memory: when the pixels of a warp tile span
@@ -1287,20 +1395,23 @@ extern "C" int cm2_amatvec_white_set_stage(int wpix) {
     return CM2_OK;
 }
 
-extern "C" int cm2_amatvec_white(const int32_t *pix, const double *c, const double *s, int64_t nt, int pol,
-                                 const double *wblk, int64_t nblocks, int64_t blocksize, const int64_t *blk_start,
-                                 const double *x, double *y, int64_t npix, int64_t nstreams, cm2_stream_t stream) {
+extern "C" int cm2_amatvec_white(const int32_t *pix, const uint64_t *pix_packed, const double *c, const double *s,
+                                 int64_t nt, int pol, const double *wblk, int64_t nblocks, int64_t blocksize,
+                                 const int64_t *blk_start, const double *x, double *y, int64_t npix, int64_t nstreams,
+                                 cm2_stream_t stream) {
     int rc = check_tod(pix, c, s, nt, pol);
     if (rc) return rc;
     rc = check_blocks(wblk, nblocks, blocksize, blk_start);
     if (rc) return rc;
     CM2_REQUIRE(npix >= 0, "npix < 0");
+    CM2_REQUIRE(aligned(pix_packed, 8), "pix_packed must be 8-byte aligned");
     cudaStream_t st = as_stream(stream);
     CM2_CUDA(zero_fill(y, npix, pol, st));
     if (nt == 0 || npix == 0) return CM2_OK;
     const BlockW bw = make_blockw(wblk, nblocks, blocksize, blk_start);
     const TileOrder ord = make_order(nt, nstreams);
     if (g_white_stage_wpix > 0) {
+        CM2_REQUIRE(pix_packed == nullptr, "the staged scatter reads int32 pixels only");
         const int wpix = g_white_stage_wpix;
         const size_t smem = sizeof(double) * (size_t)(BLOCK / 32) * pol * wpix;
         return with_pol(pol, [&](auto P) {
@@ -1309,14 +1420,28 @@ extern "C" int cm2_amatvec_white(const int32_t *pix, const double *c, const doub
     }
     if (wblk != nullptr && blk_start == nullptr && blocksize == 1) {      // one weight per sample, streamed
         CM2_REQUIRE(nblocks >= nt && aligned(wblk, 32), "per-sample weights: nt values, 32-byte aligned");
+        CM2_REQUIRE(pix_packed == nullptr, "per-sample weights read int32 pixels only");
         return with_pol(pol, [&](auto P) {
-            return launch_tod(k_amatvec_white<P, false, true>, tod_blocks(nt), 0, st, pix, c, s, nt, bw, ord, x, y);
+            return launch_tod(k_amatvec_white<P, false, true>, tod_blocks(nt), 0, st, pix, c, s, nt, bw, ord, x, y,
+                              (const uint64_t *)nullptr);
         });
     }
     return with_pol(pol, [&](auto P) {
-        return launch_tod(ord.S > 1 ? k_amatvec_white<P, true> : k_amatvec_white<P, false>, tod_blocks(nt), 0, st,
-                          pix, c, s, nt, bw, ord, x, y);
+        auto kern = ord.S > 1 ? (pix_packed ? k_amatvec_white<P, true, false, true> : k_amatvec_white<P, true>)
+                              : (pix_packed ? k_amatvec_white<P, false, false, true> : k_amatvec_white<P, false>);
+        return launch_tod(kern, tod_blocks(nt), 0, st, pix, c, s, nt, bw, ord, x, y, pix_packed);
     });
+}
+
+/* the packed pixel stream of pix (format at PK_ESCAPE) and its number of escape lanes */
+extern "C" int cm2_pack_pointing(const int32_t *pix, int64_t nt, uint64_t *packed, int64_t *nescape, cm2_stream_t stream) {
+    CM2_REQUIRE(nt >= 0, "nt < 0");
+    CM2_REQUIRE(nescape != nullptr && (nt == 0 || (pix != nullptr && packed != nullptr)), "NULL argument");
+    CM2_REQUIRE(aligned(pix, 32) && aligned(packed, 8), "pix must be 32-byte and packed 8-byte aligned");
+    cudaStream_t st = as_stream(stream);
+    CM2_CUDA(zero_fill(nescape, 1, 1, st));
+    if (nt == 0) return CM2_OK;
+    return launch_tod(k_pack_pointing, tod_blocks(nt), 0, st, pix, nt, packed, reinterpret_cast<unsigned long long *>(nescape));
 }
 
 template <int POL, int NLAG>

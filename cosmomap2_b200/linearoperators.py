@@ -578,6 +578,9 @@ WHITE_STAGE_RUN_RANGE = (3.0, 6.0)   # mean run length for which the staged scat
 WHITE_STAGE_MIN_CONTIGUITY = 0.9     # ... on sweeps along pixel rows only (a tilted scan changes row at most pixel changes)
 WHITE_STAGE_WINDOW = 288             # pixels per warp tile
 WHITE_SORT_BELOW_RUN = 3.0           # below: the white A-matvec runs over a pixel-sorted copy of the pointing
+WHITE_PACK_BELOW_RUN = 16.0          # register scatter in time order along pixel rows with shorter runs: packed pixel
+                                     # stream (measured, tools/pack_probe.py: faster at 8 samples per pixel crossing,
+                                     # slower at 32, on a tilted scan and in the detector-interleaved order)
 
 
 class _FusedWhiteA(lp.LinearOperator):
@@ -594,7 +597,12 @@ class _FusedWhiteA(lp.LinearOperator):
       the pass (0.96 / 1.83 / 2.2 ms per 1e8 samples at 2 / 1 samples per pixel / random); white noise has no
       time-domain structure, so the pass runs over a copy of the pointing SORTED BY PIXEL with per-sample
       weights instead (28 B/sample, every pixel one run: 0.45 ms).  Set-up: one stable sort; memory: a second
-      copy of the pointing."""
+      copy of the pointing.
+
+    In time order, for runs of fewer than 16 samples along pixel rows (configs[1]: 8), the register scatter reads the
+    pixel ids from a packed stream built at first use (cm2_pack_pointing: two base pixels and a 2-bit code per sample,
+    1 byte per sample instead of 4; lanes it cannot encode read the int32 ids), 17 instead of 20 B/sample.  It lives
+    as long as the operator: nt bytes of device memory (100 MB per 1e8 samples)."""
 
     def __init__(self, P, N):
         self.P, self.N = P, N
@@ -603,6 +611,8 @@ class _FusedWhiteA(lp.LinearOperator):
         self._streams = _tod_streams(P, bs)
         self._mode = None
         self._sorted = None
+        self._packed = None
+        self.nescape = 0
         super(_FusedWhiteA, self).__init__(n, n, matvec=self._run, symmetric=True, device=True)
 
     def _choose(self):
@@ -614,6 +624,24 @@ class _FusedWhiteA(lp.LinearOperator):
             self._mode = "staged"
         else:
             self._mode = "registers"
+            if self._streams == 1 and run < WHITE_PACK_BELOW_RUN and contig >= WHITE_STAGE_MIN_CONTIGUITY:
+                self._build_packed()
+
+    def _build_packed(self):
+        P = self.P
+        self._packed = torch.empty(max((P.nrows + 7) // 8, 1), dtype=torch.int64, device=P._pix_dev.device)
+        nesc = torch.empty(1, dtype=torch.int64, device=P._pix_dev.device)
+        dv.call("cm2_pack_pointing", dv.ptr(P._pix_dev), P.nrows, dv.ptr(self._packed), dv.ptr(nesc), _stream())
+        self.nescape = int(nesc.item())
+
+    def tod_bytes(self):
+        """Bytes of TOD one apply reads: 20 per sample, or with the packed pixel stream 17 per sample plus the
+        32 bytes of int32 ids of every escape lane."""
+        if self._mode is None:
+            self._choose()
+        if self._packed is not None:
+            return 17 * self.P.nrows + 32 * self.nescape
+        return 20 * self.P.nrows
 
     def _build_sorted(self):
         P, N = self.P, self.N
@@ -644,7 +672,7 @@ class _FusedWhiteA(lp.LinearOperator):
         y = dv.out_f64(P.ncols * P.pol)
         if self._mode == "sorted":
             pix, cs, sn, w, nts = self._sorted
-            dv.call("cm2_amatvec_white", dv.ptr(pix), dv.ptr(cs), dv.ptr(sn), nts, P.pol,
+            dv.call("cm2_amatvec_white", dv.ptr(pix), None, dv.ptr(cs), dv.ptr(sn), nts, P.pol,
                     dv.ptr(w) if w is not None else None, nts if w is not None else 0, 1, None, dv.ptr(x), dv.ptr(y),
                     P.ncols, 1, _stream())
             return y
@@ -656,8 +684,9 @@ class _FusedWhiteA(lp.LinearOperator):
         if self._mode == "staged":
             dv.call("cm2_amatvec_white_set_stage", WHITE_STAGE_WINDOW)
         try:
-            dv.call("cm2_amatvec_white", dv.ptr(P._pix_dev), dv.ptr(P._cos_dev), dv.ptr(P._sin_dev), P.nrows, P.pol,
-                    w, nb, bs, startp, dv.ptr(x), dv.ptr(y), P.ncols, self._streams, _stream())
+            dv.call("cm2_amatvec_white", dv.ptr(P._pix_dev), dv.ptr(self._packed),
+                    dv.ptr(P._cos_dev), dv.ptr(P._sin_dev), P.nrows, P.pol, w, nb, bs, startp, dv.ptr(x), dv.ptr(y),
+                    P.ncols, self._streams, _stream())
         finally:
             if self._mode == "staged":
                 dv.call("cm2_amatvec_white_set_stage", 0)

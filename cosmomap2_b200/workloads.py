@@ -419,11 +419,14 @@ def white(nt=1e9, nside=2048, nx=3200, ny=1600, ndet=64, steps=30):
         solver.tick()
     it_ms = time_device(one_step, steps)
     al_ms = time_device(lambda: A_local._apply(x), steps)
+    from cosmomap2_b200 import linearoperators as lo
+    fused = [f for f in A_local.planned() if isinstance(f, lo._FusedWhiteA)]
+    tod_bytes = fused[0].tod_bytes() if fused else 20.0 * nt     # 17 B/sample + escape lanes with the packed pixel stream
     out = {"config": "configs[4]: white noise, IQU nside=%d, M_BD PCG" % nside, "world": world, "nt_total": nt * world,
            "nt_per_gpu": nt, "npix": int(npix), "nside": nside, "cg_info": int(info), "relres": relres,
            "ms_per_pcg_iteration": it_ms, "samples_per_s_per_pcg_iter": nt * world / (it_ms * 1e-3),
            "A_local_apply_ms": al_ms,
-           "roofline": _roofline("k_amatvec_white<3> (cm2_amatvec_white)", 20.0 * nt + 48.0 * npix, al_ms),
+           "roofline": _roofline("k_amatvec_white<3> (cm2_amatvec_white)", tod_bytes + 48.0 * npix, al_ms),
            "solver": type(solver).__name__, "hbm_GB": torch.cuda.max_memory_allocated() / 1e9}
     _close(A)
     return out

@@ -148,11 +148,23 @@ int cm2_filter_offset_apply(const int32_t *pix, const int64_t *seg_start, const 
  * detector-major, interfaces/linearoperators.py:134-140) that are walked round-robin, tile by tile, so that
  * all detectors are processed at the same scan time and the map rows they share stay in L2 -- for maps larger
  * than L2 (nside >= 1024 patches), where time order makes every detector timeline a pass over the whole map.
- * The result is the same sum in a different order of the atomic adds. */
-int cm2_amatvec_white(const int32_t *pix, const double *cos2phi, const double *sin2phi,
-                      int64_t nt, int pol, const double *wblk, int64_t nblocks,
+ * The result is the same sum in a different order of the atomic adds.
+ * pix_packed: NULL, or the packed stream of pix from cm2_pack_pointing; the pass then reads 1 byte of pixel id
+ * per sample instead of 4 (17 instead of 20 B/sample) and pix only for escape lanes.  Not with per-sample
+ * weights (blocksize 1) or the staged scatter (cm2_amatvec_white_set_stage), which read pix. */
+int cm2_amatvec_white(const int32_t *pix, const uint64_t *pix_packed, const double *cos2phi,
+                      const double *sin2phi, int64_t nt, int pol, const double *wblk, int64_t nblocks,
                       int64_t blocksize, const int64_t *blk_start, const double *x, double *y,
                       int64_t npix, int64_t nstreams, cm2_stream_t stream);
+/* packed[(nt + 7) / 8] = pix at one byte per sample, one 64-bit word per 8 samples t0 .. t0+7 (t0 = 8 l).  With
+ * lo = the signed bits 0..31 of a word:
+ *   lo >= 0   b0 = lo, b1 = b0 + (int16) bits 32..47, codes = bits 48..63; sample j has pixel
+ *             (code_j & 2 ? b1 : b0) + (code_j & 1), code_j = (codes >> 2j) & 3;
+ *   lo == -1  all 8 samples are flagged (-1); bits 32..63 are zero;
+ *   lo == -2  escape: read the 8 pixels from pix (mixed flagged and unflagged samples, pixels the two bases do
+ *             not cover, and the last word when nt % 8 != 0).
+ * *nescape = the number of escape words.  pix 32-byte aligned. */
+int cm2_pack_pointing(const int32_t *pix, int64_t nt, uint64_t *packed, int64_t *nescape, cm2_stream_t stream);
 /* Scatter variant of cm2_amatvec_white: wpix > 0 stages the scatter of every warp tile whose pixels span fewer
  * than wpix pixels through a shared-memory window and flushes it with coalesced REDs (pixels crossed in few
  * samples: 1-4 samples per pixel crossing); 0 = run compression in registers + warp merge (the default). */
