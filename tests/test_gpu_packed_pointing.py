@@ -93,6 +93,18 @@ def _case(name):
         lanes = [[5, 5, 6, 6, 5 + d, 5 + d, 6 + d, 6 + d] for d in (2, 1000, 32767, 32768, 40000, 1 << 30)]
         lanes += [[7 + d, 7 + d, 8 + d, 7, 7, 8, 8 + d, 8] for d in (32767, 32768)]
         return np.array(lanes * 40, dtype=np.int32).ravel()
+    if name == "descending":                 # ids fall along time: b0 is a later sample of the lane; backward row jumps
+        r = np.arange(40 * 1024) // 3
+        return (10 ** 6 - (r // 97) * 300 - r % 97).astype(np.int32)
+    if name == "code3_edges":                # delta 2 and 32766 / 32767 with code 3 (b1 + 1), and 32768 (escape)
+        lanes = [[0, 0, 1, 1, 2, 2, 3, 3], [0, 32766, 32767, 0, 1, 32767, 1, 0],
+                 [32767, 32768, 0, 1, 0, 32768, 1, 32767], [32767, 32767, 32766, 0, 0, 1, 32766, 1],
+                 [0, 1, 32768, 32769, 0, 1, 32768, 32769]]
+        return (np.array(lanes * 40, dtype=np.int32) + 100).ravel()
+    if name == "flagged_by_escapes":         # all-flagged lanes next to escape lanes (mixed flags, three clusters)
+        lanes = [[-1] * 8, [4, -1, 4, 4, 5, -1, 5, 4], [-1] * 8, [0, 5, 10, 0, 5, 10, 0, 0], [-1] * 8, [7] * 8]
+        order = np.random.default_rng(5).integers(0, len(lanes), 4000)
+        return np.array(lanes, dtype=np.int32)[order].ravel()
     if name == "random":                     # mostly escape lanes
         return rng.integers(0, 3 * 10 ** 6, 50021).astype(np.int32)
     if name == "short":
@@ -102,7 +114,8 @@ def _case(name):
     raise KeyError(name)
 
 
-@pytest.mark.parametrize("case", ["raster", "odd_nt", "flags", "detector_blocks", "row_jump", "random", "short", "empty"])
+@pytest.mark.parametrize("case", ["raster", "odd_nt", "flags", "detector_blocks", "row_jump", "descending", "code3_edges",
+                                  "flagged_by_escapes", "random", "short", "empty"])
 def test_pack_round_trip(cm, case):
     pix = _case(case)
     words, nesc = pack(pix)
@@ -114,6 +127,13 @@ def test_pack_round_trip(cm, case):
         assert list(lo[:8]) == [5, 5, 5, -2, -2, -2, 7, -2]
     if case == "raster":
         assert nesc < 1e-3 * words.size
+    if case in ("descending", "code3_edges"):
+        lo = (words & 0xffffffff).astype(np.uint32).view(np.int32)
+        delta = ((words >> 32) & 0xffff).astype(np.uint16).view(np.int16)
+        if case == "descending":
+            assert np.all(np.diff(lo[lo >= 0]) <= 0) and np.count_nonzero(lo >= 0) > 0.99 * lo.size
+        else:
+            assert list(lo[:5]) == [100, 100, 100, 100, -2] and list(delta[:4]) == [2, 32766, 32767, 32766]
     if case == "random":
         assert nesc > 0.9 * words.size
 
