@@ -94,13 +94,8 @@ extern "C" int cm2_pointing_apply_t_sorted(const int64_t *rowptr, const int32_t 
     CM2_REQUIRE(pol >= 1 && pol <= 3, "No valid polarization key set! (1=I, 2=QU, 3=IQU)");
     CM2_REQUIRE(npix >= 0, "npix < 0");
     if (npix == 0) return CM2_OK;
-    cudaStream_t st = as_stream(stream);
-    int64_t blocks = (npix + 7) / 8;
-    int64_t cap = (int64_t)sm_count() * 8;
-    int g = (int)(blocks < cap ? blocks : cap);
-    if (pol == 1) k_apply_t_sorted<1><<<g, 256, 0, st>>>(rowptr, perm, c, s, d, y, npix);
-    else if (pol == 2) k_apply_t_sorted<2><<<g, 256, 0, st>>>(rowptr, perm, c, s, d, y, npix);
-    else k_apply_t_sorted<3><<<g, 256, 0, st>>>(rowptr, perm, c, s, d, y, npix);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    const int g = capped_grid(cdiv(npix, 8), 8);   // one pixel per warp
+    return with_pol(pol, [&](auto P) {
+        return launch(k_apply_t_sorted<P>, g, 256, 0, as_stream(stream), rowptr, perm, c, s, d, y, npix);
+    });
 }

@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "../../include/cosmomap2_b200.h"
 
 namespace cm2 {
@@ -34,17 +36,54 @@ int sm_count();
 
 static inline bool aligned(const void *p, size_t a) { return (reinterpret_cast<uintptr_t>(p) % a) == 0; }
 static inline cudaStream_t as_stream(cm2_stream_t s) { return reinterpret_cast<cudaStream_t>(s); }
+static inline int64_t cdiv(int64_t n, int64_t d) { return (n + d - 1) / d; }
+
+// grid of a grid-stride kernel with `ctas` CTAs of work: at least 1, at most per_sm per SM and at most max_ctas
+static inline int capped_grid(int64_t ctas, int per_sm, int64_t max_ctas = INT64_MAX) {
+    int64_t cap = (int64_t)sm_count() * per_sm;
+    if (cap > max_ctas) cap = max_ctas;
+    if (ctas > cap) ctas = cap;
+    return (int)(ctas < 1 ? 1 : ctas);
+}
 
 // grid for a persistent grid-stride kernel: a multiple of the SM count
 template <class Kernel>
 static inline int persistent_grid(Kernel k, int block, size_t smem, int64_t work_blocks, int max_per_sm = 8) {
     int per_sm = 1;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, block, smem);
-    if (per_sm < 1) per_sm = 1;
-    if (per_sm > max_per_sm) per_sm = max_per_sm;
-    int64_t g = (int64_t)sm_count() * per_sm;
-    if (work_blocks < g) g = work_blocks < 1 ? 1 : work_blocks;
-    return (int)g;
+    return capped_grid(work_blocks, per_sm < 1 ? 1 : (per_sm > max_per_sm ? max_per_sm : per_sm));
+}
+
+// f(std::integral_constant<int, P>{}) for P = pol; any pol other than 1 or 2 runs P = 3, so callers check pol first
+template <class F>
+static inline auto with_pol(int pol, F f) {
+    if (pol == 1) return f(std::integral_constant<int, 1>{});
+    if (pol == 2) return f(std::integral_constant<int, 2>{});
+    return f(std::integral_constant<int, 3>{});
+}
+
+// f(std::integral_constant<int, NK>{}) for NK = nk Legendre coefficients; any nk outside 2..4 runs NK = 5
+template <class F>
+static inline auto with_nk(int nk, F f) {
+    switch (nk) {
+        case 2: return f(std::integral_constant<int, 2>{});
+        case 3: return f(std::integral_constant<int, 3>{});
+        case 4: return f(std::integral_constant<int, 4>{});
+        default: return f(std::integral_constant<int, 5>{});
+    }
+}
+
+// one counted kernel launch; returns CM2_OK or the launch error
+template <class... Params, class... Args>
+static inline int launch(void (*kern)(Params...), int grid, int block, size_t smem, cudaStream_t st, Args... args) {
+    kern<<<grid, block, smem, st>>>(args...);
+    CM2_LAUNCHED();
+    return CM2_OK;
+}
+
+// zero fill of n entries of nv 8-byte values (e.g. the map a scatter-add accumulates into)
+static inline cudaError_t zero_fill(void *y, int64_t n, int nv, cudaStream_t st) {
+    return n > 0 ? cudaMemsetAsync(y, 0, sizeof(double) * (size_t)n * nv, st) : cudaSuccess;
 }
 
 // ---- device side: streaming loads/stores (TOD is read once: keep it out of the way of the
@@ -93,6 +132,16 @@ __device__ __forceinline__ void st_stream_d4(double *p, const D4 &v) {
 // scalar tail loads: the .L2::evict_first priority form only exists for the 256-bit vectors
 __device__ __forceinline__ int ld_stream_i1(const int32_t *p) { return __ldcs(p); }
 __device__ __forceinline__ double ld_stream_d1(const double *p) { return __ldcs(p); }
+
+// index of the last entry <= key in the ascending table[0..n), 0 when there is none
+__device__ __forceinline__ int64_t last_le(const int64_t *table, int64_t n, int64_t key) {
+    int64_t lo = 0, hi = n;
+    while (hi - lo > 1) {
+        int64_t mid = (lo + hi) >> 1;
+        if (table[mid] <= key) lo = mid; else hi = mid;
+    }
+    return lo;
+}
 
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll

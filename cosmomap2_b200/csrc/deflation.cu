@@ -143,14 +143,6 @@ __global__ void __launch_bounds__(DB) k_m2_finish(const double *__restrict__ Z, 
     }
 }
 
-static int dgrid(int64_t n, int per_sm = 4) {
-    int64_t b = (n + DB - 1) / DB;
-    int64_t cap = (int64_t)sm_count() * per_sm;
-    if (cap > DG_MAX) cap = DG_MAX;
-    if (b > cap) b = cap;
-    return (int)(b < 1 ? 1 : b);
-}
-
 }  // namespace cm2
 
 using namespace cm2;
@@ -162,7 +154,7 @@ extern "C" int cm2_defl_zt_apply(const double *Z, int64_t n, int r, int64_t ldz,
     CM2_REQUIRE(n >= 0 && r >= 1 && ncols_x >= 1 && ldz >= n, "bad sizes");
     CM2_REQUIRE(work != nullptr, "work (cm2_defl_work_doubles) required");
     cudaStream_t st = as_stream(stream);
-    const int g = dgrid(n, 2);   // 128 regs/thread -> 2 resident CTAs/SM: one wave
+    const int g = capped_grid(cdiv(n, DB), 2, DG_MAX);   // 128 regs/thread -> 2 resident CTAs/SM: one wave
     for (int k = 0; k < ncols_x; ++k) {
         launch_zt_partial(g, st, Z, n, r, ldz, X + (int64_t)k * ldx, work);
         CM2_LAUNCHED();
@@ -176,9 +168,8 @@ extern "C" int cm2_defl_z_apply(const double *Z, int64_t n, int r, int64_t ldz, 
                                 double beta, const double *y0, double *y, cm2_stream_t stream) {
     CM2_REQUIRE(n >= 0 && r >= 1 && ldz >= n, "bad sizes");
     if (n == 0) return CM2_OK;
-    k_z_apply<<<dgrid(n, 8), DB, sizeof(double) * r, as_stream(stream)>>>(Z, n, r, ldz, c, alpha, beta, y0, y);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_z_apply, capped_grid(cdiv(n, DB), 8, DG_MAX), DB, sizeof(double) * r, as_stream(stream), Z, n, r, ldz, c,
+                  alpha, beta, y0, y);
 }
 
 extern "C" int cm2_coarse_apply(const double *Einv, int r, const double *v, double *c, cm2_stream_t stream) {
@@ -295,19 +286,16 @@ extern "C" int cm2_m2_apply(const double *Z, const double *AZ, int64_t n, int r,
     CM2_REQUIRE(pol >= 1 && pol <= 3 && n == npix * pol && r >= 1 && ld >= n, "bad sizes");
     CM2_REQUIRE(work != nullptr, "work (cm2_defl_work_doubles) required");
     cudaStream_t st = as_stream(stream);
-    const int g = dgrid(n, 2);
+    const int g = capped_grid(cdiv(n, DB), 2, DG_MAX);
     double *coef = work + (int64_t)DG_MAX * r;   // r doubles: c = Einv Z^T v
     launch_zt_partial(g, st, Z, n, r, ld, v, work);
     CM2_LAUNCHED();
     k_zt_final<<<1, DB, sizeof(double) * r, st>>>(work, g, r, Einv, nullptr, coef);
     CM2_LAUNCHED();
-    const int g2 = dgrid(npix, 8);
-    const size_t sm = sizeof(double) * r;
-    if (pol == 1) k_m2_finish<1><<<g2, DB, sm, st>>>(Z, AZ, r, ld, coef, bd_inv, npix, v, y);
-    else if (pol == 2) k_m2_finish<2><<<g2, DB, sm, st>>>(Z, AZ, r, ld, coef, bd_inv, npix, v, y);
-    else k_m2_finish<3><<<g2, DB, sm, st>>>(Z, AZ, r, ld, coef, bd_inv, npix, v, y);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    const int g2 = capped_grid(cdiv(npix, DB), 8, DG_MAX);
+    return with_pol(pol, [&](auto P) {
+        return launch(k_m2_finish<P>, g2, DB, sizeof(double) * r, st, Z, AZ, r, ld, coef, bd_inv, npix, v, y);
+    });
 }
 
 
@@ -320,15 +308,14 @@ extern "C" int cm2_m2_banded_apply(const int32_t *band, const double *azb, int r
     CM2_REQUIRE(work != nullptr && band != nullptr && azb != nullptr, "NULL argument");
     if (npix == 0) return CM2_OK;
     cudaStream_t st = as_stream(stream);
-    int g = dgrid(npix, 2);
-    if (g > DG_MAX) g = DG_MAX;
+    const int g = capped_grid(cdiv(npix, DB), 2, DG_MAX);
     double *coef = work + (int64_t)DG_MAX * r;
     if (pol == 1) k_band_sums<1><<<g, DB, 0, st>>>(band, npix, r, v, work);
     else k_band_sums<3><<<g, DB, 0, st>>>(band, npix, r, v, work);
     CM2_LAUNCHED();
     k_zt_final<<<1, DB, sizeof(double) * r, st>>>(work, g, r, Einv, nullptr, coef);
     CM2_LAUNCHED();
-    const int g2 = dgrid(npix, 8);
+    const int g2 = capped_grid(cdiv(npix, DB), 8, DG_MAX);
     const size_t sm = sizeof(double) * r;
     if (pol == 1) k_m2_banded_finish<1><<<g2, DB, sm, st>>>(band, azb, r, coef, bd_inv, npix, v, y);
     else k_m2_banded_finish<3><<<g2, DB, sm, st>>>(band, azb, r, coef, bd_inv, npix, v, y);

@@ -190,10 +190,8 @@ static int launch_combine(const double *V, int64_t ldv, int64_t n, int m, const 
     if (smem > 200 * 1024) return set_error(CM2_ERR_UNSUPPORTED, "cm2_dense_combine: m = %d is too large for one panel", m);
     CM2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int64_t tiles = (n + 31) / 32;
-    const int grid = persistent_grid(kern, CB_THREADS, smem, (tiles + 7) / 8, 4);
-    kern<<<grid, CB_THREADS, smem, st>>>(V, ldv, n, m, U, ldu, r, Z, ldz, mpad, vec);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(kern, persistent_grid(kern, CB_THREADS, smem, (tiles + 7) / 8, 4), CB_THREADS, smem, st, V, ldv, n, m, U,
+                  ldu, r, Z, ldz, mpad, vec);
 }
 
 }  // namespace cm2
@@ -210,17 +208,13 @@ extern "C" int cm2_dense_gram(const double *X, int64_t ldx, int r1, const double
     CM2_REQUIRE(work != nullptr, "work (cm2_dense_gram_work_doubles) required");
     cudaStream_t st = as_stream(stream);
     const bool vec = aligned(X, 32) && aligned(Y, 32) && (ldx % 4 == 0) && (ldy % 4 == 0);
-    const int64_t chunks = (n + 15) / 16;
-    int64_t grid = (chunks + 3) / 4;
-    const int64_t cap = (int64_t)sm_count() * 4 < GR_MAXCTA ? (int64_t)sm_count() * 4 : GR_MAXCTA;
-    if (grid > cap) grid = cap;
-    if (grid < 1) grid = 1;
+    const int grid = capped_grid(cdiv(cdiv(n, 16), 4), 4, GR_MAXCTA);
     for (int i0 = 0; i0 < r1; i0 += 32) {
         for (int j0 = 0; j0 < r2; j0 += 32) {
             const int p1 = r1 - i0 < 32 ? r1 - i0 : 32, p2 = r2 - j0 < 32 ? r2 - j0 : 32;
             const int mb = blocks_for(p1), nb = blocks_for(p2);
             const double *Xp = X + (int64_t)i0 * ldx, *Yp = Y + (int64_t)j0 * ldy;
-#define CM2_GRAM(MB, NB) launch_gram<MB, NB>((int)grid, st, Xp, ldx, p1, Yp, ldy, p2, n, vec, work)
+#define CM2_GRAM(MB, NB) launch_gram<MB, NB>(grid, st, Xp, ldx, p1, Yp, ldy, p2, n, vec, work)
             if (mb == 1 && nb == 1) CM2_GRAM(1, 1);
             else if (mb == 1 && nb == 2) CM2_GRAM(1, 2);
             else if (mb == 1 && nb == 4) CM2_GRAM(1, 4);
@@ -232,7 +226,7 @@ extern "C" int cm2_dense_gram(const double *X, int64_t ldx, int r1, const double
             else CM2_GRAM(4, 4);
 #undef CM2_GRAM
             CM2_LAUNCHED();
-            k_gram_final<<<4, 256, 0, st>>>(work, (int)grid, 8 * mb, mb * nb * 64, p1, p2, out + i0 + ldo * (int64_t)j0, ldo);
+            k_gram_final<<<4, 256, 0, st>>>(work, grid, 8 * mb, mb * nb * 64, p1, p2, out + i0 + ldo * (int64_t)j0, ldo);
             CM2_LAUNCHED();
         }
     }

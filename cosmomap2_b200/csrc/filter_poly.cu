@@ -362,11 +362,8 @@ static int launch_filter_poly(const int32_t *pix, const int64_t *seg_start, cons
         const size_t smem = (size_t)capw * 12 * nstage;
         auto kern = k_filter_poly_tma<NK, OFFSET>;
         CM2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        int grid = sm_count();
-        if (nseg < grid) grid = (int)nseg;
-        kern<<<grid, TB, smem, st>>>(pix, seg_start, seg_end, nseg, d, out, nt, (int)capw, nstage, fill);
-        CM2_LAUNCHED();
-        return CM2_OK;
+        return launch(kern, capped_grid(nseg, 1), TB, smem, st, pix, seg_start, seg_end, nseg, d, out, nt, (int)capw, nstage,
+                      fill);
     }
     // variant A: shared-memory window of the longest subscan, up to 24 000 samples (216 kB); longer
     // subscans re-read their tail from global memory (L2)
@@ -377,9 +374,8 @@ static int launch_filter_poly(const int32_t *pix, const int64_t *seg_start, cons
     const size_t smem = (size_t)cap * 9;
     auto kern = k_filter_poly<NK, OFFSET>;
     CM2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<persistent_grid(kern, FB, smem, nseg), FB, smem, st>>>(pix, seg_start, seg_end, nseg, d, out, nt, cap, fill);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(kern, persistent_grid(kern, FB, smem, nseg), FB, smem, st, pix, seg_start, seg_end, nseg, d, out, nt, cap,
+                  fill);
 }
 
 // ---- ground-template filter: out = v - bins[g] / hits[g] ---------------------------------------
@@ -427,12 +423,6 @@ __global__ void __launch_bounds__(FB) k_reorganize(const double *__restrict__ ma
     }
 }
 
-static int grid_fp(int64_t blocks, int per_sm = 8) {
-    int64_t capb = (int64_t)sm_count() * per_sm;
-    if (blocks > capb) blocks = capb;
-    return (int)(blocks < 1 ? 1 : blocks);
-}
-
 }  // namespace cm2
 
 using namespace cm2;
@@ -451,7 +441,7 @@ extern "C" int cm2_filter_poly_apply(const int32_t *pix, const int64_t *seg_star
         return set_error(CM2_ERR_UNSUPPORTED, "poly_order=%d: orders 0..%d are supported", poly_order, FP_MAXNK - 1);
     cudaStream_t st = as_stream(stream);
     const int fill = sorted && nseg > 0;
-    if (nt > 0 && !fill) CM2_CUDA(cudaMemsetAsync(out, 0, sizeof(double) * (size_t)nt, st));
+    if (!fill) CM2_CUDA(zero_fill(out, nt, 1, st));
     if (nt == 0 || nseg == 0) return CM2_OK;
     const int tma = g_filter_tma;
 #define CM2_FP(NKv, OFFv) launch_filter_poly<NKv, OFFv>(pix, seg_start, seg_end, nseg, max_seg_len, d, out, nt, fill, tma, st)
@@ -480,9 +470,8 @@ extern "C" int cm2_ground_filter_sub(const int32_t *ground, int64_t nt, int64_t 
     CM2_REQUIRE(nt >= 0 && nbins >= 0, "bad sizes");
     CM2_REQUIRE(aligned(ground, 32) && aligned(v, 32) && aligned(out, 32), "TOD vectors must be 32-byte aligned");
     if (nt == 0) return CM2_OK;
-    k_ground_sub<<<grid_fp(((nt + 3) / 4 + FB - 1) / FB), FB, 0, as_stream(stream)>>>(ground, bins, hits, v, out, nt);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_ground_sub, capped_grid(cdiv(cdiv(nt, 4), FB), 8), FB, 0, as_stream(stream), ground, bins, hits, v, out,
+                  nt);
 }
 
 extern "C" int cm2_ground_filter_apply(const int32_t *ground, int64_t nt, int64_t nbins, const int64_t *hits,
@@ -499,9 +488,7 @@ extern "C" int cm2_reorganize_map(const double *map, const int64_t *obspix, int6
     CM2_REQUIRE(npix >= 0 && healpix_npix >= 0, "bad sizes");
     CM2_REQUIRE(pol >= 1 && pol <= 3, "pol must be 1, 2 or 3");
     cudaStream_t st = as_stream(stream);
-    if (healpix_npix > 0) CM2_CUDA(cudaMemsetAsync(out, 0, sizeof(double) * (size_t)healpix_npix * pol, st));
+    CM2_CUDA(zero_fill(out, healpix_npix, pol, st));
     if (npix == 0 || healpix_npix == 0) return CM2_OK;
-    k_reorganize<<<grid_fp((npix + FB - 1) / FB), FB, 0, st>>>(map, obspix, npix, pol, healpix_npix, out);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_reorganize, capped_grid(cdiv(npix, FB), 8), FB, 0, st, map, obspix, npix, pol, healpix_npix, out);
 }

@@ -264,11 +264,6 @@ __global__ void __launch_bounds__(FB) k_poly_seg_coef(const int32_t *__restrict_
     }
 }
 
-static int fgrid(int64_t n) {
-    int64_t cap = (int64_t)sm_count() * 8;
-    return (int)(n < 1 ? 1 : (n < cap ? n : cap));
-}
-
 }  // namespace cm2
 
 using namespace cm2;
@@ -282,9 +277,7 @@ extern "C" int cm2_filter_runs_mark(const int32_t *pix, const int64_t *seg_start
         CM2_CUDA(cudaMemsetAsync(pix_masked, 0xff, sizeof(int32_t) * (size_t)nt, st));   // -1 everywhere
     }
     if (nt == 0 || nseg == 0) return CM2_OK;
-    k_runs_mark<<<fgrid(nseg), FB, 0, st>>>(pix, seg_start, seg_end, nseg, flags, pix_masked);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_runs_mark, capped_grid(nseg, 8), FB, 0, st, pix, seg_start, seg_end, nseg, flags, pix_masked);
 }
 
 extern "C" int cm2_filter_runs_fill(const int32_t *pix, const double *c, const double *s, int pol,
@@ -293,10 +286,8 @@ extern "C" int cm2_filter_runs_fill(const int32_t *pix, const double *c, const d
                                     int32_t *seg_nruns, cm2_stream_t stream) {
     CM2_REQUIRE(nseg >= 0 && pol >= 1 && pol <= 3, "bad sizes");
     if (nseg == 0) return CM2_OK;
-    k_runs_fill<<<fgrid(nseg), FB, 0, as_stream(stream)>>>(pix, c, s, pol, seg_start, seg_end, nseg, runidx, run_pix, run_mom,
-                                                         seg_first, seg_nruns);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_runs_fill, capped_grid(nseg, 8), FB, 0, as_stream(stream), pix, c, s, pol, seg_start, seg_end, nseg,
+                  runidx, run_pix, run_mom, seg_first, seg_nruns);
 }
 
 extern "C" int cm2_filter_seg_mean(const int32_t *run_pix, const double *run_mom, const int64_t *seg_first,
@@ -304,12 +295,10 @@ extern "C" int cm2_filter_seg_mean(const int32_t *run_pix, const double *run_mom
                                    cm2_stream_t stream) {
     CM2_REQUIRE(nseg >= 0 && pol >= 1 && pol <= 3, "bad sizes");
     if (nseg == 0) return CM2_OK;
-    cudaStream_t st = as_stream(stream);
-    if (pol == 1) k_seg_mean<1><<<fgrid(nseg), FB, 0, st>>>(run_pix, run_mom, seg_first, seg_nruns, nseg, x, mu);
-    else if (pol == 2) k_seg_mean<2><<<fgrid(nseg), FB, 0, st>>>(run_pix, run_mom, seg_first, seg_nruns, nseg, x, mu);
-    else k_seg_mean<3><<<fgrid(nseg), FB, 0, st>>>(run_pix, run_mom, seg_first, seg_nruns, nseg, x, mu);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    const int g = capped_grid(nseg, 8);
+    return with_pol(pol, [&](auto P) {
+        return launch(k_seg_mean<P>, g, FB, 0, as_stream(stream), run_pix, run_mom, seg_first, seg_nruns, nseg, x, mu);
+    });
 }
 
 /* ---- Legendre variant of the run table (poly_order 1..4) --------------------------------------- */
@@ -319,16 +308,10 @@ extern "C" int cm2_filter_poly_gram(const int32_t *pix, const int64_t *seg_start
     if (poly_order < 1 || poly_order > 4)
         return set_error(CM2_ERR_UNSUPPORTED, "run-table Legendre filter: poly_order=%d, orders 1..4 are supported", poly_order);
     if (nseg == 0) return CM2_OK;
-    cudaStream_t st = as_stream(stream);
-    const int g = fgrid(nseg);
-    switch (poly_order) {
-        case 1: k_poly_gram<2><<<g, FB, 0, st>>>(pix, seg_start, seg_end, nseg, W, info); break;
-        case 2: k_poly_gram<3><<<g, FB, 0, st>>>(pix, seg_start, seg_end, nseg, W, info); break;
-        case 3: k_poly_gram<4><<<g, FB, 0, st>>>(pix, seg_start, seg_end, nseg, W, info); break;
-        default: k_poly_gram<5><<<g, FB, 0, st>>>(pix, seg_start, seg_end, nseg, W, info); break;
-    }
-    CM2_LAUNCHED();
-    return CM2_OK;
+    const int g = capped_grid(nseg, 8);
+    return with_nk(poly_order + 1, [&](auto NK) {
+        return launch(k_poly_gram<NK>, g, FB, 0, as_stream(stream), pix, seg_start, seg_end, nseg, W, info);
+    });
 }
 
 extern "C" int cm2_filter_poly_runs_fill(const int32_t *pix, const double *c, const double *s, int pol,
@@ -339,30 +322,11 @@ extern "C" int cm2_filter_poly_runs_fill(const int32_t *pix, const double *c, co
     if (poly_order < 1 || poly_order > 4)
         return set_error(CM2_ERR_UNSUPPORTED, "run-table Legendre filter: poly_order=%d, orders 1..4 are supported", poly_order);
     if (nseg == 0) return CM2_OK;
-    cudaStream_t st = as_stream(stream);
-    const int g = fgrid(nseg);
-#define CM2_FILL(NK) k_poly_runs_fill<NK><<<g, FB, 0, st>>>(pix, c, s, pol, seg_start, seg_end, nseg, runidx, run_pix, run_mom, seg_first, seg_nruns)
-    switch (poly_order) {
-        case 1: CM2_FILL(2); break;
-        case 2: CM2_FILL(3); break;
-        case 3: CM2_FILL(4); break;
-        default: CM2_FILL(5); break;
-    }
-#undef CM2_FILL
-    CM2_LAUNCHED();
-    return CM2_OK;
-}
-
-template <int POL>
-static void launch_poly_seg_coef(int nk, int g, cudaStream_t st, const int32_t *run_pix, const double *run_mom,
-                                 const int64_t *seg_first, const int32_t *seg_nruns, int64_t nseg, const double *W,
-                                 const double *x, double *coef) {
-    switch (nk) {
-        case 2: k_poly_seg_coef<POL, 2><<<g, FB, 0, st>>>(run_pix, run_mom, seg_first, seg_nruns, nseg, W, x, coef); break;
-        case 3: k_poly_seg_coef<POL, 3><<<g, FB, 0, st>>>(run_pix, run_mom, seg_first, seg_nruns, nseg, W, x, coef); break;
-        case 4: k_poly_seg_coef<POL, 4><<<g, FB, 0, st>>>(run_pix, run_mom, seg_first, seg_nruns, nseg, W, x, coef); break;
-        default: k_poly_seg_coef<POL, 5><<<g, FB, 0, st>>>(run_pix, run_mom, seg_first, seg_nruns, nseg, W, x, coef); break;
-    }
+    const int g = capped_grid(nseg, 8);
+    return with_nk(poly_order + 1, [&](auto NK) {
+        return launch(k_poly_runs_fill<NK>, g, FB, 0, as_stream(stream), pix, c, s, pol, seg_start, seg_end, nseg, runidx,
+                      run_pix, run_mom, seg_first, seg_nruns);
+    });
 }
 
 extern "C" int cm2_filter_poly_seg_coef(const int32_t *run_pix, const double *run_mom, const int64_t *seg_first,
@@ -372,11 +336,11 @@ extern "C" int cm2_filter_poly_seg_coef(const int32_t *run_pix, const double *ru
     if (poly_order < 1 || poly_order > 4)
         return set_error(CM2_ERR_UNSUPPORTED, "run-table Legendre filter: poly_order=%d, orders 1..4 are supported", poly_order);
     if (nseg == 0) return CM2_OK;
-    cudaStream_t st = as_stream(stream);
-    const int g = fgrid(nseg), nk = poly_order + 1;
-    if (pol == 1) launch_poly_seg_coef<1>(nk, g, st, run_pix, run_mom, seg_first, seg_nruns, nseg, W, x, coef);
-    else if (pol == 2) launch_poly_seg_coef<2>(nk, g, st, run_pix, run_mom, seg_first, seg_nruns, nseg, W, x, coef);
-    else launch_poly_seg_coef<3>(nk, g, st, run_pix, run_mom, seg_first, seg_nruns, nseg, W, x, coef);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    const int g = capped_grid(nseg, 8);
+    return with_pol(pol, [&](auto P) {
+        return with_nk(poly_order + 1, [&](auto NK) {
+            return launch(k_poly_seg_coef<P, NK>, g, FB, 0, as_stream(stream), run_pix, run_mom, seg_first, seg_nruns, nseg,
+                          W, x, coef);
+        });
+    });
 }

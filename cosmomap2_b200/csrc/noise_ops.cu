@@ -14,12 +14,7 @@ __device__ __forceinline__ int64_t find_block(const int64_t *__restrict__ start,
         int64_t b = t / blocksize;
         return b < nblocks ? b : nblocks - 1;
     }
-    int64_t lo = 0, hi = nblocks;
-    while (hi - lo > 1) {
-        int64_t mid = (lo + hi) >> 1;
-        if (start[mid] <= t) lo = mid; else hi = mid;
-    }
-    return lo;
+    return last_le(start, nblocks, t);
 }
 
 // each thread: 4 consecutive samples (256-bit load/store); the block index is looked up once
@@ -65,12 +60,7 @@ __global__ void __launch_bounds__(NB) k_toeplitz(const double *__restrict__ band
     const int64_t ntiles = tile_first[nblocks];
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         // tile -> (block b, offset within block): tile_first[b] = first tile index of block b
-        int64_t lo = 0, hi = nblocks;
-        while (hi - lo > 1) {
-            int64_t mid = (lo + hi) >> 1;
-            if (tile_first[mid] <= tile) lo = mid; else hi = mid;
-        }
-        const int64_t b = lo;
+        const int64_t b = last_le(tile_first, nblocks, tile);
         const int64_t bs = start ? start[b] : b * blocksize;
         const int64_t be = start ? start[b + 1] : (b + 1 == nblocks ? nt : (b + 1) * blocksize);
         const int64_t j0 = bs + (tile - tile_first[b]) * TT;   // first output of this tile (global index)
@@ -156,12 +146,6 @@ __global__ void __launch_bounds__(NB) k_filter_offset(const int32_t *__restrict_
     }
 }
 
-static int grid_for(int64_t blocks, int per_sm = 8) {
-    int64_t cap = (int64_t)sm_count() * per_sm;
-    if (blocks > cap) blocks = cap;
-    return (int)(blocks < 1 ? 1 : blocks);
-}
-
 }  // namespace cm2
 
 using namespace cm2;
@@ -172,9 +156,8 @@ extern "C" int cm2_noise_white_apply(const double *wblk, int64_t nblocks, int64_
     CM2_REQUIRE(blk_start != nullptr || blocksize > 0, "blocksize must be > 0");
     CM2_REQUIRE(aligned(d, 32) && aligned(out, 32), "TOD vectors must be 32-byte aligned");
     if (nt == 0) return CM2_OK;
-    k_white<<<grid_for(((nt + 3) / 4 + NB - 1) / NB), NB, 0, as_stream(stream)>>>(wblk, nblocks, blocksize, blk_start, d, out, nt);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_white, capped_grid(cdiv(cdiv(nt, 4), NB), 8), NB, 0, as_stream(stream), wblk, nblocks, blocksize,
+                  blk_start, d, out, nt);
 }
 
 extern "C" int64_t cm2_toeplitz_scratch_bytes(int64_t nblocks) { return (nblocks + 1) * (int64_t)sizeof(int64_t); }
@@ -196,14 +179,10 @@ extern "C" int cm2_noise_toeplitz_apply(const double *band, int nband, int64_t n
     k_tile_first<<<1, 1, 0, st>>>(nblocks, blocksize, blk_start, nt, tile_first);
     CM2_LAUNCHED();
     // upper bound of the tile count without reading the device prefix back
-    int64_t ntiles_ub = nt / TT + nblocks + 1;
-    int per_sm = 1;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_toeplitz, NB, smem);
-    if (per_sm < 1) per_sm = 1;
-    // the exact tile count is tile_first[nblocks], read on the device
-    k_toeplitz<<<grid_for(ntiles_ub, per_sm), NB, smem, st>>>(band, nband, nblocks, blocksize, blk_start, tile_first, d, out, nt);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    const int64_t ntiles_ub = nt / TT + nblocks + 1;
+    // the exact tile count is tile_first[nblocks], read on the device; at NB threads no more than 8 CTAs fit on an SM
+    return launch(k_toeplitz, persistent_grid(k_toeplitz, NB, smem, ntiles_ub), NB, smem, st, band, nband, nblocks,
+                  blocksize, blk_start, tile_first, d, out, nt);
 }
 
 extern "C" int cm2_filter_offset_apply(const int32_t *pix, const int64_t *seg_start, const int64_t *seg_end, int64_t nseg,
@@ -211,9 +190,7 @@ extern "C" int cm2_filter_offset_apply(const int32_t *pix, const int64_t *seg_st
     CM2_REQUIRE(nt >= 0 && nseg >= 0, "bad sizes");
     CM2_REQUIRE(d != out, "in-place filtering is not supported");
     cudaStream_t st = as_stream(stream);
-    if (nt > 0) CM2_CUDA(cudaMemsetAsync(out, 0, sizeof(double) * (size_t)nt, st));
+    CM2_CUDA(zero_fill(out, nt, 1, st));
     if (nt == 0 || nseg == 0) return CM2_OK;
-    k_filter_offset<<<grid_for(nseg), NB, 0, st>>>(pix, seg_start, seg_end, nseg, d, out);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_filter_offset, capped_grid(nseg, 8), NB, 0, st, pix, seg_start, seg_end, nseg, d, out);
 }

@@ -156,10 +156,7 @@ extern "C" int cm2_allreduce_p2p(const void *const *send_ptrs_host, void *const 
         P.sig[g] = g < world ? reinterpret_cast<ARSignals *>(signal_ptrs_host[g]) : nullptr;
         if (g < world) CM2_REQUIRE(aligned(P.send[g], 16) && aligned(P.recv[g], 16), "buffers must be 16-byte aligned");
     }
-    int64_t slice2 = (n / 2 + world - 1) / world;
-    int64_t blocks = (slice2 + AR_THREADS - 1) / AR_THREADS;
-    int cap = sm_count() < AR_MAX_BLOCKS ? sm_count() : AR_MAX_BLOCKS;
-    int grid = (int)(blocks < 1 ? 1 : (blocks > cap ? cap : blocks));
+    const int grid = capped_grid(cdiv(cdiv(n / 2, world), AR_THREADS), 1, AR_MAX_BLOCKS);
     // every rank must launch the SAME grid (per-CTA barriers): it depends only on n and world
     cudaStream_t st = as_stream(stream);
     switch (world) {

@@ -402,12 +402,5 @@ extern "C" int cm2_pcg_bd_sharded(int reset, int pol, int world, int rank0, int 
     a.rtol = rtol;
     a.timeout_ns = (long long)(timeout_s * 1e9);
     cudaStream_t st = as_stream(stream);
-    if (reset) {
-        if (pol == 1) return launch_sharded<1, true>(a, st);
-        if (pol == 2) return launch_sharded<2, true>(a, st);
-        return launch_sharded<3, true>(a, st);
-    }
-    if (pol == 1) return launch_sharded<1, false>(a, st);
-    if (pol == 2) return launch_sharded<2, false>(a, st);
-    return launch_sharded<3, false>(a, st);
+    return with_pol(pol, [&](auto P) { return reset ? launch_sharded<P, true>(a, st) : launch_sharded<P, false>(a, st); });
 }

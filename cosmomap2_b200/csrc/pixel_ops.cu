@@ -71,13 +71,7 @@ __global__ void __launch_bounds__(PB) k_moments_sorted(const int64_t *__restrict
             double w = 1.0;
             if (wsamp) w = wsamp[t];
             else if (wblk) {
-                int64_t b;
-                if (bstart == nullptr) b = t / blocksize;
-                else {
-                    int64_t lo = 0, hi = nblocks;
-                    while (hi - lo > 1) { int64_t mid = (lo + hi) >> 1; if (bstart[mid] <= t) lo = mid; else hi = mid; }
-                    b = lo;
-                }
+                const int64_t b = bstart == nullptr ? t / blocksize : last_le(bstart, nblocks, t);
                 w = wblk[b < nblocks ? b : nblocks - 1];
             }
             if (pol == 1) { h = __dadd_rn(h, w); continue; }
@@ -254,13 +248,6 @@ __global__ void __launch_bounds__(PB) k_block_apply(const double *__restrict__ b
     }
 }
 
-static int grid_for(int64_t n) {
-    int64_t b = (n + PB - 1) / PB;
-    int64_t cap = (int64_t)sm_count() * 8;
-    if (b > cap) b = cap;
-    return (int)(b < 1 ? 1 : b);
-}
-
 }  // namespace cm2
 
 using namespace cm2;
@@ -268,34 +255,26 @@ using namespace cm2;
 extern "C" int cm2_angles(const double *phi, int64_t nt, double *c, double *s, cm2_stream_t stream) {
     CM2_REQUIRE(nt >= 0, "nt < 0");
     if (nt == 0) return CM2_OK;
-    k_angles<<<grid_for(nt), PB, 0, as_stream(stream)>>>(phi, nt, c, s);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_angles, capped_grid(cdiv(nt, PB), 8), PB, 0, as_stream(stream), phi, nt, c, s);
 }
 
 extern "C" int cm2_pix_narrow(const int64_t *pix64, int64_t nt, int32_t *pix32, cm2_stream_t stream) {
     CM2_REQUIRE(nt >= 0, "nt < 0");
     if (nt == 0) return CM2_OK;
-    k_narrow<<<grid_for(nt), PB, 0, as_stream(stream)>>>(pix64, nt, pix32);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_narrow, capped_grid(cdiv(nt, PB), 8), PB, 0, as_stream(stream), pix64, nt, pix32);
 }
 
 extern "C" int cm2_pix_widen(const int32_t *pix32, int64_t nt, int64_t *pix64, cm2_stream_t stream) {
     CM2_REQUIRE(nt >= 0, "nt < 0");
     if (nt == 0) return CM2_OK;
-    k_widen<<<grid_for(nt), PB, 0, as_stream(stream)>>>(pix32, nt, pix64);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_widen, capped_grid(cdiv(nt, PB), 8), PB, 0, as_stream(stream), pix32, nt, pix64);
 }
 
 extern "C" int cm2_weights_mask(const double *mom, int64_t npix, int pol, double threshold_cond, int32_t *good,
                                 cm2_stream_t stream) {
     CM2_REQUIRE(npix >= 0 && pol >= 1 && pol <= 3, "bad npix/pol");
     if (npix == 0) return CM2_OK;
-    k_mask<<<grid_for(npix), PB, 0, as_stream(stream)>>>(mom, npix, pol, threshold_cond, good);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_mask, capped_grid(cdiv(npix, PB), 8), PB, 0, as_stream(stream), mom, npix, pol, threshold_cond, good);
 }
 
 extern "C" int cm2_weights_moments_sorted(const int64_t *rowptr, const int32_t *perm, const double *c, const double *s,
@@ -305,10 +284,8 @@ extern "C" int cm2_weights_moments_sorted(const int64_t *rowptr, const int32_t *
     CM2_REQUIRE(npix >= 0 && pol >= 1 && pol <= 3, "bad npix/pol");
     CM2_REQUIRE(wblk == nullptr || nblocks > 0, "nblocks must be > 0 when block weights are given");
     if (npix == 0) return CM2_OK;
-    k_moments_sorted<<<grid_for(npix), PB, 0, as_stream(stream)>>>(rowptr, perm, c, s, w, wblk, nblocks, blocksize, blk_start,
-                                                                 pol, mom, npix);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_moments_sorted, capped_grid(cdiv(npix, PB), 8), PB, 0, as_stream(stream), rowptr, perm, c, s, w, wblk,
+                  nblocks, blocksize, blk_start, pol, mom, npix);
 }
 
 extern "C" int64_t cm2_scan_scratch_bytes(int64_t n) {
@@ -340,46 +317,36 @@ extern "C" int cm2_compact_rows_f64(const double *src, const int32_t *old2new, i
                                     cm2_stream_t stream) {
     CM2_REQUIRE(npix >= 0 && width > 0, "bad npix/width");
     if (npix == 0) return CM2_OK;
-    k_compact_rows<double><<<grid_for(npix * width), PB, 0, as_stream(stream)>>>(src, old2new, npix, width, dst);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_compact_rows<double>, capped_grid(cdiv(npix * width, PB), 8), PB, 0, as_stream(stream), src, old2new,
+                  npix, width, dst);
 }
 
 extern "C" int cm2_compact_rows_i64(const int64_t *src, const int32_t *old2new, int64_t npix, int width, int64_t *dst,
                                     cm2_stream_t stream) {
     CM2_REQUIRE(npix >= 0 && width > 0, "bad npix/width");
     if (npix == 0) return CM2_OK;
-    k_compact_rows<int64_t><<<grid_for(npix * width), PB, 0, as_stream(stream)>>>(src, old2new, npix, width, dst);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_compact_rows<int64_t>, capped_grid(cdiv(npix * width, PB), 8), PB, 0, as_stream(stream), src, old2new,
+                  npix, width, dst);
 }
 
 extern "C" int cm2_relabel(int32_t *pix, int64_t nt, const int32_t *old2new, cm2_stream_t stream) {
     CM2_REQUIRE(nt >= 0, "nt < 0");
     if (nt == 0) return CM2_OK;
-    k_relabel<<<grid_for(nt), PB, 0, as_stream(stream)>>>(pix, nt, old2new);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_relabel, capped_grid(cdiv(nt, PB), 8), PB, 0, as_stream(stream), pix, nt, old2new);
 }
 
 extern "C" int cm2_bd_build(const double *mom, int64_t npix, int pol, double *inv, cm2_stream_t stream) {
     CM2_REQUIRE(npix >= 0 && pol >= 1 && pol <= 3, "bad npix/pol");
     if (npix == 0) return CM2_OK;
-    k_bd_build<<<grid_for(npix), PB, 0, as_stream(stream)>>>(mom, npix, pol, inv);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_bd_build, capped_grid(cdiv(npix, PB), 8), PB, 0, as_stream(stream), mom, npix, pol, inv);
 }
 
 static int block_apply(const double *blk, int64_t npix, int pol, const double *x, double *y, cm2_stream_t stream) {
     if (npix < 0 || pol < 1 || pol > 3) return set_error(CM2_ERR_ARG, "bad npix/pol");
     if (!aligned(blk, 16)) return set_error(CM2_ERR_ARG, "block coefficients must be 16-byte aligned");
     if (npix == 0) return CM2_OK;
-    cudaStream_t st = as_stream(stream);
-    if (pol == 1) k_block_apply<1><<<grid_for(npix), PB, 0, st>>>(blk, npix, x, y);
-    else if (pol == 2) k_block_apply<2><<<grid_for(npix), PB, 0, st>>>(blk, npix, x, y);
-    else k_block_apply<3><<<grid_for(npix), PB, 0, st>>>(blk, npix, x, y);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    const int g = capped_grid(cdiv(npix, PB), 8);
+    return with_pol(pol, [&](auto P) { return launch(k_block_apply<P>, g, PB, 0, as_stream(stream), blk, npix, x, y); });
 }
 
 extern "C" int cm2_bd_apply(const double *inv, int64_t npix, int pol, const double *x, double *y, cm2_stream_t stream) {

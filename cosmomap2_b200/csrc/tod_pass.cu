@@ -47,12 +47,7 @@ __device__ __forceinline__ int64_t block_of(const BlockW &bw, int64_t t) {
         if (bw.magic != 0 && ((uint64_t)t >> 32) == 0) return (int64_t)__umul64hi((uint64_t)t, bw.magic);
         return t / bw.blocksize;
     }
-    int64_t lo = 0, hi = bw.nblocks;
-    while (hi - lo > 1) {
-        int64_t mid = (lo + hi) >> 1;
-        if (bw.start[mid] <= t) lo = mid; else hi = mid;
-    }
-    return lo;
+    return last_le(bw.start, bw.nblocks, t);
 }
 
 // weights of the K samples starting at t0 (one lookup when the chunk sits inside one block)
@@ -1301,14 +1296,6 @@ __global__ void __launch_bounds__(BLOCK, 2) k_amatvec_filter_poly(const int32_t 
     }
 }
 
-// f(std::integral_constant<int, P>{}) for P = pol (check_tod has limited pol to 1..3)
-template <class F>
-static int with_pol(int pol, F f) {
-    if (pol == 1) return f(std::integral_constant<int, 1>{});
-    if (pol == 2) return f(std::integral_constant<int, 2>{});
-    return f(std::integral_constant<int, 3>{});
-}
-
 // CTAs of BLOCK / 32 warp tiles that cover nt samples, `tile` of them per warp tile
 static int64_t tod_blocks(int64_t nt, int64_t tile = TILE) {
     const int64_t ntiles = (nt + tile - 1) / tile;
@@ -1319,27 +1306,7 @@ static int64_t tod_blocks(int64_t nt, int64_t tile = TILE) {
 template <class... Params, class... Args>
 static int launch_tod(void (*kern)(Params...), int64_t blocks, size_t smem, cudaStream_t st, Args... args) {
     if (smem > 0) CM2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<persistent_grid(kern, BLOCK, smem, blocks), BLOCK, smem, st>>>(args...);
-    CM2_LAUNCHED();
-    return CM2_OK;
-}
-
-// zero fill of n entries of nv 8-byte values (the map a scatter-add accumulates into)
-static cudaError_t zero_fill(void *y, int64_t n, int nv, cudaStream_t st) {
-    return n > 0 ? cudaMemsetAsync(y, 0, sizeof(double) * (size_t)n * nv, st) : cudaSuccess;
-}
-
-template <int POL>
-static int dispatch_amatvec_filter_poly(int nk, const int32_t *pix, const double *c, const double *s, int64_t nt,
-                                        const int64_t *seg_start, const int64_t *seg_end, int64_t nseg, const double *x,
-                                        double *y, int cap, cudaStream_t st) {
-    const size_t smem = (size_t)cap * 12;
-    switch (nk) {
-        case 2: return launch_tod(k_amatvec_filter_poly<POL, 2>, nseg, smem, st, pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap);
-        case 3: return launch_tod(k_amatvec_filter_poly<POL, 3>, nseg, smem, st, pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap);
-        case 4: return launch_tod(k_amatvec_filter_poly<POL, 4>, nseg, smem, st, pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap);
-        default: return launch_tod(k_amatvec_filter_poly<POL, 5>, nseg, smem, st, pix, c, s, nt, seg_start, seg_end, nseg, x, y, cap);
-    }
+    return launch(kern, persistent_grid(kern, BLOCK, smem, blocks), BLOCK, smem, st, args...);
 }
 
 static int check_tod(const void *pix, const void *c, const void *s, int64_t nt, int pol) {
@@ -1557,18 +1524,6 @@ extern "C" int cm2_pointing_filter_mu(const int32_t *pix, const double *c, const
     return with_pol(pol, [&](auto P) { return launch_tod(k_pointing_filter_mu<P>, tod_blocks(nt), 0, st, pix, c, s, nt, sg, x, d); });
 }
 
-template <int POL>
-static int dispatch_amatvec_filter_poly_mu(int nk, const int32_t *pix, const double *c, const double *s, int64_t nt,
-                                           const SegPoly &sg, const TileOrder &ord, const double *x, double *y, cudaStream_t st) {
-    const int64_t blocks = tod_blocks(nt);
-    switch (nk) {
-        case 2: return launch_tod(k_amatvec_filter_poly_mu<POL, 2>, blocks, 0, st, pix, c, s, nt, sg, ord, x, y);
-        case 3: return launch_tod(k_amatvec_filter_poly_mu<POL, 3>, blocks, 0, st, pix, c, s, nt, sg, ord, x, y);
-        case 4: return launch_tod(k_amatvec_filter_poly_mu<POL, 4>, blocks, 0, st, pix, c, s, nt, sg, ord, x, y);
-        default: return launch_tod(k_amatvec_filter_poly_mu<POL, 5>, blocks, 0, st, pix, c, s, nt, sg, ord, x, y);
-    }
-}
-
 /* single-TOD-pass P^T F_K P given the per-subscan Legendre coefficients (cm2_filter_poly_seg_coef);
  * accumulate != 0 adds to y instead of overwriting it */
 extern "C" int cm2_amatvec_filter_poly_mu(const int32_t *pix, const double *c, const double *s, int64_t nt, int pol,
@@ -1587,7 +1542,11 @@ extern "C" int cm2_amatvec_filter_poly_mu(const int32_t *pix, const double *c, c
     SegPoly sg{seg_start, seg_end, seg_coef, tile_seg, tile_flag, nseg};
     const int nk = poly_order + 1;
     const TileOrder ord = make_order(nt, nstreams);
-    return with_pol(pol, [&](auto P) { return dispatch_amatvec_filter_poly_mu<P>(nk, pix, c, s, nt, sg, ord, x, y, st); });
+    return with_pol(pol, [&](auto P) {
+        return with_nk(nk, [&](auto NK) {
+            return launch_tod(k_amatvec_filter_poly_mu<P, NK>, tod_blocks(nt), 0, st, pix, c, s, nt, sg, ord, x, y);
+        });
+    });
 }
 
 /* fused P^T F_K P, Legendre subscan filter of order 1..4 */
@@ -1612,6 +1571,9 @@ extern "C" int cm2_amatvec_filter_poly(const int32_t *pix, const double *c, cons
     if (nt == 0 || npix == 0 || nseg == 0) return CM2_OK;
     const int nk = poly_order + 1;
     return with_pol(pol, [&](auto P) {
-        return dispatch_amatvec_filter_poly<P>(nk, pix, c, s, nt, seg_start, seg_end, nseg, x, y, (int)cap, st);
+        return with_nk(nk, [&](auto NK) {
+            return launch_tod(k_amatvec_filter_poly<P, NK>, nseg, (size_t)cap * 12, st, pix, c, s, nt, seg_start, seg_end,
+                              nseg, x, y, (int)cap);
+        });
     });
 }

@@ -160,6 +160,7 @@ __global__ void __launch_bounds__(FFT_THREADS, 1)
     const int64_t win0 = PAIR ? (blockIdx.x >> 1) : blockIdx.x, winstep = PAIR ? (gridDim.x >> 1) : gridDim.x;
     bool join_pending = false;      // PAIR: arrived at the barrier that ends a window's join, not yet waited for
     for (int64_t win = win0; win < nwin; win += winstep) {
+        // last_le(win_first, nblocks, win), written out: the shared helper swaps the operands of one subtraction here
         int64_t lo = 0, hi = nblocks;
         while (hi - lo > 1) {
             int64_t mid = (lo + hi) >> 1;
@@ -487,7 +488,7 @@ static int fft_launch(const double *coef, int nband, int64_t nblocks, int64_t bl
         count_launch();
         return CM2_OK;
     }
-    int grid = (int)(nwin_ub < sm_count() ? nwin_ub : sm_count());
+    const int grid = capped_grid(nwin_ub, 1);
     // threads per CTA (one CTA per SM): 512 by default -- the 16-point butterflies of the first / last pass
     // need the 128 registers per thread that 512 threads leave (measured at L = 4096: 1.81 ms vs 2.12 ms
     // with 1024 threads, which spill); CM2_FFT_THREADS=1024 selects the other instantiation

@@ -537,14 +537,6 @@ __global__ void __launch_bounds__(TB, CM2_BD_ITER_CTAS) k_bd_iter_tiled(const do
     }
 }
 
-static int vgrid(int64_t n) {
-    int64_t b = (n + VB - 1) / VB;
-    int64_t cap = (int64_t)sm_count() * 4;
-    if (cap > MAXP) cap = MAXP;
-    if (b > cap) b = cap;
-    return (int)(b < 1 ? 1 : b);
-}
-
 // ---- launch geometry, computed once per (device, POL) instead of once per launch ---------------------
 constexpr int MAXDEV = 64;
 struct TailGeom {
@@ -591,46 +583,38 @@ using namespace cm2;
 
 extern "C" int cm2_dot(const double *a, const double *b, int64_t n, double *out, cm2_stream_t stream) {
     CM2_REQUIRE(n >= 0, "n < 0");
-    k_dot<<<vgrid(n), VB, 0, as_stream(stream)>>>(a, b, n, out);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_dot, capped_grid(cdiv(n, VB), 4, MAXP), VB, 0, as_stream(stream), a, b, n, out);
 }
 
 extern "C" int cm2_axpby(double alpha, const double *x, double beta, double *y, int64_t n, cm2_stream_t stream) {
     CM2_REQUIRE(n >= 0, "n < 0");
     if (n == 0) return CM2_OK;
-    k_axpby<<<vgrid(n), VB, 0, as_stream(stream)>>>(alpha, x, beta, y, n);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_axpby, capped_grid(cdiv(n, VB), 4, MAXP), VB, 0, as_stream(stream), alpha, x, beta, y, n);
 }
 
 extern "C" int cm2_pcg_reset(const double *r, int64_t n, double *scal, double atol, cm2_stream_t stream) {
     CM2_REQUIRE(n >= 0, "n < 0");
-    k_reset<<<vgrid(n), VB, 0, as_stream(stream)>>>(r, n, scal, atol);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_reset, capped_grid(cdiv(n, VB), 4, MAXP), VB, 0, as_stream(stream), r, n, scal, atol);
 }
 
 extern "C" int cm2_pcg_update_p(const double *r, const double *z, double *p, int64_t n, double *scal,
                                 cm2_stream_t stream) {
     CM2_REQUIRE(n >= 0, "n < 0");
     cudaStream_t st = as_stream(stream);
-    k_rho<<<vgrid(n), VB, 0, st>>>(r, z, n, scal);
+    const int g = capped_grid(cdiv(n, VB), 4, MAXP);
+    k_rho<<<g, VB, 0, st>>>(r, z, n, scal);
     CM2_LAUNCHED();
-    k_update_p<<<vgrid(n), VB, 0, st>>>(z, p, n, scal);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_update_p, g, VB, 0, st, z, p, n, scal);
 }
 
 extern "C" int cm2_pcg_update_xr(const double *p, const double *q, double *x, double *r, int64_t n, double *scal,
                                  cm2_stream_t stream) {
     CM2_REQUIRE(n >= 0, "n < 0");
     cudaStream_t st = as_stream(stream);
-    k_pq<<<vgrid(n), VB, 0, st>>>(p, q, n, scal);
+    const int g = capped_grid(cdiv(n, VB), 4, MAXP);
+    k_pq<<<g, VB, 0, st>>>(p, q, n, scal);
     CM2_LAUNCHED();
-    k_update_xr<<<vgrid(n), VB, 0, st>>>(p, q, x, r, n, scal);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_update_xr, g, VB, 0, st, p, q, x, r, n, scal);
 }
 
 // development/test hook (cm2_pcg_bd_tail_strided): run the one-thread-per-pixel kernels at every npix
@@ -641,9 +625,8 @@ static int launch_bd_reset_tiled(const double *inv, int64_t npix, double *r, dou
                                  const double *b, double *x, double *p0, cudaStream_t st) {
     const int64_t need = (npix + TP * TW - 1) / (TP * TW);
     const int g = (int)std::max<int64_t>(1, std::min<int64_t>(need, tail_geom<POL>().reset_grid));
-    k_bd_reset_tiled<POL><<<g, TB, sizeof(double) * tile_smem_doubles<POL>(1), st>>>(inv, npix, r, scal, atol, rtol, b, x, p0);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_bd_reset_tiled<POL>, g, TB, sizeof(double) * tile_smem_doubles<POL>(1), st, inv, npix, r, scal, atol, rtol,
+                  b, x, p0);
 }
 
 extern "C" int cm2_pcg_bd_reset(const double *inv, int64_t npix, int pol, double *r, double *z, double *scal,
@@ -654,24 +637,17 @@ extern "C" int cm2_pcg_bd_reset(const double *inv, int64_t npix, int pol, double
     cudaStream_t st = as_stream(stream);
     // the x0 = 0 start that hands out p0 = z needs no z: coalesced tiles when the vectors allow 16-byte access
     if (b != nullptr && p0 != nullptr && !g_force_strided && aligned(b, 16) && aligned(r, 16) && aligned(x, 16) &&
-        aligned(p0, 16)) {
-        if (pol == 1) return launch_bd_reset_tiled<1>(inv, npix, r, scal, atol, rtol, b, x, p0, st);
-        if (pol == 2) return launch_bd_reset_tiled<2>(inv, npix, r, scal, atol, rtol, b, x, p0, st);
-        return launch_bd_reset_tiled<3>(inv, npix, r, scal, atol, rtol, b, x, p0, st);
-    }
-    const int g = vgrid(npix);
-    if (pol == 1) k_bd_reset<1><<<g, VB, 0, st>>>(inv, npix, r, z, scal, atol, rtol, b, x, p0);
-    else if (pol == 2) k_bd_reset<2><<<g, VB, 0, st>>>(inv, npix, r, z, scal, atol, rtol, b, x, p0);
-    else k_bd_reset<3><<<g, VB, 0, st>>>(inv, npix, r, z, scal, atol, rtol, b, x, p0);
-    CM2_LAUNCHED();
-    return CM2_OK;
+        aligned(p0, 16))
+        return with_pol(pol, [&](auto P) { return launch_bd_reset_tiled<P>(inv, npix, r, scal, atol, rtol, b, x, p0, st); });
+    const int g = capped_grid(cdiv(npix, VB), 4, MAXP);
+    return with_pol(pol, [&](auto P) {
+        return launch(k_bd_reset<P>, g, VB, 0, st, inv, npix, r, z, scal, atol, rtol, b, x, p0);
+    });
 }
 
 extern "C" int cm2_pcg_bd_update_p(const double *z, double *p, int64_t n, double *scal, cm2_stream_t stream) {
     CM2_REQUIRE(n >= 0, "n < 0");
-    k_update_p<<<vgrid(n), VB, 0, as_stream(stream)>>>(z, p, n, scal);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return launch(k_update_p, capped_grid(cdiv(n, VB), 4, MAXP), VB, 0, as_stream(stream), z, p, n, scal);
 }
 
 extern "C" int cm2_pcg_bd_update(const double *inv, int64_t npix, int pol, const double *p, const double *q, double *x,
@@ -680,14 +656,10 @@ extern "C" int cm2_pcg_bd_update(const double *inv, int64_t npix, int pol, const
     CM2_REQUIRE(aligned(inv, 16), "inverse blocks must be 16-byte aligned");
     cudaStream_t st = as_stream(stream);
     const int64_t n = npix * pol;
-    k_pq<<<vgrid(n), VB, 0, st>>>(p, q, n, scal);
+    k_pq<<<capped_grid(cdiv(n, VB), 4, MAXP), VB, 0, st>>>(p, q, n, scal);
     CM2_LAUNCHED();
-    const int g = vgrid(npix);
-    if (pol == 1) k_bd_update<1><<<g, VB, 0, st>>>(inv, npix, p, q, x, r, z, scal);
-    else if (pol == 2) k_bd_update<2><<<g, VB, 0, st>>>(inv, npix, p, q, x, r, z, scal);
-    else k_bd_update<3><<<g, VB, 0, st>>>(inv, npix, p, q, x, r, z, scal);
-    CM2_LAUNCHED();
-    return CM2_OK;
+    const int g = capped_grid(cdiv(npix, VB), 4, MAXP);
+    return with_pol(pol, [&](auto P) { return launch(k_bd_update<P>, g, VB, 0, st, inv, npix, p, q, x, r, z, scal); });
 }
 
 // test hook (cm2_pcg_bd_iter_refuse): make the cooperative launch fail the way a GPU that refuses
@@ -735,10 +707,8 @@ extern "C" int cm2_pcg_bd_tail_strided(int on) {
 }
 
 extern "C" int64_t cm2_pcg_bd_iter_max_npix(int pol) {
-    if (pol == 1) return tiled_iter_max_npix<1>();
-    if (pol == 2) return tiled_iter_max_npix<2>();
-    if (pol == 3) return tiled_iter_max_npix<3>();
-    return 0;
+    if (pol < 1 || pol > 3) return 0;
+    return with_pol(pol, [](auto P) { return tiled_iter_max_npix<P>(); });
 }
 
 extern "C" int cm2_pcg_bd_iter(const double *inv, int64_t npix, int pol, double *p, const double *q, double *x,
@@ -746,7 +716,5 @@ extern "C" int cm2_pcg_bd_iter(const double *inv, int64_t npix, int pol, double 
     CM2_REQUIRE(npix >= 0 && pol >= 1 && pol <= 3, "bad npix/pol");
     CM2_REQUIRE(aligned(inv, 16), "inverse blocks must be 16-byte aligned");
     cudaStream_t st = as_stream(stream);
-    if (pol == 1) return launch_bd_iter<1>(inv, npix, p, q, x, r, z, scal, st);
-    if (pol == 2) return launch_bd_iter<2>(inv, npix, p, q, x, r, z, scal, st);
-    return launch_bd_iter<3>(inv, npix, p, q, x, r, z, scal, st);
+    return with_pol(pol, [&](auto P) { return launch_bd_iter<P>(inv, npix, p, q, x, r, z, scal, st); });
 }
