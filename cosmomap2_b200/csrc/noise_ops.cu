@@ -167,6 +167,7 @@ extern "C" int cm2_noise_toeplitz_apply(const double *band, int nband, int64_t n
                                         void *scratch, cm2_stream_t stream) {
     CM2_REQUIRE(nt >= 0 && nblocks > 0 && nband >= 1, "bad sizes");
     CM2_REQUIRE(blk_start != nullptr || blocksize > 0, "blocksize must be > 0");
+    CM2_REQUIRE(blk_start != nullptr || nblocks - 1 <= nt / blocksize, "equal blocks past nt: (nblocks-1)*blocksize > nt");
     CM2_REQUIRE(scratch != nullptr, "scratch (cm2_toeplitz_scratch_bytes) required");
     CM2_REQUIRE(d != out, "in-place Toeplitz apply is not supported");
     if (nt == 0) return CM2_OK;

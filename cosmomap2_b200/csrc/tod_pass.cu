@@ -651,7 +651,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_toeplitz(const int32_t *__res
             int64_t b0 = block_of(tw.blk, t0);
             if (b0 >= tw.blk.nblocks) b0 = tw.blk.nblocks - 1;
             const int64_t bs = tw.blk.start ? __ldg(tw.blk.start + b0) : b0 * tw.blk.blocksize;
-            int64_t be = tw.blk.start ? __ldg(tw.blk.start + b0 + 1) : (b0 + 1) * tw.blk.blocksize;
+            int64_t be = tw.blk.start ? __ldg(tw.blk.start + b0 + 1) : (b0 + 1 == tw.blk.nblocks ? nt : (b0 + 1) * tw.blk.blocksize);
             if (be > nt) be = nt;
             if (t0 + K <= be) {                // the lane's 8 samples lie in one noise block (the common case)
                 const double *a = tw.band + b0 * tw.nband;
@@ -683,7 +683,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_toeplitz(const int32_t *__res
                     int64_t b = block_of(tw.blk, t);
                     if (b >= tw.blk.nblocks) b = tw.blk.nblocks - 1;
                     const int64_t s0 = tw.blk.start ? __ldg(tw.blk.start + b) : b * tw.blk.blocksize;
-                    int64_t s1 = tw.blk.start ? __ldg(tw.blk.start + b + 1) : (b + 1) * tw.blk.blocksize;
+                    int64_t s1 = tw.blk.start ? __ldg(tw.blk.start + b + 1) : (b + 1 == tw.blk.nblocks ? nt : (b + 1) * tw.blk.blocksize);
                     if (s1 > nt) s1 = nt;
                     const double *a = tw.band + b * tw.nband;
                     double acc = __ldg(a) * v[j];
@@ -1438,7 +1438,8 @@ extern "C" int cm2_amatvec_toeplitz(const int32_t *pix, const double *c, const d
     CM2_REQUIRE(band != nullptr && nband >= 1, "band required");
     rc = check_blocks(band, nblocks, blocksize, blk_start);
     if (rc) return rc;
-    if (nband > cm2_amatvec_toeplitz_max_band())
+    CM2_REQUIRE(blk_start != nullptr || nblocks - 1 <= nt / blocksize, "equal blocks past nt: (nblocks-1)*blocksize > nt");
+    if (nband >cm2_amatvec_toeplitz_max_band())
         return set_error(CM2_ERR_UNSUPPORTED, "fused Toeplitz A-matvec: nband=%d, bands of up to %d coefficients are supported",
                          nband, cm2_amatvec_toeplitz_max_band());
     CM2_REQUIRE(npix >= 0, "npix < 0");

@@ -446,6 +446,7 @@ static int fft_launch(const double *coef, int nband, int64_t nblocks, int64_t bl
                       const double *d, double *out, int64_t nt, void *scratch, int init, int pair, cudaStream_t st) {
     CM2_REQUIRE(nt >= 0 && nblocks > 0 && nband >= 1, "bad sizes");
     CM2_REQUIRE(blk_start != nullptr || blocksize > 0, "blocksize must be > 0");
+    CM2_REQUIRE(blk_start != nullptr || nblocks - 1 <= nt / blocksize, "equal blocks past nt: (nblocks-1)*blocksize > nt");
     CM2_REQUIRE(pair == 0 || pair == 1, "pair must be 0 or 1");
     CM2_REQUIRE(2 * (nband - 1) < (pair ? FFT_NF : FFT_NF / 2), "band too wide for the overlap-save window (4096 coefficients; 8192 in pair mode)");
     CM2_REQUIRE(scratch != nullptr && aligned(scratch, 16) && aligned(coef, 16), "scratch/coef must be 16-byte aligned");

@@ -108,8 +108,13 @@ int cm2_bdfwd_apply(const double *mom, int64_t npix, int pol, const double *x, d
                     cm2_stream_t stream);
 
 /* ---- a3/a4/a5: noise operators ------------------------------------------------------------ */
-/* white: out[t] = w[block(t)] * d[t]; equal blocks of `blocksize` when blk_start is NULL, else
- * block b = [blk_start[b], blk_start[b+1])   (linearoperators.py:676-683, blkop.py:178-208,
+/* Noise blocks (here, for the Toeplitz entry points below and cm2_amatvec_toeplitz):
+ *  - blk_start == NULL: equal blocks, block b = [b*blocksize, (b+1)*blocksize) and the last block
+ *    [(nblocks-1)*blocksize, nt), which also takes the remainder past nblocks*blocksize.  The Toeplitz
+ *    entry points refuse (nblocks-1)*blocksize > nt with CM2_ERR_ARG.
+ *  - else block b = [blk_start[b], blk_start[b+1]) with blk_start[0] = 0, blk_start non-decreasing
+ *    and blk_start[nblocks] = nt; empty blocks are allowed.  This is not checked on the device.
+ * white: out[t] = w[block(t)] * d[t]   (linearoperators.py:676-683, blkop.py:178-208,
  * WeightingLO :606-617).  in-place allowed (out == d). */
 int cm2_noise_white_apply(const double *wblk, int64_t nblocks, int64_t blocksize,
                           const int64_t *blk_start, const double *d, double *out, int64_t nt,
@@ -237,7 +242,7 @@ int cm2_pointing_filter_mu(const int32_t *pix, const double *cos2phi, const doub
  * (ToeplitzLO.mult interfaces/linearoperators.py:582-595 applied per block, :672-674; the composition
  * A = P.T*N*P of tests/test_2level_preconditioner.py:16-29, tests/test_coarse_operator.py:15-26):
  * one TOD pass, no time-domain temporary.  band[nblocks][nband] = a_0 .. a_{nband-1} per block,
- * nband <= cm2_amatvec_toeplitz_max_band(); block geometry as for cm2_amatvec_white. */
+ * nband <= cm2_amatvec_toeplitz_max_band(); noise blocks as for cm2_noise_toeplitz_apply. */
 int cm2_amatvec_toeplitz_max_band(void);
 int cm2_amatvec_toeplitz(const int32_t *pix, const double *cos2phi, const double *sin2phi,
                          int64_t nt, int pol, const double *band, int nband, int64_t nblocks,

@@ -78,13 +78,13 @@ def nt_trips():
 
 
 class Guarded:
-    """An n-element output at 32 bytes into a buffer of sentinel words."""
+    """An n-element output at 32 bytes (+ 8 * shift) into a buffer of sentinel words."""
 
-    def __init__(self, n, dtype=None):
+    def __init__(self, n, dtype=None, shift=0):
         import torch
-        self.n = int(n)
-        self.buf = torch.full((4 + self.n + GUARD_HI,), SENTINEL, dtype=torch.int64, device="cuda")
-        self.view = self.buf[4:4 + self.n]
+        self.n, self.lo = int(n), 4 + shift
+        self.buf = torch.full((self.lo + self.n + GUARD_HI,), SENTINEL, dtype=torch.int64, device="cuda")
+        self.view = self.buf[self.lo:self.lo + self.n]
         if dtype is not torch.int64:
             self.view = self.view.view(torch.float64)
 
@@ -93,7 +93,7 @@ class Guarded:
 
     def result(self, what):
         b = self.buf
-        ok = bool((b[:4] == SENTINEL).all().item()) and bool((b[4 + self.n:] == SENTINEL).all().item())
+        ok = bool((b[:self.lo] == SENTINEL).all().item()) and bool((b[self.lo + self.n:] == SENTINEL).all().item())
         assert ok, "%s: wrote outside its output" % what
         return self.view.cpu().numpy()
 
