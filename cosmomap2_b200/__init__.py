@@ -28,6 +28,7 @@ from .utilities import (dgemm, norm2, scalprod, get_legendre_polynomials, is_sor
                         noise_val, subscan_resize, system_setup, reorganize_map, profile_run,
                         output_profile, subtract_offset, rescalepixels)
 from .pcg import cg  # noqa: F401
+from .noise import noise_psd, inverse_noise_bands  # noqa: F401
 from . import IOfiles  # noqa: F401
 from .IOfiles import (read_from_data, read_multiple_ces, read_from_data_with_subscan_resize,  # noqa: F401
                       read_ces_shard, flagging_subscan, flagging_not_in_allCES,

@@ -45,6 +45,8 @@ SIGNATURES = {
     "cm2_toeplitz_fft_points": (_int, []),
     "cm2_toeplitz_fft_scratch_bytes": (_i64, [_i64]),
     "cm2_noise_toeplitz_fft_apply": (_int, [_vp, _int, _i64, _i64, _vp, _vp, _vp, _i64, _vp, _int, _int, _vp]),
+    "cm2_noise_psd_scratch_bytes": (_i64, [_i64]),
+    "cm2_noise_psd": (_int, [_vp, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp, _int, _vp]),
     "cm2_filter_offset_apply": (_int, [_vp, _vp, _vp, _i64, _vp, _vp, _i64, _vp]),
     "cm2_amatvec_white": (_int, [_vp, _vp, _vp, _vp, _i64, _int, _vp, _i64, _i64, _vp, _vp, _vp, _i64, _i64, _vp]),
     "cm2_pack_pointing": (_int, [_vp, _i64, _vp, _vp, _vp]),
@@ -104,7 +106,8 @@ SIGNATURES = {
 # entry points that return a size/count rather than a status
 _NOT_STATUS = {"cm2_version", "cm2_last_error", "cm2_launch_count", "cm2_scan_scratch_bytes",
                "cm2_toeplitz_scratch_bytes", "cm2_defl_work_doubles", "cm2_allreduce_p2p_signal_bytes",
-               "cm2_toeplitz_fft_points", "cm2_toeplitz_fft_scratch_bytes", "cm2_filter_poly_max_order", "cm2_filter_poly_set_tma",
+               "cm2_toeplitz_fft_points", "cm2_toeplitz_fft_scratch_bytes", "cm2_noise_psd_scratch_bytes",
+               "cm2_filter_poly_max_order", "cm2_filter_poly_set_tma",
                "cm2_amatvec_filter_poly_max_order", "cm2_amatvec_toeplitz_max_band",
                "cm2_allreduce_p2p_set_timeout", "cm2_pcg_bd_iter_refuse", "cm2_pcg_bd_iter_max_npix",
                "cm2_pcg_bd_tail_strided",

@@ -128,3 +128,17 @@ def toeplitz_bands(ndet, nband, seed=0, eps=0.3, alpha=1.5):
         a[1:] = -eps * (1.0 + 0.1 * rng.random()) * base
         bands.append(a)
     return bands
+
+
+def one_over_f_noise(ns, ndet, sigma, fknee, alpha, seed):
+    """Seeded 1/f noise, detector-major (ndet timelines of ns samples): per detector, white noise shaped in
+    Fourier space to the PSD P(f) = sigma^2 (1 + (fknee / |f|)^alpha), f in cycles per sample (periodic over the
+    timeline; the mean mode keeps the white level sigma^2)."""
+    rng = np.random.default_rng(seed)
+    f = np.fft.rfftfreq(int(ns))
+    gain = np.full(f.shape, float(sigma))
+    gain[1:] *= np.sqrt(1.0 + (float(fknee) / f[1:]) ** float(alpha))
+    out = np.empty(int(ns) * int(ndet))
+    for b in range(int(ndet)):
+        out[b * ns:(b + 1) * ns] = np.fft.irfft(np.fft.rfft(rng.standard_normal(int(ns))) * gain, int(ns))
+    return out

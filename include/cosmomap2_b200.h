@@ -140,6 +140,23 @@ int64_t cm2_toeplitz_fft_scratch_bytes(int64_t nblocks);
 int cm2_noise_toeplitz_fft_apply(const double *coef, int nband, int64_t nblocks, int64_t blocksize,
                                  const int64_t *blk_start, const double *d, double *out,
                                  int64_t nt, void *scratch, int init, int pair, cm2_stream_t stream);
+/* Welch periodogram sums per noise block (blocks as above), for estimating N^-1 from the data.  With
+ * M = cm2_toeplitz_fft_points() and NF = 2M: block b of n_b samples holds floor((n_b - NF)/M) + 1 windows
+ * of NF samples at hop M from its first sample if n_b >= NF, none otherwise; samples past the last full
+ * window are not used.  In window w, x_t = h_t m_t d_t with the periodic Hann window h_t = sin^2(pi t/NF)
+ * and m_t = 0 where pix[t] < 0 (pix may be NULL: no mask).  A flagged sample is selected away, so NaN in a
+ * flagged d never reaches the result; nothing is detrended.  Outputs, for k = 0..M:
+ *   psd[b][k] = S_b(k) = sum_w |X_w(k)|^2  (X_w the NF-point DFT of window w's x),
+ *   wsum[b]   = W_b    = sum_w sum_t (h_t m_t)^2,
+ * 0 for a block without windows.  S_b / W_b is the pooled one-sided-range estimate of the two-sided PSD
+ * (without flags: scipy.signal.welch(window='hann', nperseg=NF, noverlap=M, detrend=False,
+ * return_onesided=False)[:M+1]).  Deterministic: a repeated call gives the same bits, whatever the
+ * alignment of d and pix.  scratch: cm2_noise_psd_scratch_bytes(nblocks) bytes for the current device,
+ * 16-byte aligned; pass init != 0 on the first call with a given scratch (twiddle and window tables). */
+int64_t cm2_noise_psd_scratch_bytes(int64_t nblocks);
+int cm2_noise_psd(const double *d, const int32_t *pix /* NULL: no mask */, int64_t nblocks, int64_t blocksize,
+                  const int64_t *blk_start, int64_t nt, double *psd /* [nblocks][M+1] */, double *wsum /* [nblocks] */,
+                  void *scratch, int init, cm2_stream_t stream);
 /* subscan offset filter (FilterLO.mult :129-168): out = 0; for each segment [seg_start[k],
  * seg_end[k]): mu = mean of d over unflagged samples; skipped if none; out = d - mu */
 int cm2_filter_offset_apply(const int32_t *pix, const int64_t *seg_start, const int64_t *seg_end,
