@@ -45,6 +45,8 @@ SIGNATURES = {
     "cm2_toeplitz_fft_points": (_int, []),
     "cm2_toeplitz_fft_scratch_bytes": (_i64, [_i64]),
     "cm2_noise_toeplitz_fft_apply": (_int, [_vp, _int, _i64, _i64, _vp, _vp, _vp, _i64, _vp, _int, _int, _vp]),
+    "cm2_noise_simulate": (_int, [_vp, _int, _i64, _i64, _vp, _vp, ctypes.c_uint64, ctypes.c_uint32, _vp, _i64, _int,
+                                  _vp, _int, _int, _vp]),
     "cm2_noise_psd_scratch_bytes": (_i64, [_i64]),
     "cm2_noise_psd": (_int, [_vp, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp, _int, _vp]),
     "cm2_filter_offset_apply": (_int, [_vp, _vp, _vp, _i64, _vp, _vp, _i64, _vp]),

@@ -203,6 +203,43 @@ __device__ __forceinline__ void fft_forward(int tid, const double2 *__restrict__
 #undef z
 }
 
+// ---- window sources of k_toeplitz_fft ---------------------------------------------------------------------------
+// Without a generator the window is read from d, zero outside the noise block (the apply's non-circulant boundary).
+// NoiseWindow: the window is generated, w_b(r) for the offsets r from the block start, for every integer r (no
+// boundary): one Philox4x32-10 call per pair p = r / 2 (counter (lo p, hi p, id_b, realization), key (lo seed,
+// hi seed)) and Box-Muller, w(2p) = rho cospi(2 u2), w(2p+1) = rho sinpi(2 u2), rho = sqrt(-2 ln u1),
+// u1 = (a + 1) 2^-53 from x0:x1, u2 = c 2^-53 from x2:x3 (DESIGN.md section 4d).  Overlapping windows regenerate
+// the same samples, so the result depends on (seed, realization, id_b, offset) only.
+// ADD_: out += n instead of out = n.
+template <bool ADD_>
+struct NoiseWindow {
+    static constexpr bool ADD = ADD_;
+    uint64_t seed;
+    const int64_t *ids;      // id_b = (uint32) ids[b]; nullptr: b
+    uint32_t realization;
+};
+
+__device__ __forceinline__ double2 philox_normal_pair(uint64_t seed, uint32_t id, uint32_t realization, int64_t p) {
+    uint32_t c0 = (uint32_t)p, c1 = (uint32_t)((uint64_t)p >> 32), c2 = id, c3 = realization;
+    uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        if (r) { k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+        c0 = hi1 ^ c1 ^ k0;
+        c1 = lo1;
+        c2 = hi0 ^ c3 ^ k1;
+        c3 = lo0;
+    }
+    const uint64_t a = ((((uint64_t)c0) << 32) | c1) >> 11, c = ((((uint64_t)c2) << 32) | c3) >> 11;
+    const double u1 = __ull2double_rn(a + 1) * 0x1p-53, u2 = __ull2double_rn(c) * 0x1p-53;     // both exact
+    const double rho = sqrt(-2.0 * log(u1));
+    double sn, cs;
+    sincospi(2.0 * u2, &sn, &cs);
+    return make_double2(rho * cs, rho * sn);
+}
+
 // one CTA per window.  win_first[b] = first window index of noise block b (prefix, nblocks+1).
 // PAIR: a window of 2 NF = 32768 samples on a CLUSTER of two CTAs (one 16384-point complex transform split by one
 // radix-2 stage).  With z the packed window, W = exp(-2 pi i / 2M): CTA 0 transforms u[n] = z[n] + z[n+M] (the even
@@ -213,15 +250,37 @@ __device__ __forceinline__ void fft_forward(int tid, const double2 *__restrict__
 // the window is U[n] + conj(W^n) V[n] (first half, written by CTA 0) and U[n] - conj(W^n) V[n] (second half,
 // CTA 1): each CTA reads the other's result over distributed shared memory.  At 4096 coefficients 75 % of a window
 // is alias-free instead of 50 %.
-template <int FFT_THREADS, bool PAIR = false>
+// Gen: empty (the apply: the window is read from d) or one NoiseWindow<ADD> (the simulation: the window is generated,
+// d is unused; ADD: out += result).  An empty pack keeps the apply's instantiations, names and parameters as they were.
+template <int FFT_THREADS, bool PAIR = false, class... Gen>
 __global__ void __launch_bounds__(FFT_THREADS, 1)
     k_toeplitz_fft(const double2 *__restrict__ coef,   // [nblocks][2][M]: C1 then C2, indexed by PHYSICAL (bit-reversed) position
                    const double2 *__restrict__ tw, int L, int64_t nblocks, int64_t blocksize,
                    const int64_t *__restrict__ start, const int64_t *__restrict__ win_first,
                    const double *__restrict__ d, double *__restrict__ out, int64_t nt,
-                   const double2 *__restrict__ tw2) {
+                   const double2 *__restrict__ tw2, Gen... gen) {
+    static_assert(sizeof...(Gen) <= 1, "at most one window generator");
+    constexpr bool GEN = sizeof...(Gen) == 1;
+    constexpr bool ADD = GEN && (Gen::ADD && ...);
+    uint64_t seed = 0;
+    const int64_t *ids = nullptr;
+    uint32_t realization = 0;
+    ((seed = gen.seed, ids = gen.ids, realization = gen.realization), ...);
     extern __shared__ double2 zs[];   // M complex points, one pad element per 8 (bank-conflict relief)
 #define z(i) zs[(i) + ((i) >> 3)]
+    // the stores of the alias-free outputs: plain writes, or out += result (ADD)
+    auto put2 = [&](int64_t t, double2 r) {
+        double2 *o = reinterpret_cast<double2 *>(out + t);
+        if constexpr (ADD) {
+            const double2 x = *o;
+            r = make_double2(x.x + r.x, x.y + r.y);
+        }
+        *o = r;
+    };
+    auto put1 = [&](int64_t t, double r) {
+        if constexpr (ADD) out[t] += r;
+        else out[t] = r;
+    };
     // window positions [HD, HD + S) are alias-free; HD = L - 1 rounded up to even and S even, so that a window
     // starts on an even sample whenever its noise block does and the window moves as 16-byte pairs
     const int HD = (L - 1) + ((L - 1) & 1);
@@ -248,8 +307,11 @@ __global__ void __launch_bounds__(FFT_THREADS, 1)
         __syncthreads();
         // ---- forward FFT (fft_forward): the window's inputs straight from global memory, zero outside the noise
         // block (the non-circulant boundary)
+        uint32_t idb = 0;
+        if constexpr (GEN) idb = ids ? (uint32_t)ids[b] : (uint32_t)b;
         auto winload1 = [&](int i) {
             const int64_t t = w0 + 2 * (int64_t)i;
+            if constexpr (GEN) return philox_normal_pair(seed, idb, realization, (t - bs) >> 1);   // t - bs even
             double2 v;
             if (al && t >= bs && t + 1 < be) return *reinterpret_cast<const double2 *>(d + t);
             v.x = (t >= bs && t < be) ? d[t] : 0.0;
@@ -380,9 +442,9 @@ __global__ void __launch_bounds__(FFT_THREADS, 1)
                     for (int m = 0; m < 16; ++m) {
                         const int r0 = 2 * (i0 + m * q) - HD;             // output index of v.x within the window's S outputs (even)
                         if (r0 < 0 || r0 >= S) continue;
-                        if (al && j0 + r0 + 1 < be) { *reinterpret_cast<double2 *>(out + j0 + r0) = v[m]; continue; }
-                        if (j0 + r0 < be) out[j0 + r0] = v[m].x;
-                        if (j0 + r0 + 1 < be) out[j0 + r0 + 1] = v[m].y;
+                        if (al && j0 + r0 + 1 < be) { put2(j0 + r0, v[m]); continue; }
+                        if (j0 + r0 < be) put1(j0 + r0, v[m].x);
+                        if (j0 + r0 + 1 < be) put1(j0 + r0 + 1, v[m].y);
                     }
                 }
             }
@@ -412,9 +474,9 @@ __global__ void __launch_bounds__(FFT_THREADS, 1)
                     const double2 U = crank ? oth[u] : own[u], V = crank ? own[u] : oth[u];
                     const double2 t = cmul(w[u], V);
                     const double2 r = crank ? make_double2(U.x - t.x, U.y - t.y) : make_double2(U.x + t.x, U.y + t.y);
-                    if (al && j0 + r0 + 1 < be) { *reinterpret_cast<double2 *>(out + j0 + r0) = r; continue; }
-                    if (j0 + r0 < be) out[j0 + r0] = r.x;
-                    if (j0 + r0 + 1 < be) out[j0 + r0 + 1] = r.y;
+                    if (al && j0 + r0 + 1 < be) { put2(j0 + r0, r); continue; }
+                    if (j0 + r0 < be) put1(j0 + r0, r.x);
+                    if (j0 + r0 + 1 < be) put1(j0 + r0 + 1, r.y);
                 }
             }
             // the partner has read my half once it, too, arrives here; waited for before the next window's first
@@ -598,15 +660,57 @@ extern "C" int64_t cm2_toeplitz_fft_scratch_bytes(int64_t nblocks) {
     return (nblocks + 1) * (int64_t)sizeof(int64_t) + 2 * (int64_t)FFT_M * (int64_t)sizeof(double2) + 64;
 }
 
+
+// one launch of an overlap-save kernel: persistent CTAs (grid), or 2-CTA clusters (PAIR, grid = 2 x clusters)
+template <bool PAIR, class... Params, class... Args>
+static int fft_run(void (*kern)(Params...), int threads, int grid, size_t smem, cudaStream_t st, Args... args) {
+    CM2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if constexpr (!PAIR) {
+        kern<<<grid, threads, smem, st>>>(args...);
+        CM2_LAUNCHED();
+        return CM2_OK;
+    }
+    // one window per 2-CTA cluster (distributed shared memory for the joining stage)
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)grid);
+    cfg.blockDim = dim3(threads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 2;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    CM2_CUDA(cudaLaunchKernelEx(&cfg, kern, args...));
+    count_launch();
+    return CM2_OK;
+}
+
+template <int T, bool PAIR, class... Gen>
+static int fft_kernel(int grid, size_t smem, cudaStream_t st, const double2 *cf, const double2 *tw, int nband,
+                      int64_t nblocks, int64_t blocksize, const int64_t *blk_start, const int64_t *win_first,
+                      const double *d, double *out, int64_t nt, const double2 *tw2, Gen... gen) {
+    return fft_run<PAIR>(k_toeplitz_fft<T, PAIR, Gen...>, T, grid, smem, st, cf, tw, nband, nblocks, blocksize, blk_start,
+                         win_first, d, out, nt, tw2, gen...);
+}
+
+// The overlap-save launcher of the apply (no generator, d the input) and of the noise simulation (one NoiseWindow,
+// d = nullptr): argument checks, twiddles, window plan and grid in one place.
+template <class... Gen>
 static int fft_launch(const double *coef, int nband, int64_t nblocks, int64_t blocksize, const int64_t *blk_start,
-                      const double *d, double *out, int64_t nt, void *scratch, int init, int pair, cudaStream_t st) {
+                      const double *d, double *out, int64_t nt, void *scratch, int init, int pair, cudaStream_t st,
+                      Gen... gen) {
     CM2_REQUIRE(nt >= 0 && nblocks > 0 && nband >= 1, "bad sizes");
     CM2_REQUIRE(blk_start != nullptr || blocksize > 0, "blocksize must be > 0");
     CM2_REQUIRE(blk_start != nullptr || nblocks - 1 <= nt / blocksize, "equal blocks past nt: (nblocks-1)*blocksize > nt");
     CM2_REQUIRE(pair == 0 || pair == 1, "pair must be 0 or 1");
     CM2_REQUIRE(2 * (nband - 1) < (pair ? FFT_NF : FFT_NF / 2), "band too wide for the overlap-save window (4096 coefficients; 8192 in pair mode)");
     CM2_REQUIRE(scratch != nullptr && aligned(scratch, 16) && aligned(coef, 16), "scratch/coef must be 16-byte aligned");
-    CM2_REQUIRE(d != out, "in-place Toeplitz apply is not supported");
+    constexpr bool GEN = sizeof...(Gen) == 1;
+    CM2_REQUIRE(GEN || d != out, "in-place Toeplitz apply is not supported");
+    CM2_REQUIRE(!GEN || nt == 0 || out != nullptr, "out is required");
     if (nt == 0) return CM2_OK;
     double2 *tw = reinterpret_cast<double2 *>(scratch);
     double2 *tw2 = tw + FFT_M;
@@ -624,44 +728,27 @@ static int fft_launch(const double *coef, int nband, int64_t nblocks, int64_t bl
     int64_t nwin_ub = nt / S + nblocks + 1;
     const double2 *cf = reinterpret_cast<const double2 *>(coef);
     if (pair) {
-        // one window per 2-CTA cluster (distributed shared memory for the joining stage)
         int64_t ncl = sm_count() / 2;
         if (nwin_ub < ncl) ncl = nwin_ub;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)(2 * ncl));
-        cfg.blockDim = dim3(512);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = 2;
-        attr[0].val.clusterDim.y = 1;
-        attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        CM2_CUDA(cudaFuncSetAttribute(k_toeplitz_fft<512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        CM2_CUDA(cudaLaunchKernelEx(&cfg, k_toeplitz_fft<512, true>, cf, (const double2 *)tw, nband, nblocks, blocksize,
-                                    blk_start, (const int64_t *)win_first, d, out, nt, (const double2 *)tw2));
-        count_launch();
-        return CM2_OK;
+        return fft_kernel<512, true>((int)(2 * ncl), smem, st, cf, tw, nband, nblocks, blocksize, blk_start, win_first,
+                                     d, out, nt, tw2, gen...);
     }
     const int grid = capped_grid(nwin_ub, 1);
     // threads per CTA (one CTA per SM): 512 by default -- the 16-point butterflies of the first / last pass
     // need the 128 registers per thread that 512 threads leave (measured at L = 4096: 1.81 ms vs 2.12 ms
-    // with 1024 threads, which spill); CM2_FFT_THREADS=1024 selects the other instantiation
-    static const int threads = [] {
-        const char *e = getenv("CM2_FFT_THREADS");
-        return (e && atoi(e) == 1024) ? 1024 : 512;
-    }();
-    if (threads == 512) {
-        CM2_CUDA(cudaFuncSetAttribute(k_toeplitz_fft<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_toeplitz_fft<512><<<grid, 512, smem, st>>>(cf, tw, nband, nblocks, blocksize, blk_start, win_first, d, out, nt, tw2);
-    } else {
-        CM2_CUDA(cudaFuncSetAttribute(k_toeplitz_fft<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_toeplitz_fft<1024><<<grid, 1024, smem, st>>>(cf, tw, nband, nblocks, blocksize, blk_start, win_first, d, out, nt, tw2);
+    // with 1024 threads, which spill); CM2_FFT_THREADS=1024 selects the apply's other instantiation.  The
+    // simulation runs at 512 threads (at 256 it spills nothing but takes 1.15-1.5x as long, DESIGN.md section 4d).
+    if constexpr (!GEN) {
+        static const int threads = [] {
+            const char *e = getenv("CM2_FFT_THREADS");
+            return (e && atoi(e) == 1024) ? 1024 : 512;
+        }();
+        if (threads == 1024)
+            return fft_kernel<1024, false>(grid, smem, st, cf, tw, nband, nblocks, blocksize, blk_start, win_first, d,
+                                           out, nt, tw2);
     }
-    CM2_LAUNCHED();
-    return CM2_OK;
+    return fft_kernel<512, false>(grid, smem, st, cf, tw, nband, nblocks, blocksize, blk_start, win_first, d, out, nt,
+                                  tw2, gen...);
 }
 
 // coef: device, [nblocks][2][M] complex (C1, C2 stored at the bit-reversed position of their frequency, 1/M folded in);
@@ -672,6 +759,20 @@ extern "C" int cm2_noise_toeplitz_fft_apply(const double *coef, int nband, int64
                                             const int64_t *blk_start, const double *d, double *out, int64_t nt,
                                             void *scratch, int init, int pair, cm2_stream_t stream) {
     return fft_launch(coef, nband, nblocks, blocksize, blk_start, d, out, nt, scratch, init, pair, as_stream(stream));
+}
+
+// n_t = sum_{|k|<L} h_b[|k|] w_b(t - k - s_b) per noise block, w_b the Philox / Box-Muller stream of NoiseWindow keyed on
+// (seed, realization, block_ids[b] or b); out = n (add = 0) or out += n (add != 0).  coef, scratch, init, pair as
+// for cm2_noise_toeplitz_fft_apply.
+extern "C" int cm2_noise_simulate(const double *coef, int nband, int64_t nblocks, int64_t blocksize,
+                                  const int64_t *blk_start, const int64_t *block_ids, uint64_t seed, uint32_t realization,
+                                  double *out, int64_t nt, int add, void *scratch, int init, int pair,
+                                  cm2_stream_t stream) {
+    if (add)
+        return fft_launch(coef, nband, nblocks, blocksize, blk_start, nullptr, out, nt, scratch, init, pair,
+                          as_stream(stream), NoiseWindow<true>{seed, block_ids, realization});
+    return fft_launch(coef, nband, nblocks, blocksize, blk_start, nullptr, out, nt, scratch, init, pair,
+                      as_stream(stream), NoiseWindow<false>{seed, block_ids, realization});
 }
 
 // scratch: twiddles (2 M double2), Hann window (NF doubles), win_first (nblocks + 1), one slot of M + 2 doubles per

@@ -1,11 +1,13 @@
 """
 The noise model from the data: per-detector Welch PSD on the GPU, and the N^-1 Toeplitz bands for
-``BlockLO(blocksize, bands, offdiag=True)`` (DESIGN.md section 4c).
+``BlockLO(blocksize, bands, offdiag=True)`` (DESIGN.md section 4c), and noise simulations with that model
+(section 4d).
 
     freqs, psd = noise_psd(d, blocksize, pix=pix)     # cm2_noise_psd: one pass over the TOD on the device
     bands = inverse_noise_bands(psd, nband)            # host, NumPy: nblocks x (M+1) values
     N = BlockLO(blocksize, bands, offdiag=True)
     Mbd_weights = [t[0] for t in bands]
+    n = simulate_noise(noise_sim_bands(psd, nband), blocksize, seed, realization)   # on the device
 
 Noise blocks are BlockLO's partition: ``blocksize`` an int (equal blocks, the remainder past
 ``nblocks * blocksize`` in the last one, nblocks = len(d) // blocksize) or one size per block.
@@ -20,7 +22,7 @@ import numpy as np
 import torch
 
 from . import _device as dv
-from .linearoperators import _block_starts
+from .linearoperators import _block_starts, _Blocks, toeplitz_fft_tables
 
 
 def _points():
@@ -101,6 +103,12 @@ def inverse_noise_bands(psd, nband):
     ``BlockLO(blocksize, bands, offdiag=True)``; the M_BD weights are ``[t[0] for t in bands]``.
     Raises ValueError when a block's PSD has a value <= 0 or not finite.
     """
+    return _tapered_bands(psd, nband, lambda p: 1.0 / p)
+
+
+def _tapered_bands(psd, nband, symbol):
+    """t_b[j] = c_b[j] (1 - j / nband), c_b = irfft(symbol(psd_b), NF)[:nband]: the Bartlett lag taper shared by
+    the N^-1 bands and the simulation bands."""
     psd = np.atleast_2d(np.asarray(psd, dtype=np.float64))
     M = psd.shape[1] - 1
     nband = int(nband)
@@ -109,6 +117,99 @@ def inverse_noise_bands(psd, nband):
     for b in range(psd.shape[0]):
         if not np.all(np.isfinite(psd[b]) & (psd[b] > 0)):
             raise ValueError("noise block %d: the PSD has a value <= 0 or not finite" % b)
-    c = np.fft.irfft(1.0 / psd, 2 * M, axis=1)[:, :nband]
+    c = np.fft.irfft(symbol(psd), 2 * M, axis=1)[:, :nband]
     t = c * (1.0 - np.arange(nband) / float(nband))
     return [t[b].copy() for b in range(psd.shape[0])]
+
+
+def noise_sim_bands(psd, nband):
+    """Simulation bands from the PSDs of ``noise_psd`` (host, NumPy), one per block, for ``simulate_noise``:
+
+        c_b = irfft(sqrt(psd_b), NF)[:nband],   t_b[j] = c_b[j] (1 - j / nband),   1 <= nband <= M.
+
+    The Bartlett lag taper of ``inverse_noise_bands`` keeps the symbol smooth, so truncation makes no Gibbs
+    notches.  Noise drawn with band t_b has exactly the PSD |sum_{|j|<nband} t_b[|j|] e^{-2 pi i f j}|^2; at
+    nband = M that is psd_b smoothed by the Fejer kernel, and nothing below the resolution 1/NF of the estimate
+    is invented.  ``nband = 1`` gives white noise of amplitude mean(sqrt(psd_b)) over the full circle of NF
+    frequencies.  Raises ValueError when a block's PSD has a value <= 0 or not finite.
+    """
+    return _tapered_bands(psd, nband, np.sqrt)
+
+
+# Bands of at least this many coefficients are simulated on 32768-sample windows on 2-CTA clusters: only those that one
+# CTA's window cannot hold.  Unlike the apply (TOEPLITZ_FFT_PAIR_MIN_BAND), each CTA of a cluster generates both halves
+# of its window, twice the generator work per output.  Measured per 1e8 samples on a B200, one-CTA / cluster windows:
+# 1.29 / 2.17 ms at 1 coefficient, 1.34 / 2.18 at 256, 2.41 / 2.78 at 4096 (DESIGN.md section 4d).
+NOISE_SIM_PAIR_MIN_BAND = 4097
+
+
+class NoiseSimulator(object):
+    """The device tables of ``simulate_noise`` for one set of bands and blocks, kept for many draws (a Monte Carlo):
+    ``NoiseSimulator(bands, blocksize)(seed, realization=0, block_ids=None, add_to=None)``."""
+
+    def __init__(self, bands, blocksize):
+        bands = [np.atleast_1d(np.asarray(a, dtype=np.float64)) for a in bands]
+        nb = len(bands)
+        if nb == 0:
+            raise ValueError("no noise blocks")
+        M = _points()
+        L = max(len(a) for a in bands)
+        if 2 * (L - 1) >= 2 * M:
+            raise ValueError("bands of %d coefficients: at most %d can be simulated" % (L, M))
+        band = np.zeros((nb, L))
+        for i, a in enumerate(bands):
+            band[i, :len(a)] = a
+        self.nband, self.nblocks = L, nb
+        self.pair = 1 if L >= NOISE_SIM_PAIR_MIN_BAND else 0
+        self._blk = _Blocks(_block_starts(blocksize, nb))
+        self.nt = self._blk.nt
+        coef = toeplitz_fft_tables(band, L, M, pair=bool(self.pair))
+        self._coef = dv.to_dev_f64(coef.view(np.float64).reshape(-1))
+        self._scratch = torch.empty(int(dv.call("cm2_toeplitz_fft_scratch_bytes", nb)) // 8 + 2, dtype=torch.float64,
+                                    device=self._coef.device)
+        self._init = 1
+
+    def __call__(self, seed, realization=0, block_ids=None, add_to=None):
+        ids = None
+        if block_ids is not None:
+            ids = np.asarray(block_ids, dtype=np.int64).reshape(-1)
+            if ids.size != self.nblocks or np.any(ids < 0) or np.any(ids >= 1 << 32):
+                raise ValueError("block_ids: one id in [0, 2^32) per noise block")
+            ids = dv.to_dev(ids, torch.int64)
+        seed, realization = int(seed), int(realization)
+        if not 0 <= seed < 1 << 64 or not 0 <= realization < 1 << 32:
+            raise ValueError("seed must be in [0, 2^64) and realization in [0, 2^32)")
+        if add_to is None:
+            out = torch.empty(self.nt, dtype=torch.float64, device=self._coef.device)
+        else:
+            out = add_to
+            if not (isinstance(out, torch.Tensor) and out.is_cuda and out.device == self._coef.device
+                    and out.dtype == torch.float64 and out.is_contiguous()):
+                raise ValueError("add_to must be a contiguous float64 tensor on %s" % self._coef.device)
+            if out.numel() != self.nt:
+                raise ValueError("add_to has %d samples, the noise blocks %d" % (out.numel(), self.nt))
+        nb, bs, startp = self._blk.args()
+        dv.call("cm2_noise_simulate", dv.ptr(self._coef), self.nband, nb, bs, startp, dv.ptr(ids), seed, realization,
+                dv.ptr(out), self.nt, int(add_to is not None), dv.ptr(self._scratch), self._init, self.pair,
+                dv.stream())
+        self._init = 0
+        return out
+
+
+def simulate_noise(bands, blocksize, seed, realization=0, block_ids=None, add_to=None):
+    """Gaussian noise with the band ``bands[b]`` in noise block b, drawn on the GPU (``cm2_noise_simulate``):
+
+        n_t = sum_{|k|<L} h_b[|k|] w_b(t - k - s_b),   s_b <= t < e_b,
+
+    with w_b a unit Gaussian stream (Philox4x32-10 and Box-Muller, DESIGN.md section 4d) keyed on
+    ``(seed, realization, block_ids[b])`` and defined past the block edges, so the noise is stationary up to them.
+    A sample depends on that key and its offset in the block only: the same detector gets the same noise however
+    the TOD is split over calls or ranks.  Sharded use: each rank passes the global ids of its own blocks
+    (default ``range(len(bands))``).  The blocks are BlockLO's partition ``_block_starts(blocksize, len(bands))``,
+    so ``BlockLO(blocksize, bands)`` and the simulation agree; bands of different lengths are zero-padded.  Use
+    ``noise_sim_bands(psd, nband)`` for bands with the PSD of ``noise_psd``; bands of up to M = 8192 coefficients.
+    Returns a new float64 device tensor, or adds the noise in place to ``add_to`` (d = P m + n without a second
+    TOD buffer), which must have exactly the partition's number of samples, and returns it.  For many draws with
+    the same bands, keep a ``NoiseSimulator``.
+    """
+    return NoiseSimulator(bands, blocksize)(seed, realization, block_ids, add_to)

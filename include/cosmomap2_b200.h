@@ -140,6 +140,20 @@ int64_t cm2_toeplitz_fft_scratch_bytes(int64_t nblocks);
 int cm2_noise_toeplitz_fft_apply(const double *coef, int nband, int64_t nblocks, int64_t blocksize,
                                  const int64_t *blk_start, const double *d, double *out,
                                  int64_t nt, void *scratch, int init, int pair, cm2_stream_t stream);
+/* Gaussian noise with a given band per noise block (blocks as above), generated on the device by the same
+ * overlap-save windows:  n_t = sum_{|k|<nband} h_b[|k|] w_b(t - k - s_b)  for s_b <= t < e_b, with no boundary:
+ * w_b(r) is a unit Gaussian stream defined for every integer offset r from the block start, keyed on
+ * (seed, realization, id_b), id_b = (uint32_t) block_ids[b] (block_ids NULL: b).  One Philox4x32-10 call
+ * (counter (lo32 p, hi32 p, id_b, realization), key (lo32 seed, hi32 seed)) gives the pair p = floor(r/2) by
+ * Box-Muller: a = (x0:x1) >> 11, c = (x2:x3) >> 11, u1 = (a+1) 2^-53, u2 = c 2^-53, rho = sqrt(-2 ln u1),
+ * w(2p) = rho cospi(2 u2), w(2p+1) = rho sinpi(2 u2).  So a sample depends on (seed, realization, id_b, t - s_b)
+ * only: not on the call, the CTA or how the blocks are split over calls or ranks.  add = 0: out = n;
+ * add != 0: out += n.  coef, nband, scratch, init and pair as for cm2_noise_toeplitz_fft_apply (coef from the
+ * bands h_b).  Refuses bands too wide for the mode, misaligned coef / scratch and
+ * (nblocks-1)*blocksize > nt; nt = 0 does nothing. */
+int cm2_noise_simulate(const double *coef, int nband, int64_t nblocks, int64_t blocksize, const int64_t *blk_start,
+                       const int64_t *block_ids /* NULL: b */, uint64_t seed, uint32_t realization,
+                       double *out, int64_t nt, int add, void *scratch, int init, int pair, cm2_stream_t stream);
 /* Welch periodogram sums per noise block (blocks as above), for estimating N^-1 from the data.  With
  * M = cm2_toeplitz_fft_points() and NF = 2M: block b of n_b samples holds floor((n_b - NF)/M) + 1 windows
  * of NF samples at hop M from its first sample if n_b >= NF, none otherwise; samples past the last full
