@@ -49,6 +49,7 @@ SIGNATURES = {
                                   _vp, _int, _int, _vp]),
     "cm2_noise_psd_scratch_bytes": (_i64, [_i64]),
     "cm2_noise_psd": (_int, [_vp, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp, _int, _vp]),
+    "cm2_noise_psd_residual": (_int, [_vp, _vp, _vp, _vp, _int, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp, _int, _vp]),
     "cm2_filter_offset_apply": (_int, [_vp, _vp, _vp, _i64, _vp, _vp, _i64, _vp]),
     "cm2_amatvec_white": (_int, [_vp, _vp, _vp, _vp, _i64, _int, _vp, _i64, _i64, _vp, _vp, _vp, _i64, _i64, _vp]),
     "cm2_pack_pointing": (_int, [_vp, _i64, _vp, _vp, _vp]),

@@ -143,6 +143,15 @@ __device__ __forceinline__ int64_t last_le(const int64_t *table, int64_t n, int6
     return lo;
 }
 
+// (P x)_t of one sample from its pixel's POL map values xv and cos / sin 2 phi (not read for POL = 1): the one
+// expression of the pointing apply (tod_pass.cu) and of the residual PSD loader (toeplitz_fft.cu)
+template <int POL>
+__device__ __forceinline__ double project(const double (&xv)[POL], double c, double s) {
+    if constexpr (POL == 1) return xv[0];
+    else if constexpr (POL == 2) return fma(xv[1], s, xv[0] * c);
+    else return fma(xv[2], s, fma(xv[1], c, xv[0]));
+}
+
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -244,13 +244,6 @@ __device__ __forceinline__ void gather_x(const double *__restrict__ x, const int
     }
 }
 
-template <int POL>
-__device__ __forceinline__ double project(const double (&xv)[POL], double c, double s) {
-    if constexpr (POL == 1) return xv[0];
-    else if constexpr (POL == 2) return fma(xv[1], s, xv[0] * c);
-    else return fma(xv[2], s, fma(xv[1], c, xv[0]));
-}
-
 // (P x) of sample j of the chunk (c, s are not read for POL = 1)
 template <int POL>
 __device__ __forceinline__ double project(const double (&xv)[K][POL], const double (&c)[K], const double (&s)[K], int j) {

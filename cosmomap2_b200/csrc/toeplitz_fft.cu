@@ -522,6 +522,18 @@ __global__ void k_win_first(int64_t nblocks, int64_t blocksize, const int64_t *_
 constexpr int PSD_THREADS = 256;    // 128 registers per thread (512 threads) spill in the radix-16 pass
 constexpr int PSD_SLOT = FFT_M + 2;    // S(0..M), W
 
+// ---- sample sources of k_noise_psd ------------------------------------------------------------------------------
+// Without a source the samples are d_t.  Residual<POL>: the samples are the map residual r_t = d_t - (P x)_t, with
+// (P x)_t = project<POL> of x[POL pix_t ..] and cos / sin 2 phi_t (not read for POL = 1): the expression of
+// k_pointing_apply, so r_t is bit for bit d_t - P.mult(x)_t.  Where pix_t < 0 nothing is gathered and the existing
+// select masks the sample (DESIGN.md section 4e).  pix is required with a Residual.
+template <int POL_>
+struct Residual {
+    static constexpr int POL = POL_;
+    const double *cs, *sn;      // cos 2 phi, sin 2 phi: nt values each (POL > 1)
+    const double *x;            // the map: POL values per pixel, every pixel id < its pixel count
+};
+
 __global__ void k_hann(double *__restrict__ hann) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t < FFT_NF) {
@@ -530,11 +542,19 @@ __global__ void k_hann(double *__restrict__ hann) {
     }
 }
 
+// Src: empty (the samples are d) or one Residual<POL> (the samples are d - P x).  An empty pack keeps the kernel's
+// parameters and code as they were.
+template <class... Src>
 __global__ void __launch_bounds__(PSD_THREADS, 1)
     k_noise_psd(const double2 *__restrict__ tw, const double2 *__restrict__ tw2, const double *__restrict__ hann,
                 int64_t nblocks, int64_t blocksize, const int64_t *__restrict__ start,
                 const int64_t *__restrict__ win_first, const double *__restrict__ d, const int32_t *__restrict__ pix,
-                int64_t nt, double *__restrict__ slots) {
+                int64_t nt, double *__restrict__ slots, Src... src) {
+    static_assert(sizeof...(Src) <= 1, "at most one sample source");
+    constexpr bool RES = sizeof...(Src) == 1;
+    constexpr int POL = (Src::POL * ... * 1);
+    const double *cs = nullptr, *sn = nullptr, *xmap = nullptr;
+    ((cs = src.cs, sn = src.sn, xmap = src.x), ...);
     extern __shared__ double2 zs[];
 #define z(i) zs[(i) + ((i) >> 3)]
     double *acc = reinterpret_cast<double *>(zs + FFT_M + FFT_M / 8);     // [M + 1], by physical position; M last
@@ -558,6 +578,8 @@ __global__ void __launch_bounds__(PSD_THREADS, 1)
         const double *dw = d + t0;
         const int32_t *pw = pix ? pix + t0 : nullptr;
         const bool ald = ((uintptr_t)dw & 15) == 0, alp = ((uintptr_t)pw & 7) == 0;
+        const double *cw = POL > 1 ? cs + t0 : nullptr, *sw = POL > 1 ? sn + t0 : nullptr;
+        const bool alc = ((((uintptr_t)cw) | (uintptr_t)sw) & 15) == 0;
         __syncthreads();                    // the previous window's power step has read zs
         // this thread's sum of (h m)^2 over the run, compensated (Neumaier), in shared memory: as registers across the
         // transform it spills
@@ -566,11 +588,20 @@ __global__ void __launch_bounds__(PSD_THREADS, 1)
             wrun[PSD_THREADS + tid] += fabs(ws) >= fabs(a) ? (ws - s) + a : (a - s) + ws;
             wrun[tid] = s;
         };
+        // r_t = d_t - (P x)_t for an unflagged sample (Residual); a flagged one is returned as is and selected away
+        auto resid = [&](double dv, int p, double c, double s) {
+            if (p < 0) return dv;
+            double xv[POL];
+#pragma unroll
+            for (int k = 0; k < POL; ++k) xv[k] = __ldg(xmap + (int64_t)POL * p + k);
+            return dv - project<POL>(xv, c, s);
+        };
         auto load16 = [&](int i0, int q, double2 (&v)[16]) {
-            // groups of 4 points, every load of a group issued before its first use (48 loads in flight spill)
+            // groups of 4 points, every load of a group issued before its first use (48 loads in flight spill; the
+            // residual's cos / sin and x gathers fit: 217 / 240 / 250 registers at POL 1 / 2 / 3, no spill)
 #pragma unroll
             for (int g = 0; g < 16; g += 4) {
-                double2 x[4], h[4];
+                double2 x[4], h[4], c[4], s[4];
                 int2 p[4];
 #pragma unroll
                 for (int m = 0; m < 4; ++m) {
@@ -579,6 +610,17 @@ __global__ void __launch_bounds__(PSD_THREADS, 1)
                     h[m] = __ldg(reinterpret_cast<const double2 *>(hann) + i);
                     p[m] = !pw ? make_int2(0, 0)
                                : alp ? __ldcs(reinterpret_cast<const int2 *>(pw) + i) : make_int2(__ldcs(pw + 2 * i), __ldcs(pw + 2 * i + 1));
+                    if constexpr (RES && POL > 1) {
+                        c[m] = alc ? __ldcs(reinterpret_cast<const double2 *>(cw) + i) : make_double2(__ldcs(cw + 2 * i), __ldcs(cw + 2 * i + 1));
+                        s[m] = alc ? __ldcs(reinterpret_cast<const double2 *>(sw) + i) : make_double2(__ldcs(sw + 2 * i), __ldcs(sw + 2 * i + 1));
+                    } else {
+                        c[m] = s[m] = make_double2(0.0, 0.0);
+                    }
+                }
+                if constexpr (RES) {
+#pragma unroll
+                    for (int m = 0; m < 4; ++m)
+                        x[m] = make_double2(resid(x[m].x, p[m].x, c[m].x, s[m].x), resid(x[m].y, p[m].y, c[m].y, s[m].y));
                 }
                 double a[4];
 #pragma unroll
@@ -783,15 +825,18 @@ extern "C" int64_t cm2_noise_psd_scratch_bytes(int64_t nblocks) {
                                       ((int64_t)sm_count() + nblocks) * PSD_SLOT);
 }
 
-extern "C" int cm2_noise_psd(const double *d, const int32_t *pix, int64_t nblocks, int64_t blocksize,
-                             const int64_t *blk_start, int64_t nt, double *psd, double *wsum, void *scratch, int init,
-                             cm2_stream_t stream) {
+// The Welch launcher of cm2_noise_psd (no source: the samples are d) and cm2_noise_psd_residual (one Residual<POL>):
+// argument checks, tables, window plan, grid and the slot sums in one place.
+template <class... Src>
+static int psd_launch(const double *d, const int32_t *pix, int64_t nblocks, int64_t blocksize, const int64_t *blk_start,
+                      int64_t nt, double *psd, double *wsum, void *scratch, int init, cudaStream_t st, Src... src) {
     CM2_REQUIRE(nt >= 0 && nblocks > 0, "bad sizes");
     CM2_REQUIRE(blk_start != nullptr || blocksize > 0, "blocksize must be > 0");
     CM2_REQUIRE(blk_start != nullptr || nblocks - 1 <= nt / blocksize, "equal blocks past nt: (nblocks-1)*blocksize > nt");
     CM2_REQUIRE(d != nullptr && psd != nullptr && wsum != nullptr, "d, psd and wsum are required");
     CM2_REQUIRE(scratch != nullptr && aligned(scratch, 16), "scratch (cm2_noise_psd_scratch_bytes) must be 16-byte aligned");
-    cudaStream_t st = as_stream(stream);
+    // cm2_noise_psd writes zero sums for an empty TOD; the residual entry point writes nothing
+    if (sizeof...(Src) == 1 && nt == 0) return CM2_OK;
     double2 *tw = reinterpret_cast<double2 *>(scratch);
     double2 *tw2 = tw + FFT_M;
     double *hann = reinterpret_cast<double *>(tw2 + FFT_M);
@@ -808,11 +853,32 @@ extern "C" int cm2_noise_psd(const double *d, const int32_t *pix, int64_t nblock
     // one CTA per SM (the transform's shared memory), never more CTAs than windows could exist
     const size_t smem = sizeof(double2) * (FFT_M + FFT_M / 8) + sizeof(double) * (FFT_M + 1 + 2 * PSD_THREADS);
     const int grid = capped_grid(nt / FFT_M + 1, 1);
-    CM2_CUDA(cudaFuncSetAttribute(k_noise_psd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (int rc = launch(k_noise_psd, grid, PSD_THREADS, smem, st, (const double2 *)tw, (const double2 *)tw2,
-                        (const double *)hann, nblocks, blocksize, blk_start, (const int64_t *)win_first, d, pix, nt, slots))
+    CM2_CUDA(cudaFuncSetAttribute(k_noise_psd<Src...>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (int rc = launch(k_noise_psd<Src...>, grid, PSD_THREADS, smem, st, (const double2 *)tw, (const double2 *)tw2,
+                        (const double *)hann, nblocks, blocksize, blk_start, (const int64_t *)win_first, d, pix, nt, slots,
+                        src...))
         return rc;
     const int64_t n = nblocks * PSD_SLOT;
     return launch(k_psd_sum, capped_grid(cdiv(n, 256), 8), 256, 0, st, (const int64_t *)win_first, nblocks, grid,
                   (const double *)slots, psd, wsum);
+}
+
+extern "C" int cm2_noise_psd(const double *d, const int32_t *pix, int64_t nblocks, int64_t blocksize,
+                             const int64_t *blk_start, int64_t nt, double *psd, double *wsum, void *scratch, int init,
+                             cm2_stream_t stream) {
+    return psd_launch(d, pix, nblocks, blocksize, blk_start, nt, psd, wsum, scratch, init, as_stream(stream));
+}
+
+// cm2_noise_psd of r = d - P x (Residual): pix is the pointing's own pixel table and masks as in cm2_noise_psd
+extern "C" int cm2_noise_psd_residual(const double *d, const int32_t *pix, const double *cos2phi, const double *sin2phi,
+                                      int pol, const double *x, int64_t nblocks, int64_t blocksize,
+                                      const int64_t *blk_start, int64_t nt, double *psd, double *wsum, void *scratch,
+                                      int init, cm2_stream_t stream) {
+    CM2_REQUIRE(d != nullptr && pix != nullptr && x != nullptr, "d, pix and x are required");
+    CM2_REQUIRE(pol >= 1 && pol <= 3, "pol must be 1, 2 or 3");
+    CM2_REQUIRE(pol == 1 || (cos2phi != nullptr && sin2phi != nullptr), "cos2phi and sin2phi are required for pol > 1");
+    return with_pol(pol, [&](auto P) {
+        return psd_launch(d, pix, nblocks, blocksize, blk_start, nt, psd, wsum, scratch, init, as_stream(stream),
+                          Residual<P>{cos2phi, sin2phi, x});
+    });
 }

@@ -1,13 +1,20 @@
 """
 The noise model from the data: per-detector Welch PSD on the GPU, and the N^-1 Toeplitz bands for
-``BlockLO(blocksize, bands, offdiag=True)`` (DESIGN.md section 4c), and noise simulations with that model
-(section 4d).
+``BlockLO(blocksize, bands, offdiag=True)`` (DESIGN.md section 4c), noise simulations with that model
+(section 4d), and the noise model from the map residual d - P x (section 4e).
 
     freqs, psd = noise_psd(d, blocksize, pix=pix)     # cm2_noise_psd: one pass over the TOD on the device
     bands = inverse_noise_bands(psd, nband)            # host, NumPy: nblocks x (M+1) values
     N = BlockLO(blocksize, bands, offdiag=True)
     Mbd_weights = [t[0] for t in bands]
     n = simulate_noise(noise_sim_bands(psd, nband), blocksize, seed, realization)   # on the device
+
+The PSD of ``d`` includes the sky, which is strongest at the scan frequencies.  Estimate the noise from the
+residual of a first solve and solve again (section 4e); the residual is formed inside the PSD pass:
+
+    x0 = solve with N0 = BlockLO(blocksize, inverse_noise_bands(noise_psd(d, blocksize, pix=pix)[1], nband), True)
+    freqs, psd = noise_psd(d, blocksize, P=P, x=x0)    # PSD of d - P x0, masked by P's own pixel table
+    x1 = solve with N1 = BlockLO(blocksize, inverse_noise_bands(psd, nband), offdiag=True)
 
 Noise blocks are BlockLO's partition: ``blocksize`` an int (equal blocks, the remainder past
 ``nblocks * blocksize`` in the last one, nblocks = len(d) // blocksize) or one size per block.
@@ -22,7 +29,7 @@ import numpy as np
 import torch
 
 from . import _device as dv
-from .linearoperators import _block_starts, _Blocks, toeplitz_fft_tables
+from .linearoperators import SparseLO, _block_starts, _Blocks, toeplitz_fft_tables
 
 
 def _points():
@@ -42,8 +49,9 @@ def _block_edges(nt, blocksize):
     return np.r_[np.arange(nb, dtype=np.int64) * bs, nt], bs
 
 
-def noise_psd(d, blocksize, pix=None):
-    """Welch PSD of every noise block of the TOD ``d`` (host array or device tensor), computed on the GPU.
+def noise_psd(d, blocksize, pix=None, P=None, x=None):
+    """Welch PSD of every noise block of the TOD ``d`` (host array or device tensor), computed on the GPU, or of the
+    map residual ``d - P x`` when a pointing ``P`` and a map ``x`` are given.
 
     Windows of NF = 2M = 16384 samples (M = ``cm2_toeplitz_fft_points()``) at hop M (50 % overlap) from
     each block's first sample; samples past the last full window are not used.  Each window is tapered
@@ -59,8 +67,29 @@ def noise_psd(d, blocksize, pix=None):
     shape (nblocks, M+1).  Raises ValueError for a block shorter than one window or with every window
     sample flagged.  With an int ``blocksize`` that does not divide len(d) the last block holds the
     remainder; give BlockLO the same partition as per-block sizes.
+
+    Residual (``cm2_noise_psd_residual``): with ``P`` a ``SparseLO`` and ``x`` its map (host or device,
+    ``P.pol * P.ncols`` float64 values), the samples are ``r_t = d_t - (P x)_t``, formed inside the PSD pass: no
+    residual TOD is written.  The mask is ``P``'s own pixel table, so samples whose pixel ProcessTimeSamples dropped
+    are masked too.  The result is bit for bit ``noise_psd(d - P.mult(x), blocksize, pix=<P's pixel table>)``.  The
+    two-pass estimate: solve with bands from ``noise_psd(d, ...)``, then estimate again from
+    ``noise_psd(d, ..., P=P, x=x0)`` and solve with the new bands (DESIGN.md section 4e).  Raises ValueError for
+    ``pix`` together with ``P``, only one of ``P`` and ``x``, a ``P`` that is not a ``SparseLO`` (composite operators
+    are not accepted), ``len(d) != P.nrows`` or a wrong length of ``x``.
     """
     nt = int(d.numel() if dv.is_dev(d) else np.size(d))
+    if P is not None and pix is not None:
+        raise ValueError("pass pix or P, not both: the residual is masked by P's own pixel table")
+    if (P is None) != (x is None):
+        raise ValueError("a residual needs both P and x")
+    if P is not None:
+        if not isinstance(P, SparseLO):
+            raise ValueError("P must be a SparseLO pointing operator, got %s" % type(P).__name__)
+        if nt != P.nrows:
+            raise ValueError("d has %d samples, P has %d rows" % (nt, P.nrows))
+        nx = int(x.numel() if dv.is_dev(x) else np.size(x))
+        if nx != P.pol * P.ncols:
+            raise ValueError("x has %d values, P needs pol * ncols = %d" % (nx, P.pol * P.ncols))
     M = _points()
     NF = 2 * M
     edges, bs = _block_edges(nt, blocksize)
@@ -81,8 +110,13 @@ def noise_psd(d, blocksize, pix=None):
                           device=dd.device)
     S = torch.empty(nb * (M + 1), dtype=torch.float64, device=dd.device)
     W = torch.empty(nb, dtype=torch.float64, device=dd.device)
-    dv.call("cm2_noise_psd", dv.ptr(dd), dv.ptr(pp), nb, bs, dv.ptr(start), nt, dv.ptr(S), dv.ptr(W),
-            dv.ptr(scratch), 1, dv.stream())
+    if P is None:
+        dv.call("cm2_noise_psd", dv.ptr(dd), dv.ptr(pp), nb, bs, dv.ptr(start), nt, dv.ptr(S), dv.ptr(W),
+                dv.ptr(scratch), 1, dv.stream())
+    else:
+        xx = dv.to_dev_f64(x).reshape(-1)
+        dv.call("cm2_noise_psd_residual", dv.ptr(dd), dv.ptr(P._pix_dev), dv.ptr(P._cos_dev), dv.ptr(P._sin_dev),
+                P.pol, dv.ptr(xx), nb, bs, dv.ptr(start), nt, dv.ptr(S), dv.ptr(W), dv.ptr(scratch), 1, dv.stream())
     S = dv.to_host(S).reshape(nb, M + 1)
     W = dv.to_host(W)
     empty = np.flatnonzero(~(W > 0))

@@ -171,6 +171,18 @@ int64_t cm2_noise_psd_scratch_bytes(int64_t nblocks);
 int cm2_noise_psd(const double *d, const int32_t *pix /* NULL: no mask */, int64_t nblocks, int64_t blocksize,
                   const int64_t *blk_start, int64_t nt, double *psd /* [nblocks][M+1] */, double *wsum /* [nblocks] */,
                   void *scratch, int init, cm2_stream_t stream);
+/* cm2_noise_psd of the map residual r = d - P x, formed in the window loader (no residual TOD is written):
+ * r_t = d_t - (P x)_t with (P x)_t the expression of cm2_pointing_apply (pol 1, 2, 3; cos2phi and sin2phi are not
+ * read for pol = 1), so the sums are bit for bit those of cm2_noise_psd on d - P x with the same pix.  pix is
+ * required: it is the pointing operator's own pixel table, after ProcessTimeSamples' compaction, so a sample whose
+ * pixel was dropped there (-1) is masked like a flagged one; x is not read for it and NaN in its d never reaches the
+ * sums.  Every pixel id must be less than the map's pixel count (x holds pol values per pixel; not checked, as for
+ * cm2_pointing_apply).  Blocks, outputs, scratch and init as for cm2_noise_psd.  Refuses NULL d, pix or x, pol
+ * outside 1..3 and NULL cos2phi / sin2phi for pol > 1; nt = 0 writes nothing. */
+int cm2_noise_psd_residual(const double *d, const int32_t *pix, const double *cos2phi, const double *sin2phi,
+                           int pol, const double *x, int64_t nblocks, int64_t blocksize, const int64_t *blk_start,
+                           int64_t nt, double *psd /* [nblocks][M+1] */, double *wsum /* [nblocks] */, void *scratch,
+                           int init, cm2_stream_t stream);
 /* subscan offset filter (FilterLO.mult :129-168): out = 0; for each segment [seg_start[k],
  * seg_end[k]): mu = mean of d over unflagged samples; skipped if none; out = d - mu */
 int cm2_filter_offset_apply(const int32_t *pix, const int64_t *seg_start, const int64_t *seg_end,
