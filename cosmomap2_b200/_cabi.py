@@ -75,6 +75,9 @@ SIGNATURES = {
     "cm2_ground_filter_apply": (_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     "cm2_ground_filter_sub": (_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     "cm2_reorganize_map": (_int, [_vp, _vp, _i64, _int, _i64, _vp, _vp]),
+    "cm2_destripe_scatter": (_int, [_vp, _vp, _vp, _vp, _i64, _int, _int, _vp, _vp, _f64, _vp, _i64, _int, _vp]),
+    "cm2_destripe_dot": (_int, [_vp, _vp, _vp, _vp, _i64, _int, _int, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "cm2_destripe_tod_sums": (_int, [_vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp]),
     "cm2_defl_work_doubles": (_i64, [_int]),
     "cm2_defl_zt_apply": (_int, [_vp, _i64, _int, _i64, _vp, _int, _i64, _vp, _vp, _vp]),
     "cm2_defl_z_apply": (_int, [_vp, _i64, _int, _i64, _vp, _f64, _f64, _vp, _vp, _vp]),

@@ -4,7 +4,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ["cabi.cu", "tod_pass.cu", "pixel_ops.cu", "noise_ops.cu", "deflation.cu", "vecops.cu", "p2p_allreduce.cu", "pcg_sharded.cu", "dense_z.cu", "toeplitz_fft.cu", "filter_runs.cu", "filter_poly.cu"]
+SOURCES = ["cabi.cu", "tod_pass.cu", "pixel_ops.cu", "noise_ops.cu", "deflation.cu", "vecops.cu", "p2p_allreduce.cu", "pcg_sharded.cu", "dense_z.cu", "toeplitz_fft.cu", "filter_runs.cu", "filter_poly.cu", "destripe.cu"]
 LIB = os.path.join(HERE, "libcosmomap2_b200.so")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]

@@ -714,17 +714,16 @@ def _tile_tables(seg_start, seg_end, nseg, nt):
     return tile_seg.to(torch.int32), tile_flag
 
 
-def _build_filter_runs(P, F):
-    """Run-compressed table of u_k = P^T 1_k per subscan + the per-tile subscan lookup (csrc/filter_runs.cu),
-    built on the device; False when the subscans are unsorted or the pointing has no runs."""
+def _build_run_table(P, seg_start, seg_end, nseg, need_runs):
+    """Run-compressed table of u_k = P^T 1_k over the unflagged samples of each of the ``nseg`` sorted,
+    non-overlapping segments [seg_start[k], seg_end[k]) (device int64), built on the device (csrc/filter_runs.cu).
+    ``need_runs``: False when the pointing has fewer than 2 samples per run, where the table is no smaller than
+    the TOD.  Returns dict(run_pix, run_mom, seg_first, seg_nruns, nruns), or False when it has no run."""
     nt, st = P.nrows, _stream()
     dev = P._pix_dev.device
-    ss, se = F._seg_start_host, F._seg_end_host
-    if F.nseg == 0 or np.any(ss[1:] < se[:-1]):
-        return False                                    # unsorted / overlapping subscans
     flags = torch.empty(max(nt, 1), dtype=torch.int32, device=dev)
     pixm = torch.empty(max(nt, 1), dtype=torch.int32, device=dev)
-    dv.call("cm2_filter_runs_mark", dv.ptr(P._pix_dev), dv.ptr(F._seg_start), dv.ptr(F._seg_end), F.nseg, nt,
+    dv.call("cm2_filter_runs_mark", dv.ptr(P._pix_dev), dv.ptr(seg_start), dv.ptr(seg_end), nseg, nt,
             dv.ptr(flags), dv.ptr(pixm), st)
     runidx = torch.empty(max(nt, 1), dtype=torch.int32, device=dev)
     count = torch.zeros(1, dtype=torch.int64, device=dev)
@@ -732,20 +731,30 @@ def _build_filter_runs(P, F):
     dv.call("cm2_weights_old2new", dv.ptr(flags), nt, dv.ptr(runidx), dv.ptr(count), dv.ptr(scratch), st)
     nruns = int(count.item())
     del flags, scratch
-    if nruns == 0 or 2 * nruns > nt:
+    if nruns == 0 or (need_runs and 2 * nruns > nt):
         return False
     run_pix = torch.empty(nruns, dtype=torch.int32, device=dev)
     run_mom = torch.empty(3 * nruns, dtype=torch.float64, device=dev)
-    seg_first = torch.empty(max(F.nseg, 1), dtype=torch.int64, device=dev)
-    seg_nruns = torch.empty(max(F.nseg, 1), dtype=torch.int32, device=dev)
+    seg_first = torch.empty(max(nseg, 1), dtype=torch.int64, device=dev)
+    seg_nruns = torch.empty(max(nseg, 1), dtype=torch.int32, device=dev)
     dv.call("cm2_filter_runs_fill", dv.ptr(pixm), dv.ptr(P._cos_dev), dv.ptr(P._sin_dev), P.pol,
-            dv.ptr(F._seg_start), dv.ptr(F._seg_end), F.nseg, dv.ptr(runidx), dv.ptr(run_pix), dv.ptr(run_mom),
+            dv.ptr(seg_start), dv.ptr(seg_end), nseg, dv.ptr(runidx), dv.ptr(run_pix), dv.ptr(run_mom),
             dv.ptr(seg_first), dv.ptr(seg_nruns), st)
-    del pixm, runidx
-    tile_seg, tile_flag = _tile_tables(F._seg_start, F._seg_end, F.nseg, nt)
-    mu = torch.empty(max(F.nseg, 1), dtype=torch.float64, device=dev)
-    return dict(run_pix=run_pix, run_mom=run_mom, seg_first=seg_first, seg_nruns=seg_nruns, nruns=nruns,
-                tile_seg=tile_seg, tile_flag=tile_flag, mu=mu)
+    return dict(run_pix=run_pix, run_mom=run_mom, seg_first=seg_first, seg_nruns=seg_nruns, nruns=nruns)
+
+
+def _build_filter_runs(P, F):
+    """Run-compressed table of u_k = P^T 1_k per subscan + the per-tile subscan lookup (csrc/filter_runs.cu),
+    built on the device; False when the subscans are unsorted or the pointing has no runs."""
+    ss, se = F._seg_start_host, F._seg_end_host
+    if F.nseg == 0 or np.any(ss[1:] < se[:-1]):
+        return False                                    # unsorted / overlapping subscans
+    rt = _build_run_table(P, F._seg_start, F._seg_end, F.nseg, need_runs=True)
+    if not rt:
+        return False
+    rt["tile_seg"], rt["tile_flag"] = _tile_tables(F._seg_start, F._seg_end, F.nseg, P.nrows)
+    rt["mu"] = torch.empty(max(F.nseg, 1), dtype=torch.float64, device=P._pix_dev.device)
+    return rt
 
 
 def _filter_runs(P, F):

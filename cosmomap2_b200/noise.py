@@ -247,3 +247,57 @@ def simulate_noise(bands, blocksize, seed, realization=0, block_ids=None, add_to
     the same bands, keep a ``NoiseSimulator``.
     """
     return NoiseSimulator(bands, blocksize)(seed, realization, block_ids, add_to)
+
+
+def baseline_prior_bands(psd, L, nband, white=None):
+    """``(weights, bands)`` of a destriper with a noise prior (``Destriper``, DESIGN.md section 4f) from the PSDs of
+    ``noise_psd`` (host, NumPy), for baselines of ``L`` samples.  For each block b:
+
+    1. the white level sigma2_b = ``white[b]``, by default the median of psd_b over the bins k >= M/2;
+    2. the correlated part C_b = max(psd_b - sigma2_b, 0);
+    3. the spectral density of the baseline means, S_b(F) = (1/L) sum_{m=0}^{L-1} C_b(f_m) K_L(f_m) with
+       f_m = (F + m)/L folded into [-1/2, 1/2] and K_L(f) = [sin(pi L f) / (L sin(pi f))]^2, on F_k = k/(2M),
+       k = 0..M, with C_b interpolated linearly in |f|;
+    4. bands = the Bartlett-tapered coefficients of 1/S_b (as ``inverse_noise_bands``), so the prior's Toeplitz
+       symbol is positive; ``weights[b]`` = 1/sigma2_b.
+
+    The densities are two-sided, with their integral over [-1/2, 1/2] the variance, as ``noise_psd``'s.  Pass
+    ``weights`` to ``BlockLO(blocksize, weights)`` and ``bands`` as the ``prior``.  Raises ValueError for nband
+    outside [1, M], L < 1, a wrong length of ``white`` and a block whose S_b is not positive somewhere (a PSD with
+    no correlated part, for instance).
+    """
+    psd = np.atleast_2d(np.asarray(psd, dtype=np.float64))
+    nb, M = psd.shape[0], psd.shape[1] - 1
+    L, nband = int(L), int(nband)
+    if M < 1 or not 1 <= nband <= M:
+        raise ValueError("nband must be in [1, %d], got %d" % (M, nband))
+    if L < 1:
+        raise ValueError("the baseline length must be >= 1 sample, got %d" % L)
+    k = np.arange(M + 1)
+    if white is None:
+        sigma2 = np.median(psd[:, k >= M / 2.0], axis=1)
+    else:
+        sigma2 = np.asarray(white, dtype=np.float64).reshape(-1)
+        if sigma2.size != nb:
+            raise ValueError("white has %d values, psd has %d blocks" % (sigma2.size, nb))
+    if not np.all(np.isfinite(sigma2) & (sigma2 > 0)):
+        raise ValueError("the white level must be positive and finite in every block")
+    C = np.maximum(psd - sigma2[:, None], 0.0)
+    f = k / (2.0 * M)                                   # the PSD bins and the baseline frequencies F_k alike
+    S = np.zeros((nb, M + 1))
+    step = max(1, (1 << 22) // (M + 1))                 # aliases per chunk: bounded temporaries for long baselines
+    for m0 in range(0, L, step):
+        fm = (f[:, None] + np.arange(m0, min(L, m0 + step))[None, :]) / L
+        fm -= np.round(fm)
+        sf = np.sin(np.pi * fm)
+        tiny = np.abs(sf) < 1e-300
+        K = np.where(tiny, 1.0, np.sin(np.pi * L * fm) / (L * np.where(tiny, 1.0, sf))) ** 2
+        af = np.abs(fm).reshape(-1)
+        for b in range(nb):
+            S[b] += (np.interp(af, f, C[b]).reshape(K.shape) * K).sum(axis=1)
+    S /= L
+    for b in range(nb):
+        if not np.all(np.isfinite(S[b]) & (S[b] > 0)):
+            raise ValueError("noise block %d: the baseline spectrum is not positive everywhere (no correlated noise "
+                             "at some frequency): no prior can be formed" % b)
+    return 1.0 / sigma2, _tapered_bands(S, nband, lambda s: 1.0 / s)

@@ -292,6 +292,30 @@ int cm2_amatvec_toeplitz(const int32_t *pix, const double *cos2phi, const double
                          int64_t blocksize, const int64_t *blk_start, const double *x, double *y,
                          int64_t npix, cm2_stream_t stream);
 
+/* ---- destriper with a noise prior (csrc/destripe.cu, DESIGN.md section 4f) -------------------------
+ * Baseline j (a run of L samples inside one noise block; the last one of a block may be short) is a segment of
+ * the run table of cm2_filter_runs_mark / scan / cm2_filter_runs_fill: u_j = P^T 1_j over its unflagged samples,
+ * runs base_first[j] .. base_first[j] + base_nruns[j] - 1, run_mom[r] = {n, sum cos, sum sin}.  bw[j] = the white
+ * weight w_b of baseline j's noise block.  The destriper operator
+ *     q = (F^T W Z F + C_a^-1) a,   Z = I - P M_BD P^T W
+ * is, with n_j = sum of n over baseline j's runs and m = M_BD y (cm2_bd_apply):
+ *   scatter: y (+)= alpha sum_j bw_j c_j u_j   (bw NULL: 1; accumulate = 0 zero-fills y first; atomic adds)
+ *   dot    : out_j = bw_j (n_j a_j - u_j . m) + add_j   (a NULL: 0, add NULL: 0; add = C_a^-1 a, the prior term);
+ *            a fixed-order sum per baseline: a repeated call gives the same bits
+ * Neither reads the TOD.  group = lanes per baseline (4, 8, 16 or 32): pick it near the mean runs per baseline.
+ * tod_sums: out_j = bw_j sum_{t in [base_start[j], base_end[j]), pix[t] >= 0} d[t], the F^T W d of the
+ * right-hand side F^T W Z d = tod_sums - (the dot with a = NULL and m = M_BD P^T W d); NaN in flagged d is not
+ * read into the sums. */
+int cm2_destripe_scatter(const int32_t *run_pix, const double *run_mom, const int64_t *base_first,
+                         const int32_t *base_nruns, int64_t nbase, int pol, int group, const double *c,
+                         const double *bw, double alpha, double *y, int64_t npix, int accumulate,
+                         cm2_stream_t stream);
+int cm2_destripe_dot(const int32_t *run_pix, const double *run_mom, const int64_t *base_first,
+                     const int32_t *base_nruns, int64_t nbase, int pol, int group, const double *bw,
+                     const double *a, const double *m, const double *add, double *out, cm2_stream_t stream);
+int cm2_destripe_tod_sums(const int32_t *pix, const double *d, const int64_t *base_start, const int64_t *base_end,
+                          int64_t nbase, const double *bw, double *out, cm2_stream_t stream);
+
 /* ---- a10/a11/a13: deflation, coarse operator, two-level preconditioner ---------------------- */
 /* Z is n x r, column-major (column i at Z + i*ldz), as DeflationLO stores columns (:1058-1062).
  * `work`: cm2_defl_work_doubles(r) doubles of device scratch. */
