@@ -18,8 +18,6 @@
 // Bound: the L1/shared-memory data pipe (each fused pass moves 32 B per point, 4 passes per transform, the
 // first and the last of the window fused with the global load / store), ~60x fewer flops than the direct
 // form at L = 4096.
-#include <cstdlib>
-
 #include <cooperative_groups.h>
 
 #include "cm2_common.cuh"
@@ -130,6 +128,84 @@ __device__ __forceinline__ void butterfly16(double2 (&v)[16], double2 w16) {
     }
 }
 
+// The 8-point butterfly of the forward radix-8 passes (decimation in frequency, half-sizes 4q, 2q, q) and of the
+// inverse ones (decimation in time, q, 2q, 4q; INV: w8 is already conjugated and the rotations are the conjugate ones).
+template <bool INV>
+__device__ __forceinline__ void butterfly8(double2 (&v)[8], double2 w8) {
+    const double2 w4 = cmul(w8, w8), w2 = cmul(w4, w4);
+    if (!INV) {
+        dif(v[0], v[4], w8);                       // half-size 4q
+        dif(v[1], v[5], rot1(w8));
+        dif(v[2], v[6], rot2(w8));
+        dif(v[3], v[7], rot3(w8));
+        const double2 w4r = rot2(w4);
+        dif(v[0], v[2], w4);                       // half-size 2q
+        dif(v[1], v[3], w4r);
+        dif(v[4], v[6], w4);
+        dif(v[5], v[7], w4r);
+        dif(v[0], v[1], w2);                       // half-size q
+        dif(v[2], v[3], w2);
+        dif(v[4], v[5], w2);
+        dif(v[6], v[7], w2);
+    } else {
+        dit(v[0], v[1], w2);                       // half-size q
+        dit(v[2], v[3], w2);
+        dit(v[4], v[5], w2);
+        dit(v[6], v[7], w2);
+        const double2 w4r = rot2c(w4);
+        dit(v[0], v[2], w4);                       // half-size 2q
+        dit(v[1], v[3], w4r);
+        dit(v[4], v[6], w4);
+        dit(v[5], v[7], w4r);
+        dit(v[0], v[4], w8);                       // half-size 4q
+        dit(v[1], v[5], rot1c(w8));
+        dit(v[2], v[6], rot2c(w8));
+        dit(v[3], v[7], rot3c(w8));
+    }
+}
+
+// One radix-8 pass of eighth-size q = 2^lq through the transform in zs, in place, ending with a barrier: butterfly8<INV>
+// with the pass's twiddle tw[q + pos] (conjugated for INV).  tid = threadIdx.x, read by the kernel (see fft_forward).
+template <int FFT_THREADS, bool INV>
+__device__ __forceinline__ void pass8(int tid, const double2 *__restrict__ tw, int lq) {
+    extern __shared__ double2 zs[];
+#define z(i) zs[(i) + ((i) >> 3)]
+    const int q = 1 << lq;
+    // NB butterflies per thread and loop trip, every input loaded before the first output is stored: the loads of the
+    // second butterfly overlap the arithmetic of the first (the compiler cannot move them above the stores itself: same
+    // shared-memory array)
+    constexpr int NB = (FFT_M / 8) % (2 * FFT_THREADS) == 0 ? 2 : 1;
+    for (int j = tid; j < FFT_M / 8; j += NB * FFT_THREADS) {
+        double2 v[NB][8];
+        int i0[NB];
+        double2 w8[NB];
+#pragma unroll
+        for (int b = 0; b < NB; ++b) {
+            const int jb = j + b * FFT_THREADS;
+            const int pos = jb & (q - 1);
+            i0[b] = ((jb >> lq) << (lq + 3)) + pos;
+#pragma unroll
+            for (int m = 0; m < 8; ++m) v[b][m] = z(i0[b] + m * q);
+            w8[b] = __ldg(tw + q + pos);
+            if (INV) w8[b].y = -w8[b].y;
+        }
+#pragma unroll
+        for (int b = 0; b < NB; ++b) {
+            butterfly8<INV>(v[b], w8[b]);
+#pragma unroll
+            for (int m = 0; m < 8; ++m) z(i0[b] + m * q) = v[b][m];
+        }
+    }
+    __syncthreads();
+#undef z
+}
+
+// The even- and odd-sample spectra of the packed real transform at frequency k from Z_k and Z_{M-k}:
+// E_k = (Z_k + conj Z_{M-k}) / 2,  O_k = (Z_k - conj Z_{M-k}) / 2i
+__device__ __forceinline__ void split_packed(double2 zk, double2 zm, double2 &Ek, double2 &Ok) {
+    Ek = make_double2(0.5 * (zk.x + zm.x), 0.5 * (zk.y - zm.y));
+    Ok = make_double2(0.5 * (zk.y + zm.y), -0.5 * (zk.x - zm.x));
+}
 
 // The forward FFT of one window, decimation in frequency, natural in -> bit-reversed out, in place in zs (one pad
 // element per 8 points).  Radix-2 stages are fused into passes whose points stay in registers: one radix-16 pass
@@ -159,47 +235,7 @@ __device__ __forceinline__ void fft_forward(int tid, const double2 *__restrict__
         }
         __syncthreads();
     }
-    for (int lq = FFT_LOG2M - 7; lq >= 0; lq -= 3) {
-        const int q = 1 << lq;
-        // NB butterflies per thread and loop trip, every input loaded before the first output is stored:
-        // the loads of the second butterfly overlap the arithmetic of the first (the compiler cannot move
-        // them above the stores itself: same shared-memory array)
-        constexpr int NB = (FFT_M / 8) % (2 * FFT_THREADS) == 0 ? 2 : 1;
-        for (int j = tid; j < FFT_M / 8; j += NB * FFT_THREADS) {
-            double2 v[NB][8];
-            int i0[NB];
-            double2 w8[NB];
-#pragma unroll
-            for (int b = 0; b < NB; ++b) {
-                const int jb = j + b * FFT_THREADS;
-                const int pos = jb & (q - 1);
-                i0[b] = ((jb >> lq) << (lq + 3)) + pos;
-#pragma unroll
-                for (int m = 0; m < 8; ++m) v[b][m] = z(i0[b] + m * q);
-                w8[b] = __ldg(tw + q + pos);
-            }
-#pragma unroll
-            for (int b = 0; b < NB; ++b) {
-                const double2 w4 = cmul(w8[b], w8[b]), w2 = cmul(w4, w4);
-                dif(v[b][0], v[b][4], w8[b]);                       // half-size 4q
-                dif(v[b][1], v[b][5], rot1(w8[b]));
-                dif(v[b][2], v[b][6], rot2(w8[b]));
-                dif(v[b][3], v[b][7], rot3(w8[b]));
-                const double2 w4r = rot2(w4);
-                dif(v[b][0], v[b][2], w4);                          // half-size 2q
-                dif(v[b][1], v[b][3], w4r);
-                dif(v[b][4], v[b][6], w4);
-                dif(v[b][5], v[b][7], w4r);
-                dif(v[b][0], v[b][1], w2);                          // half-size q
-                dif(v[b][2], v[b][3], w2);
-                dif(v[b][4], v[b][5], w2);
-                dif(v[b][6], v[b][7], w2);
-#pragma unroll
-                for (int m = 0; m < 8; ++m) z(i0[b] + m * q) = v[b][m];
-            }
-        }
-        __syncthreads();
-    }
+    for (int lq = FFT_LOG2M - 7; lq >= 0; lq -= 3) pass8<FFT_THREADS, false>(tid, tw, lq);
 #undef z
 }
 
@@ -369,10 +405,8 @@ __global__ void __launch_bounds__(FFT_THREADS, 1)
             const int k = __brev((unsigned)pk) >> (32 - FFT_LOG2M);
             const int km = (FFT_M - k) & (FFT_M - 1);
             const int pm = (PAIR && crank == 1) ? (FFT_M - 1 - pk) : (int)(__brev((unsigned)km) >> (32 - FFT_LOG2M));
-            const double2 zk = z(pk), zm = z(pm);
-            // E[k] = (Z[k] + conj Z[M-k])/2 ; O[k] = (Z[k] - conj Z[M-k])/(2i)
-            const double2 Ek = make_double2(0.5 * (zk.x + zm.x), 0.5 * (zk.y - zm.y));
-            const double2 Ok = make_double2(0.5 * (zk.y + zm.y), -0.5 * (zk.x - zm.x));
+            double2 Ek, Ok;
+            split_packed(z(pk), z(pm), Ek, Ok);
             const double2 a1 = cmul(__ldg(c1 + pk), Ek), a2 = cmul(__ldg(c2 + pk), Ok);
             res[i] = make_double2(a1.x + a2.x, a1.y + a2.y);
         }
@@ -383,45 +417,7 @@ __global__ void __launch_bounds__(FFT_THREADS, 1)
         // ---- inverse FFT, decimation in time, bit-reversed in -> natural out (conjugate twiddles):
         // radix-8 passes (half-sizes q, 2q, 4q), then the radix-16 pass whose outputs -- the window in
         // natural order -- go straight to global memory
-        for (int lq = 0; lq + 4 < FFT_LOG2M; lq += 3) {
-            const int q = 1 << lq;
-            constexpr int NB = (FFT_M / 8) % (2 * FFT_THREADS) == 0 ? 2 : 1;
-            for (int j = threadIdx.x; j < FFT_M / 8; j += NB * FFT_THREADS) {
-                double2 v[NB][8];
-                int i0[NB];
-                double2 w8[NB];
-#pragma unroll
-                for (int b = 0; b < NB; ++b) {
-                    const int jb = j + b * FFT_THREADS;
-                    const int pos = jb & (q - 1);
-                    i0[b] = ((jb >> lq) << (lq + 3)) + pos;
-#pragma unroll
-                    for (int m = 0; m < 8; ++m) v[b][m] = z(i0[b] + m * q);
-                    w8[b] = __ldg(tw + q + pos);
-                    w8[b].y = -w8[b].y;                                     // inverse transform: conjugates
-                }
-#pragma unroll
-                for (int b = 0; b < NB; ++b) {
-                    const double2 w4 = cmul(w8[b], w8[b]), w2 = cmul(w4, w4);
-                    dit(v[b][0], v[b][1], w2);                          // half-size q
-                    dit(v[b][2], v[b][3], w2);
-                    dit(v[b][4], v[b][5], w2);
-                    dit(v[b][6], v[b][7], w2);
-                    const double2 w4r = rot2c(w4);
-                    dit(v[b][0], v[b][2], w4);                          // half-size 2q
-                    dit(v[b][1], v[b][3], w4r);
-                    dit(v[b][4], v[b][6], w4);
-                    dit(v[b][5], v[b][7], w4r);
-                    dit(v[b][0], v[b][4], w8[b]);                       // half-size 4q
-                    dit(v[b][1], v[b][5], rot1c(w8[b]));
-                    dit(v[b][2], v[b][6], rot2c(w8[b]));
-                    dit(v[b][3], v[b][7], rot3c(w8[b]));
-#pragma unroll
-                    for (int m = 0; m < 8; ++m) z(i0[b] + m * q) = v[b][m];
-                }
-            }
-            __syncthreads();
-        }
+        for (int lq = 0; lq + 4 < FFT_LOG2M; lq += 3) pass8<FFT_THREADS, true>(threadIdx.x, tw, lq);
         {
             constexpr int lq = FFT_LOG2M - 4, q = 1 << lq;
             for (int j = threadIdx.x; j < FFT_M / 16; j += FFT_THREADS) {
@@ -639,9 +635,8 @@ __global__ void __launch_bounds__(PSD_THREADS, 1)
             const int pk = tid + i * PSD_THREADS;
             const int k = __brev((unsigned)pk) >> (32 - FFT_LOG2M);
             const int pm = __brev((unsigned)((FFT_M - k) & (FFT_M - 1))) >> (32 - FFT_LOG2M);
-            const double2 zk = z(pk), zm = z(pm);
-            const double2 Ek = make_double2(0.5 * (zk.x + zm.x), 0.5 * (zk.y - zm.y));
-            const double2 Ok = make_double2(0.5 * (zk.y + zm.y), -0.5 * (zk.x - zm.x));
+            double2 Ek, Ok;
+            split_packed(z(pk), z(pm), Ek, Ok);
             const double2 wO = cmul(__ldg(tw2 + k), Ok);
             const double2 X = make_double2(Ek.x + wO.x, Ek.y + wO.y);
             acc[pk] += fma(X.x, X.x, X.y * X.y);
@@ -696,12 +691,40 @@ __global__ void k_psd_sum(const int64_t *__restrict__ win_first, int64_t nblocks
 
 using namespace cm2;
 
+// The scratch of both launchers begins with the twiddle tables: tw (M entries, the radix-16 and radix-8 passes), then
+// tw2 (M entries, W^n = exp(-2 pi i n / 2M)).  Each launcher's own tables follow from byte TWIDDLE_BYTES.
+constexpr int64_t TWIDDLE_BYTES = 2 * (int64_t)FFT_M * (int64_t)sizeof(double2);
+constexpr size_t FFT_SMEM = sizeof(double2) * (FFT_M + FFT_M / 8);      // zs: M points, one pad element per 8
+
 extern "C" int cm2_toeplitz_fft_points(void) { return FFT_M; }
 
+// scratch: the twiddles, then win_first (nblocks + 1)
 extern "C" int64_t cm2_toeplitz_fft_scratch_bytes(int64_t nblocks) {
-    return (nblocks + 1) * (int64_t)sizeof(int64_t) + 2 * (int64_t)FFT_M * (int64_t)sizeof(double2) + 64;
+    return TWIDDLE_BYTES + (nblocks + 1) * (int64_t)sizeof(int64_t) + 64;
 }
 
+// The block partition, checked first by both launchers
+static int check_partition(int64_t nblocks, int64_t blocksize, const int64_t *blk_start, int64_t nt) {
+    CM2_REQUIRE(nt >= 0 && nblocks > 0, "bad sizes");
+    CM2_REQUIRE(blk_start != nullptr || blocksize > 0, "blocksize must be > 0");
+    CM2_REQUIRE(blk_start != nullptr || nblocks - 1 <= nt / blocksize, "equal blocks past nt: (nblocks-1)*blocksize > nt");
+    return CM2_OK;
+}
+
+// The set-up of both launchers after their argument checks: the twiddle tables at the head of scratch (built when
+// init != 0) and the window plan win_first for windows of `span` samples at `hop`
+static int plan_windows(void *scratch, int init, int64_t nblocks, int64_t blocksize, const int64_t *blk_start,
+                        int64_t nt, int span, int hop, int64_t *win_first, cudaStream_t st) {
+    double2 *tw = static_cast<double2 *>(scratch);
+    if (init) {
+        k_fft_twiddles<<<(FFT_M / 4 + 255) / 256, 256, 0, st>>>(tw);
+        k_fft_twiddles_pair<<<(FFT_M + 255) / 256, 256, 0, st>>>(tw + FFT_M);
+        CM2_LAUNCHED();
+    }
+    k_win_first<<<1, 1, 0, st>>>(nblocks, blocksize, blk_start, nt, span, hop, win_first);
+    CM2_LAUNCHED();
+    return CM2_OK;
+}
 
 // one launch of an overlap-save kernel: persistent CTAs (grid), or 2-CTA clusters (PAIR, grid = 2 x clusters)
 template <bool PAIR, class... Params, class... Args>
@@ -730,23 +753,25 @@ static int fft_run(void (*kern)(Params...), int threads, int grid, size_t smem, 
     return CM2_OK;
 }
 
-template <int T, bool PAIR, class... Gen>
-static int fft_kernel(int grid, size_t smem, cudaStream_t st, const double2 *cf, const double2 *tw, int nband,
-                      int64_t nblocks, int64_t blocksize, const int64_t *blk_start, const int64_t *win_first,
-                      const double *d, double *out, int64_t nt, const double2 *tw2, Gen... gen) {
-    return fft_run<PAIR>(k_toeplitz_fft<T, PAIR, Gen...>, T, grid, smem, st, cf, tw, nband, nblocks, blocksize, blk_start,
-                         win_first, d, out, nt, tw2, gen...);
+// 512 threads per CTA, one CTA per SM: the 16-point butterflies of the first / last pass need the 128 registers per
+// thread that 512 threads leave.  The simulation runs at 512 threads too (at 256 it spills nothing but takes 1.15-1.5x
+// as long, DESIGN.md section 4d).
+template <bool PAIR, class... Gen>
+static int fft_kernel(int grid, cudaStream_t st, const double2 *cf, const double2 *tw, int nband, int64_t nblocks,
+                      int64_t blocksize, const int64_t *blk_start, const int64_t *win_first, const double *d,
+                      double *out, int64_t nt, const double2 *tw2, Gen... gen) {
+    return fft_run<PAIR>(k_toeplitz_fft<512, PAIR, Gen...>, 512, grid, FFT_SMEM, st, cf, tw, nband, nblocks, blocksize,
+                         blk_start, win_first, d, out, nt, tw2, gen...);
 }
 
 // The overlap-save launcher of the apply (no generator, d the input) and of the noise simulation (one NoiseWindow,
-// d = nullptr): argument checks, twiddles, window plan and grid in one place.
+// d = nullptr): argument checks, window plan and grid in one place.
 template <class... Gen>
 static int fft_launch(const double *coef, int nband, int64_t nblocks, int64_t blocksize, const int64_t *blk_start,
                       const double *d, double *out, int64_t nt, void *scratch, int init, int pair, cudaStream_t st,
                       Gen... gen) {
-    CM2_REQUIRE(nt >= 0 && nblocks > 0 && nband >= 1, "bad sizes");
-    CM2_REQUIRE(blk_start != nullptr || blocksize > 0, "blocksize must be > 0");
-    CM2_REQUIRE(blk_start != nullptr || nblocks - 1 <= nt / blocksize, "equal blocks past nt: (nblocks-1)*blocksize > nt");
+    if (int rc = check_partition(nblocks, blocksize, blk_start, nt)) return rc;
+    CM2_REQUIRE(nband >= 1, "nband must be >= 1");
     CM2_REQUIRE(pair == 0 || pair == 1, "pair must be 0 or 1");
     CM2_REQUIRE(2 * (nband - 1) < (pair ? FFT_NF : FFT_NF / 2), "band too wide for the overlap-save window (4096 coefficients; 8192 in pair mode)");
     CM2_REQUIRE(scratch != nullptr && aligned(scratch, 16) && aligned(coef, 16), "scratch/coef must be 16-byte aligned");
@@ -754,43 +779,21 @@ static int fft_launch(const double *coef, int nband, int64_t nblocks, int64_t bl
     CM2_REQUIRE(GEN || d != out, "in-place Toeplitz apply is not supported");
     CM2_REQUIRE(!GEN || nt == 0 || out != nullptr, "out is required");
     if (nt == 0) return CM2_OK;
-    double2 *tw = reinterpret_cast<double2 *>(scratch);
-    double2 *tw2 = tw + FFT_M;
-    int64_t *win_first = reinterpret_cast<int64_t *>(reinterpret_cast<char *>(scratch) + 2 * FFT_M * sizeof(double2));
-    if (init) {
-        k_fft_twiddles<<<(FFT_M / 4 + 255) / 256, 256, 0, st>>>(tw);
-        k_fft_twiddles_pair<<<(FFT_M + 255) / 256, 256, 0, st>>>(tw2);
-        CM2_LAUNCHED();
-    }
     const int HD = (nband - 1) + ((nband - 1) & 1);
     const int S = ((pair ? 2 * FFT_NF : FFT_NF) - HD - (nband - 1)) & ~1;       // as in the kernel
-    k_win_first<<<1, 1, 0, st>>>(nblocks, blocksize, blk_start, nt, 1, S, win_first);
-    CM2_LAUNCHED();
-    const size_t smem = sizeof(double2) * (FFT_M + FFT_M / 8);
-    int64_t nwin_ub = nt / S + nblocks + 1;
+    int64_t *win_first = reinterpret_cast<int64_t *>(static_cast<char *>(scratch) + TWIDDLE_BYTES);
+    if (int rc = plan_windows(scratch, init, nblocks, blocksize, blk_start, nt, 1, S, win_first, st)) return rc;
+    const double2 *tw = static_cast<const double2 *>(scratch), *tw2 = tw + FFT_M;
     const double2 *cf = reinterpret_cast<const double2 *>(coef);
+    const int64_t nwin_ub = nt / S + nblocks + 1;
     if (pair) {
         int64_t ncl = sm_count() / 2;
         if (nwin_ub < ncl) ncl = nwin_ub;
-        return fft_kernel<512, true>((int)(2 * ncl), smem, st, cf, tw, nband, nblocks, blocksize, blk_start, win_first,
-                                     d, out, nt, tw2, gen...);
+        return fft_kernel<true>((int)(2 * ncl), st, cf, tw, nband, nblocks, blocksize, blk_start, win_first, d, out, nt,
+                                tw2, gen...);
     }
-    const int grid = capped_grid(nwin_ub, 1);
-    // threads per CTA (one CTA per SM): 512 by default -- the 16-point butterflies of the first / last pass
-    // need the 128 registers per thread that 512 threads leave (measured at L = 4096: 1.81 ms vs 2.12 ms
-    // with 1024 threads, which spill); CM2_FFT_THREADS=1024 selects the apply's other instantiation.  The
-    // simulation runs at 512 threads (at 256 it spills nothing but takes 1.15-1.5x as long, DESIGN.md section 4d).
-    if constexpr (!GEN) {
-        static const int threads = [] {
-            const char *e = getenv("CM2_FFT_THREADS");
-            return (e && atoi(e) == 1024) ? 1024 : 512;
-        }();
-        if (threads == 1024)
-            return fft_kernel<1024, false>(grid, smem, st, cf, tw, nband, nblocks, blocksize, blk_start, win_first, d,
-                                           out, nt, tw2);
-    }
-    return fft_kernel<512, false>(grid, smem, st, cf, tw, nband, nblocks, blocksize, blk_start, win_first, d, out, nt,
-                                  tw2, gen...);
+    return fft_kernel<false>(capped_grid(nwin_ub, 1), st, cf, tw, nband, nblocks, blocksize, blk_start, win_first, d,
+                             out, nt, tw2, gen...);
 }
 
 // coef: device, [nblocks][2][M] complex (C1, C2 stored at the bit-reversed position of their frequency, 1/M folded in);
@@ -817,12 +820,12 @@ extern "C" int cm2_noise_simulate(const double *coef, int nband, int64_t nblocks
                       as_stream(stream), NoiseWindow<false>{seed, block_ids, realization});
 }
 
-// scratch: twiddles (2 M double2), Hann window (NF doubles), win_first (nblocks + 1), one slot of M + 2 doubles per
-// (CTA, block) run: at most (CTAs of the current device) + nblocks
+// scratch: the twiddles, Hann window (NF doubles), win_first (nblocks + 1), one slot of M + 2 doubles per (CTA, block)
+// run: at most (CTAs of the current device) + nblocks
 extern "C" int64_t cm2_noise_psd_scratch_bytes(int64_t nblocks) {
     if (nblocks < 1) return 0;
-    return (int64_t)sizeof(double) * (4 * (int64_t)FFT_M + FFT_NF + 2 * cdiv(nblocks + 1, 2) +
-                                      ((int64_t)sm_count() + nblocks) * PSD_SLOT);
+    return TWIDDLE_BYTES + (int64_t)sizeof(double) * (FFT_NF + 2 * cdiv(nblocks + 1, 2) +
+                                                      ((int64_t)sm_count() + nblocks) * PSD_SLOT);
 }
 
 // The Welch launcher of cm2_noise_psd (no source: the samples are d) and cm2_noise_psd_residual (one Residual<POL>):
@@ -830,33 +833,25 @@ extern "C" int64_t cm2_noise_psd_scratch_bytes(int64_t nblocks) {
 template <class... Src>
 static int psd_launch(const double *d, const int32_t *pix, int64_t nblocks, int64_t blocksize, const int64_t *blk_start,
                       int64_t nt, double *psd, double *wsum, void *scratch, int init, cudaStream_t st, Src... src) {
-    CM2_REQUIRE(nt >= 0 && nblocks > 0, "bad sizes");
-    CM2_REQUIRE(blk_start != nullptr || blocksize > 0, "blocksize must be > 0");
-    CM2_REQUIRE(blk_start != nullptr || nblocks - 1 <= nt / blocksize, "equal blocks past nt: (nblocks-1)*blocksize > nt");
+    if (int rc = check_partition(nblocks, blocksize, blk_start, nt)) return rc;
     CM2_REQUIRE(d != nullptr && psd != nullptr && wsum != nullptr, "d, psd and wsum are required");
     CM2_REQUIRE(scratch != nullptr && aligned(scratch, 16), "scratch (cm2_noise_psd_scratch_bytes) must be 16-byte aligned");
     // cm2_noise_psd writes zero sums for an empty TOD; the residual entry point writes nothing
     if (sizeof...(Src) == 1 && nt == 0) return CM2_OK;
-    double2 *tw = reinterpret_cast<double2 *>(scratch);
-    double2 *tw2 = tw + FFT_M;
-    double *hann = reinterpret_cast<double *>(tw2 + FFT_M);
+    double *hann = reinterpret_cast<double *>(static_cast<char *>(scratch) + TWIDDLE_BYTES);
     int64_t *win_first = reinterpret_cast<int64_t *>(hann + FFT_NF);
     double *slots = reinterpret_cast<double *>(win_first) + 2 * cdiv(nblocks + 1, 2);
+    if (int rc = plan_windows(scratch, init, nblocks, blocksize, blk_start, nt, FFT_NF, FFT_M, win_first, st)) return rc;
     if (init) {
-        k_fft_twiddles<<<(FFT_M / 4 + 255) / 256, 256, 0, st>>>(tw);
-        k_fft_twiddles_pair<<<(FFT_M + 255) / 256, 256, 0, st>>>(tw2);
-        CM2_LAUNCHED();
         if (int rc = launch(k_hann, FFT_NF / 256, 256, 0, st, hann)) return rc;
     }
-    k_win_first<<<1, 1, 0, st>>>(nblocks, blocksize, blk_start, nt, FFT_NF, FFT_M, win_first);
-    CM2_LAUNCHED();
+    const double2 *tw = static_cast<const double2 *>(scratch), *tw2 = tw + FFT_M;
     // one CTA per SM (the transform's shared memory), never more CTAs than windows could exist
-    const size_t smem = sizeof(double2) * (FFT_M + FFT_M / 8) + sizeof(double) * (FFT_M + 1 + 2 * PSD_THREADS);
+    const size_t smem = FFT_SMEM + sizeof(double) * (FFT_M + 1 + 2 * PSD_THREADS);
     const int grid = capped_grid(nt / FFT_M + 1, 1);
     CM2_CUDA(cudaFuncSetAttribute(k_noise_psd<Src...>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (int rc = launch(k_noise_psd<Src...>, grid, PSD_THREADS, smem, st, (const double2 *)tw, (const double2 *)tw2,
-                        (const double *)hann, nblocks, blocksize, blk_start, (const int64_t *)win_first, d, pix, nt, slots,
-                        src...))
+    if (int rc = launch(k_noise_psd<Src...>, grid, PSD_THREADS, smem, st, tw, tw2, (const double *)hann, nblocks,
+                        blocksize, blk_start, (const int64_t *)win_first, d, pix, nt, slots, src...))
         return rc;
     const int64_t n = nblocks * PSD_SLOT;
     return launch(k_psd_sum, capped_grid(cdiv(n, 256), 8), 256, 0, st, (const int64_t *)win_first, nblocks, grid,

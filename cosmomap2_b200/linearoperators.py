@@ -168,21 +168,20 @@ class _Blocks(object):
 
 
 class ToeplitzLO(lp.LinearOperator):
-    """Symmetric banded Toeplitz block, zero boundaries -- interfaces/linearoperators.py:560-602."""
+    """Symmetric banded Toeplitz block, zero boundaries -- interfaces/linearoperators.py:560-602.  Applied as the one
+    block of a BlockLO(offdiag=True), built at first use."""
 
     def __init__(self, a, size):
         self.array = a
-        self._blocks = _Blocks([0, int(size)])
-        self._band_dev = None
+        self._size = int(size)
+        self._N = None
         super(ToeplitzLO, self).__init__(nargin=size, nargout=size, matvec=self.mult, symmetric=True,
                                          device=True)
 
     def mult(self, v):                                    # :582-595
-        if self._band_dev is None:
-            band = np.atleast_1d(np.asarray(self.array, dtype=np.float64))
-            self._band_dev = dv.to_dev_f64(band)
-            self._fft = _ToeplitzFFT(band, len(band)) if len(band) >= TOEPLITZ_FFT_MIN_BAND else None
-        return _toeplitz_apply(self._band_dev, self._band_dev.numel(), self._blocks, v, self._fft)
+        if self._N is None:
+            self._N = BlockLO(self._size, [self.array], offdiag=True)
+        return self._N._apply_all(v)
 
 
 TOEPLITZ_FFT_MIN_BAND = 48     # bands at least this wide go through the overlap-save FFT kernel (measured
@@ -244,11 +243,12 @@ def toeplitz_fft_tables(band_host, nband, M, pair=False):
 
 
 class _ToeplitzFFT(object):
-    """Host-built packed transfer functions + device scratch for cm2_noise_toeplitz_fft_apply."""
+    """Host-built packed transfer functions + device scratch for cm2_noise_toeplitz_fft_apply and cm2_noise_simulate
+    (``pair``: 2-CTA cluster windows); ``ok`` is False, and nothing is built, when the band is too wide for them."""
 
-    def __init__(self, band_host, nband):
+    def __init__(self, band_host, nband, pair):
         M = int(dv.call("cm2_toeplitz_fft_points"))
-        self.pair = 1 if nband >= TOEPLITZ_FFT_PAIR_MIN_BAND else 0
+        self.pair = 1 if pair else 0
         self.ok = 2 * (nband - 1) < (2 * M if self.pair else M)
         if not self.ok:
             return
@@ -414,7 +414,7 @@ class BlockLO(BlockDiagonalLinearOperator):
         """Device band and (for wide bands) the overlap-save FFT tables, built at first use."""
         if self._band_dev is None:
             self._band_dev = dv.to_dev_f64(self._band_host.reshape(-1))
-            self._fft = (_ToeplitzFFT(self._band_host, self._nband)
+            self._fft = (_ToeplitzFFT(self._band_host, self._nband, pair=self._nband >= TOEPLITZ_FFT_PAIR_MIN_BAND)
                          if self._nband >= TOEPLITZ_FFT_MIN_BAND else None)
         return self._fft
 
@@ -953,9 +953,7 @@ class _FusedToeplitzA(lp.LinearOperator):
     def _run(self, x):
         P, N = self.P, self.N
         y = dv.out_f64(P.ncols * P.pol)
-        if N._band_dev is None:
-            N._band_dev = dv.to_dev_f64(N._band_host.reshape(-1))
-            N._fft = None
+        N._toeplitz_state()
         nb, bs, startp = N._blk.args()
         dv.call("cm2_amatvec_toeplitz", dv.ptr(P._pix_dev), dv.ptr(P._cos_dev), dv.ptr(P._sin_dev), P.nrows, P.pol,
                 dv.ptr(N._band_dev), int(N._nband), nb, bs, startp, dv.ptr(x), dv.ptr(y), P.ncols, _stream())

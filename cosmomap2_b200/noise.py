@@ -29,7 +29,7 @@ import numpy as np
 import torch
 
 from . import _device as dv
-from .linearoperators import SparseLO, _block_starts, _Blocks, toeplitz_fft_tables
+from .linearoperators import SparseLO, _block_starts, _Blocks, _ToeplitzFFT
 
 
 def _points():
@@ -186,22 +186,16 @@ class NoiseSimulator(object):
         nb = len(bands)
         if nb == 0:
             raise ValueError("no noise blocks")
-        M = _points()
         L = max(len(a) for a in bands)
-        if 2 * (L - 1) >= 2 * M:
-            raise ValueError("bands of %d coefficients: at most %d can be simulated" % (L, M))
         band = np.zeros((nb, L))
         for i, a in enumerate(bands):
             band[i, :len(a)] = a
+        self._fft = _ToeplitzFFT(band, L, pair=L >= NOISE_SIM_PAIR_MIN_BAND)
+        if not self._fft.ok:
+            raise ValueError("bands of %d coefficients: at most %d can be simulated" % (L, _points()))
         self.nband, self.nblocks = L, nb
-        self.pair = 1 if L >= NOISE_SIM_PAIR_MIN_BAND else 0
         self._blk = _Blocks(_block_starts(blocksize, nb))
         self.nt = self._blk.nt
-        coef = toeplitz_fft_tables(band, L, M, pair=bool(self.pair))
-        self._coef = dv.to_dev_f64(coef.view(np.float64).reshape(-1))
-        self._scratch = torch.empty(int(dv.call("cm2_toeplitz_fft_scratch_bytes", nb)) // 8 + 2, dtype=torch.float64,
-                                    device=self._coef.device)
-        self._init = 1
 
     def __call__(self, seed, realization=0, block_ids=None, add_to=None):
         ids = None
@@ -213,20 +207,20 @@ class NoiseSimulator(object):
         seed, realization = int(seed), int(realization)
         if not 0 <= seed < 1 << 64 or not 0 <= realization < 1 << 32:
             raise ValueError("seed must be in [0, 2^64) and realization in [0, 2^32)")
+        fft = self._fft
         if add_to is None:
-            out = torch.empty(self.nt, dtype=torch.float64, device=self._coef.device)
+            out = torch.empty(self.nt, dtype=torch.float64, device=fft.coef.device)
         else:
             out = add_to
-            if not (isinstance(out, torch.Tensor) and out.is_cuda and out.device == self._coef.device
+            if not (isinstance(out, torch.Tensor) and out.is_cuda and out.device == fft.coef.device
                     and out.dtype == torch.float64 and out.is_contiguous()):
-                raise ValueError("add_to must be a contiguous float64 tensor on %s" % self._coef.device)
+                raise ValueError("add_to must be a contiguous float64 tensor on %s" % fft.coef.device)
             if out.numel() != self.nt:
                 raise ValueError("add_to has %d samples, the noise blocks %d" % (out.numel(), self.nt))
         nb, bs, startp = self._blk.args()
-        dv.call("cm2_noise_simulate", dv.ptr(self._coef), self.nband, nb, bs, startp, dv.ptr(ids), seed, realization,
-                dv.ptr(out), self.nt, int(add_to is not None), dv.ptr(self._scratch), self._init, self.pair,
-                dv.stream())
-        self._init = 0
+        dv.call("cm2_noise_simulate", dv.ptr(fft.coef), self.nband, nb, bs, startp, dv.ptr(ids), seed, realization,
+                dv.ptr(out), self.nt, int(add_to is not None), dv.ptr(fft.scratch), fft.init, fft.pair, dv.stream())
+        fft.init = 0
         return out
 
 

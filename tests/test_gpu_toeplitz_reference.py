@@ -3,8 +3,8 @@ instantiation (direct or FFT, one-CTA or 2-CTA-cluster windows, the NLAG of the 
 by the planner's band thresholds in linearoperators.py.
 
     cm2_noise_toeplitz_apply       k_toeplitz, the direct kernel: persistent CTAs over 1024-sample tiles
-    cm2_noise_toeplitz_fft_apply   k_toeplitz_fft<512>, <1024> (CM2_FFT_THREADS=1024) and <512, true>: persistent
-                                   CTAs (clusters) over overlap-save windows of 2M (4M) samples
+    cm2_noise_toeplitz_fft_apply   k_toeplitz_fft<512> and <512, true>: persistent CTAs (clusters) over overlap-save
+                                   windows of 2M (4M) samples
     cm2_amatvec_toeplitz           k_amatvec_toeplitz<POL, NLAG>: y = P^T T P x in one TOD pass
 
 All three walk their tiles or windows in trips over a persistent grid, so each runs here at >= 3 trips as well as at
@@ -24,10 +24,6 @@ that block's data and band (at most one window or tile per CTA there), and the s
 off 16-byte alignment.  Every output sits in a sentinel-guarded buffer: nothing may be written outside it, and every
 output sample must be written.
 """
-import os
-import subprocess
-import sys
-
 import numpy as np
 import pytest
 
@@ -332,7 +328,7 @@ def test_fft_cluster_windows(cm, L, layout):
 @pytest.mark.parametrize("layout", LAYOUTS)
 @pytest.mark.parametrize("L", [1, 2, 48, 200, 2047, 4096])
 def test_fft_one_cta_windows(cm, L, layout):
-    """k_toeplitz_fft<512> (or <1024> under CM2_FFT_THREADS=1024) at >= 3 windows per CTA."""
+    """k_toeplitz_fft<512> at >= 3 windows per CTA."""
     check_noise(L, 0, layout, seed=L + 1)
 
 
@@ -345,24 +341,10 @@ def test_direct_tiles(cm, L, layout):
 
 
 @gpu
-def test_fft_1024_threads(cm):
-    """The one-CTA window cases with CM2_FFT_THREADS=1024 (read once per process: a fresh interpreter)."""
-    env = dict(os.environ, CM2_FFT_THREADS="1024", PYTHONDONTWRITEBYTECODE="1")
-    here = os.path.dirname(os.path.abspath(__file__))
-    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", "-s",
-                        os.path.abspath(__file__), "-k", "test_fft_one_cta_windows or test_fft_threads_in_use"],
-                       cwd=os.path.dirname(here), env=env, capture_output=True, text=True)
-    print(r.stdout[-3000:])
-    assert r.returncode == 0, r.stdout[-6000:] + r.stderr[-3000:]
-    assert " passed" in r.stdout and "skipped" not in r.stdout.splitlines()[-1]
-
-
-@gpu
 def test_fft_threads_in_use(cm):
-    """The one-CTA FFT kernel that runs is the instantiation CM2_FFT_THREADS selects (512 unless it is 1024)."""
+    """The one-CTA FFT kernel that runs is k_toeplitz_fft<512, false>."""
     import torch
     from torch.profiler import ProfilerActivity, profile
-    threads = 1024 if os.environ.get("CM2_FFT_THREADS") == "1024" else 512
     rng = np.random.default_rng(5)
     lay = Layout("one", 40000, 1, 40000)
     kern = NoiseKernel(200, 0, make_bands(1, 200, rng))
@@ -372,8 +354,7 @@ def test_fft_threads_in_use(cm):
         checked(kern(*lay.args(), d.data_ptr(), y.ptr(), lay.nt), "FFT")
         torch.cuda.synchronize()
     names = {e.name for e in prof.events() if "k_toeplitz_fft" in e.name}
-    assert names and all("k_toeplitz_fft<%d, false>" % threads in n or "k_toeplitz_fftILi%dELb0E" % threads in n
-                         for n in names), names
+    assert names and all("k_toeplitz_fft<512, false>" in n or "k_toeplitz_fftILi512ELb0E" in n for n in names), names
 
 
 # ---- small cases and argument checks of the noise kernels ------------------------------------------------------------

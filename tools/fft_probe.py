@@ -18,7 +18,7 @@ def main():
     nt, ndet = 100000000, 64
     ns = nt // ndet
     d = dv.to_dev_f64(np.random.default_rng(2).standard_normal(nt))
-    out = {"threads": os.environ.get("CM2_FFT_THREADS", "1024")}
+    out = {}
     for L in [int(a) for a in sys.argv[1:]] or [256, 4096]:
         N = cm.BlockLO(ns, synthetic.toeplitz_bands(ndet, L), offdiag=True)
         t = timeit(lambda: N._apply(d), reps=5, warm=2)
