@@ -36,44 +36,6 @@ __global__ void __launch_bounds__(FB) k_runs_mark(const int32_t *__restrict__ pi
     }
 }
 
-// one thread per run start: walk the run, accumulate (n, sum cos, sum sin); per segment the first
-// run index and the number of runs
-__global__ void __launch_bounds__(FB) k_runs_fill(const int32_t *__restrict__ pix, const double *__restrict__ cs,
-                                                  const double *__restrict__ sn, int pol,
-                                                  const int64_t *__restrict__ seg_start, const int64_t *__restrict__ seg_end,
-                                                  int64_t nseg, const int32_t *__restrict__ runidx,
-                                                  int32_t *__restrict__ run_pix, double *__restrict__ run_mom,
-                                                  int64_t *__restrict__ seg_first, int32_t *__restrict__ seg_nruns) {
-    __shared__ int s_first, s_count;
-    for (int64_t k = blockIdx.x; k < nseg; k += gridDim.x) {
-        const int64_t a = seg_start[k], b = seg_end[k];
-        if (threadIdx.x == 0) { s_first = 0x7fffffff; s_count = 0; }
-        __syncthreads();
-        for (int64_t t = a + threadIdx.x; t < b; t += FB) {
-            const int32_t r = runidx[t];
-            if (r < 0) continue;
-            const int32_t p = pix[t];
-            double n = 0.0, c = 0.0, s = 0.0;
-            for (int64_t u = t; u < b && pix[u] == p; ++u) {
-                n += 1.0;
-                if (pol > 1) { c += cs[u]; s += sn[u]; }
-            }
-            run_pix[r] = p;
-            run_mom[3 * (int64_t)r] = n;
-            run_mom[3 * (int64_t)r + 1] = c;
-            run_mom[3 * (int64_t)r + 2] = s;
-            atomicMin(&s_first, r);
-            atomicAdd(&s_count, 1);
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            seg_first[k] = s_count > 0 ? s_first : 0;
-            seg_nruns[k] = s_count;
-        }
-        __syncthreads();
-    }
-}
-
 template <int POL>
 __global__ void __launch_bounds__(FB) k_seg_mean(const int32_t *__restrict__ run_pix, const double *__restrict__ run_mom,
                                                  const int64_t *__restrict__ seg_first, const int32_t *__restrict__ seg_nruns,
@@ -168,7 +130,9 @@ __global__ void __launch_bounds__(FB) k_poly_gram(const int32_t *__restrict__ pi
     }
 }
 
-// one thread per run start (runidx >= 0): Legendre-weighted sums of the run
+// one thread per run start (runidx >= 0): walk the run and store its Legendre-weighted sums; per segment the first
+// run index and the number of runs.  NK = 1 (L_0 = 1) is the offset filter's table {n, sum cos, sum sin}: with
+// fma(1.0, c, m) rounding as m + c, and 0 for the cos and sin sums at pol 1.
 template <int NK>
 __global__ void __launch_bounds__(FB) k_poly_runs_fill(const int32_t *__restrict__ pix, const double *__restrict__ cs,
                                                        const double *__restrict__ sn, int pol,
@@ -286,8 +250,8 @@ extern "C" int cm2_filter_runs_fill(const int32_t *pix, const double *c, const d
                                     int32_t *seg_nruns, cm2_stream_t stream) {
     CM2_REQUIRE(nseg >= 0 && pol >= 1 && pol <= 3, "bad sizes");
     if (nseg == 0) return CM2_OK;
-    return launch(k_runs_fill, capped_grid(nseg, 8), FB, 0, as_stream(stream), pix, c, s, pol, seg_start, seg_end, nseg,
-                  runidx, run_pix, run_mom, seg_first, seg_nruns);
+    return launch(k_poly_runs_fill<1>, capped_grid(nseg, 8), FB, 0, as_stream(stream), pix, c, s, pol, seg_start, seg_end,
+                  nseg, runidx, run_pix, run_mom, seg_first, seg_nruns);
 }
 
 extern "C" int cm2_filter_seg_mean(const int32_t *run_pix, const double *run_mom, const int64_t *seg_first,

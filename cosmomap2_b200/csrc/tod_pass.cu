@@ -700,17 +700,48 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_toeplitz(const int32_t *__res
     run_merge<POL, POL>(y, rs);
 }
 
-// Fused y = P^T (P x - mu_seg) over the unflagged samples inside subscans: the offset-filtered
-// A-matvec in ONE pass over the TOD, given the subscan means mu (k_seg_mean, filter_runs.cu).
-// tile_seg[tile] = index of the first segment whose end lies beyond the tile's first sample.
+// The subscan table of the single-pass filter kernels below: the segments, a value per segment (the means of
+// the offset filter, or NK Legendre coefficients per segment) and the per-tile lookup.
 struct SegInfo {
     const int64_t *start, *end;   // nseg, sorted, non-overlapping
-    const double *mu;             // nseg
+    const double *val;            // nseg means, or nseg x NK coefficients
     const int32_t *tile_seg;      // ntiles: first segment ending beyond the tile's first sample
     const uint8_t *tile_flag;     // ntiles: 0 = tile outside every segment, 1 = inside one, 2 = mixed
     int64_t nseg;
 };
 
+// The segment lookup of a lane whose tile holds a boundary: k = the first segment whose end lies beyond the sample,
+// [a, b) its bounds (INT64_MAX past the table), mu its mean in a MEAN walk (0 past the table).  The step loop
+// `while (w.k < sg.nseg && t >= w.b) w.next<MEAN>(sg)` stays in each kernel, and k_amatvec_filter_mu keeps its own
+// lookup: either one through a helper changes that kernel's SASS (nvcc 12.9).
+struct SegWalk {
+    int64_t k, a, b;
+    double mu;
+
+    template <bool MEAN>
+    __device__ __forceinline__ void load(const SegInfo &sg) {
+        a = k < sg.nseg ? __ldg(sg.start + k) : INT64_MAX;
+        b = k < sg.nseg ? __ldg(sg.end + k) : INT64_MAX;
+        if constexpr (MEAN) mu = k < sg.nseg ? __ldg(sg.val + k) : 0.0;
+    }
+    // from k0 = tile_seg of t's tile to the segment of t; skip = false when k0 is known to be it
+    template <bool MEAN>
+    __device__ __forceinline__ void seek(const SegInfo &sg, int64_t k0, int64_t t, bool skip = true) {
+        k = k0;
+        if (skip) {
+            while (k < sg.nseg && __ldg(sg.end + k) <= t) ++k;
+        }
+        load<MEAN>(sg);
+    }
+    template <bool MEAN>
+    __device__ __forceinline__ void next(const SegInfo &sg) {
+        ++k;
+        load<MEAN>(sg);
+    }
+};
+
+// Fused y = P^T (P x - mu_seg) over the unflagged samples inside subscans: the offset-filtered
+// A-matvec in ONE pass over the TOD, given the subscan means mu = sg.val (k_seg_mean, filter_runs.cu).
 template <int POL>
 __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_mu(const int32_t *__restrict__ pix, const double *__restrict__ cs,
                                                              const double *__restrict__ sn, int64_t nt, SegInfo sg, TileOrder ord,
@@ -736,7 +767,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_mu(const int32_t *__re
         flag = __ldg(sg.tile_flag + tile);
         k0 = __ldg(sg.tile_seg + tile);
         if (tile2 >= 0) { flag2 = __ldg(sg.tile_flag + tile2); k02 = __ldg(sg.tile_seg + tile2); }
-        m0 = flag == 1 ? __ldg(sg.mu + k0) : 0.0;
+        m0 = flag == 1 ? __ldg(sg.val + k0) : 0.0;
     }
     while (tile >= 0) {
         const int64_t t0 = tile * TILE + (int64_t)lane * K;
@@ -751,7 +782,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_mu(const int32_t *__re
             int64_t k = k0;
             while (k < sg.nseg && __ldg(sg.end + k) <= t0) ++k;
             int64_t a = k < sg.nseg ? __ldg(sg.start + k) : INT64_MAX, b = k < sg.nseg ? __ldg(sg.end + k) : INT64_MAX;
-            double m = k < sg.nseg ? __ldg(sg.mu + k) : 0.0;
+            double m = k < sg.nseg ? __ldg(sg.val + k) : 0.0;
             if (t0 >= a && t0 + K <= b) {      // this lane's chunk is still inside one subscan
 #pragma unroll
                 for (int j = 0; j < K; ++j) mu[j] = m;
@@ -766,7 +797,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_mu(const int32_t *__re
                         ++k;
                         a = k < sg.nseg ? __ldg(sg.start + k) : INT64_MAX;
                         b = k < sg.nseg ? __ldg(sg.end + k) : INT64_MAX;
-                        m = k < sg.nseg ? __ldg(sg.mu + k) : 0.0;
+                        m = k < sg.nseg ? __ldg(sg.val + k) : 0.0;
                     }
                     if (t < a || k >= sg.nseg) p[j] = -1;
                     mu[j] = m;
@@ -786,7 +817,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_mu(const int32_t *__re
         if (tile2 >= 0) {     // warp-uniform: the next tile's TOD loads and mean, the lookup of the tile after it
             const int64_t t1 = tile2 * TILE + (int64_t)lane * K;
             load_tod<POL>(pix, cs, sn, t1, nt, p, c, s);
-            m0 = flag2 == 1 ? __ldg(sg.mu + k02) : 0.0;
+            m0 = flag2 == 1 ? __ldg(sg.val + k02) : 0.0;
             v3 = ord.next(v2 + nwarps, nwarps, ntiles, tile3);
             if (tile3 >= 0) { flag3 = __ldg(sg.tile_flag + tile3); k03 = __ldg(sg.tile_seg + tile3); }
         }
@@ -798,15 +829,7 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_mu(const int32_t *__re
 
 // Fused y = P^T (P x - sum_k c_k L_k(x_t)) over the unflagged samples inside subscans: the Legendre-
 // filtered A-matvec in ONE pass over the TOD, given the per-subscan coefficients (k_poly_seg_coef,
-// filter_runs.cu).  Same tile / subscan lookup as k_amatvec_filter_mu; x_t = -1 + 2 (t - a)/(len - 1).
-struct SegPoly {
-    const int64_t *start, *end;   // nseg, sorted, non-overlapping (the subscans this path handles)
-    const double *coef;           // nseg x NK
-    const int32_t *tile_seg;
-    const uint8_t *tile_flag;
-    int64_t nseg;
-};
-
+// filter_runs.cu) in sg.val.  Same tile / subscan lookup as k_amatvec_filter_mu; x_t = -1 + 2 (t - a)/(len - 1).
 template <int NK>
 __device__ __forceinline__ double poly_eval(const double (&cf)[NK], double xt) {
     double L[NK];
@@ -819,7 +842,7 @@ __device__ __forceinline__ double poly_eval(const double (&cf)[NK], double xt) {
 
 template <int POL, int NK>
 __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_poly_mu(const int32_t *__restrict__ pix, const double *__restrict__ cs,
-                                                                  const double *__restrict__ sn, int64_t nt, SegPoly sg, TileOrder ord,
+                                                                  const double *__restrict__ sn, int64_t nt, SegInfo sg, TileOrder ord,
                                                                   const double *__restrict__ x, double *__restrict__ y) {
     const int lane = threadIdx.x & 31;
     const int64_t nwarps = (int64_t)gridDim.x * (BLOCK / 32);
@@ -841,38 +864,31 @@ __global__ void __launch_bounds__(BLOCK) k_amatvec_filter_poly_mu(const int32_t 
 #pragma unroll
             for (int j = 0; j < K; ++j) { pv[j] = 0.0; p[j] = -1; }
         } else {
-            int64_t k = k0;
-            if (flag != 1) {
-                while (k < sg.nseg && __ldg(sg.end + k) <= t0) ++k;
-            }
-            int64_t a = k < sg.nseg ? __ldg(sg.start + k) : INT64_MAX, b = k < sg.nseg ? __ldg(sg.end + k) : INT64_MAX;
-            if (flag == 1 || (t0 >= a && t0 + K <= b)) {   // the lane's chunk lies inside one subscan
+            SegWalk w;                                     // the coefficients are loaded once the sample is inside
+            w.seek<false>(sg, k0, t0, flag != 1);
+            if (flag == 1 || (t0 >= w.a && t0 + K <= w.b)) {   // the lane's chunk lies inside one subscan
                 double cf[NK];
 #pragma unroll
-                for (int i = 0; i < NK; ++i) cf[i] = __ldg(sg.coef + k * NK + i);
-                const double step = b - a > 1 ? 2.0 / (double)(b - a - 1) : 0.0;
-                const double x0 = fma((double)(t0 - a), step, -1.0);
+                for (int i = 0; i < NK; ++i) cf[i] = __ldg(sg.val + w.k * NK + i);
+                const double step = w.b - w.a > 1 ? 2.0 / (double)(w.b - w.a - 1) : 0.0;
+                const double x0 = fma((double)(t0 - w.a), step, -1.0);
 #pragma unroll
                 for (int j = 0; j < K; ++j) pv[j] = poly_eval<NK>(cf, fma((double)j, step, x0));
-            } else if (t0 + K <= a) {                      // ... or entirely in a gap
+            } else if (t0 + K <= w.a) {                    // ... or entirely in a gap
 #pragma unroll
                 for (int j = 0; j < K; ++j) { pv[j] = 0.0; p[j] = -1; }
             } else {                                       // a subscan boundary inside the lane's 8 samples
 #pragma unroll
                 for (int j = 0; j < K; ++j) {
                     const int64_t t = t0 + j;
-                    while (k < sg.nseg && t >= b) {
-                        ++k;
-                        a = k < sg.nseg ? __ldg(sg.start + k) : INT64_MAX;
-                        b = k < sg.nseg ? __ldg(sg.end + k) : INT64_MAX;
-                    }
+                    while (w.k < sg.nseg && t >= w.b) w.next<false>(sg);
                     pv[j] = 0.0;
-                    if (k >= sg.nseg || t < a) { p[j] = -1; continue; }
+                    if (w.k >= sg.nseg || t < w.a) { p[j] = -1; continue; }
                     double cf[NK];
 #pragma unroll
-                    for (int i = 0; i < NK; ++i) cf[i] = __ldg(sg.coef + k * NK + i);
-                    const double step = b - a > 1 ? 2.0 / (double)(b - a - 1) : 0.0;
-                    pv[j] = poly_eval<NK>(cf, fma((double)(t - a), step, -1.0));
+                    for (int i = 0; i < NK; ++i) cf[i] = __ldg(sg.val + w.k * NK + i);
+                    const double step = w.b - w.a > 1 ? 2.0 / (double)(w.b - w.a - 1) : 0.0;
+                    pv[j] = poly_eval<NK>(cf, fma((double)(t - w.a), step, -1.0));
                 }
             }
         }
@@ -903,11 +919,11 @@ __global__ void __launch_bounds__(BLOCK) k_pointing_filter_mu(const int32_t *__r
     int flag = __ldg(sg.tile_flag + tile), k0 = __ldg(sg.tile_seg + tile);
     int flag2 = 0, k02 = 0;
     if (tile + nwarps < ntiles) { flag2 = __ldg(sg.tile_flag + tile + nwarps); k02 = __ldg(sg.tile_seg + tile + nwarps); }
-    double m0 = flag == 1 ? __ldg(sg.mu + k0) : 0.0;
+    double m0 = flag == 1 ? __ldg(sg.val + k0) : 0.0;
     for (; tile < ntiles; tile += nwarps) {
         const int64_t t0 = tile * TILE + (int64_t)lane * K;
         // next trip's mean and the lookup of the trip after it, before this tile's loads are waited for
-        const double m0n = (tile + nwarps < ntiles && flag2 == 1) ? __ldg(sg.mu + k02) : 0.0;
+        const double m0n = (tile + nwarps < ntiles && flag2 == 1) ? __ldg(sg.val + k02) : 0.0;
         int flag3 = 0, k03 = 0;
         if (tile + 2 * nwarps < ntiles) { flag3 = __ldg(sg.tile_flag + tile + 2 * nwarps); k03 = __ldg(sg.tile_seg + tile + 2 * nwarps); }
         if (t0 < nt) {
@@ -922,21 +938,14 @@ __global__ void __launch_bounds__(BLOCK) k_pointing_filter_mu(const int32_t *__r
 #pragma unroll
                 for (int j = 0; j < K; ++j) { mu[j] = 0.0; in[j] = false; }
             } else {
-                int64_t k = k0;
-                while (k < sg.nseg && __ldg(sg.end + k) <= t0) ++k;
-                int64_t a = k < sg.nseg ? __ldg(sg.start + k) : INT64_MAX, b = k < sg.nseg ? __ldg(sg.end + k) : INT64_MAX;
-                double m = k < sg.nseg ? __ldg(sg.mu + k) : 0.0;
+                SegWalk w;
+                w.seek<true>(sg, k0, t0);
 #pragma unroll
                 for (int j = 0; j < K; ++j) {
                     const int64_t t = t0 + j;
-                    while (k < sg.nseg && t >= b) {
-                        ++k;
-                        a = k < sg.nseg ? __ldg(sg.start + k) : INT64_MAX;
-                        b = k < sg.nseg ? __ldg(sg.end + k) : INT64_MAX;
-                        m = k < sg.nseg ? __ldg(sg.mu + k) : 0.0;
-                    }
-                    in[j] = k < sg.nseg && t >= a;
-                    mu[j] = m;
+                    while (w.k < sg.nseg && t >= w.b) w.next<true>(sg);
+                    in[j] = w.k < sg.nseg && t >= w.a;
+                    mu[j] = w.mu;
                 }
             }
 #pragma unroll
@@ -1533,7 +1542,7 @@ extern "C" int cm2_amatvec_filter_poly_mu(const int32_t *pix, const double *c, c
     cudaStream_t st = as_stream(stream);
     if (!accumulate) CM2_CUDA(zero_fill(y, npix, pol, st));
     if (nt == 0 || npix == 0 || nseg == 0) return CM2_OK;
-    SegPoly sg{seg_start, seg_end, seg_coef, tile_seg, tile_flag, nseg};
+    SegInfo sg{seg_start, seg_end, seg_coef, tile_seg, tile_flag, nseg};
     const int nk = poly_order + 1;
     const TileOrder ord = make_order(nt, nstreams);
     return with_pol(pol, [&](auto P) {

@@ -714,9 +714,11 @@ def _tile_tables(seg_start, seg_end, nseg, nt):
     return tile_seg.to(torch.int32), tile_flag
 
 
-def _build_run_table(P, seg_start, seg_end, nseg, need_runs):
+def _build_run_table(P, seg_start, seg_end, nseg, need_runs, order=0):
     """Run-compressed table of u_k = P^T 1_k over the unflagged samples of each of the ``nseg`` sorted,
     non-overlapping segments [seg_start[k], seg_end[k]) (device int64), built on the device (csrc/filter_runs.cu).
+    ``order`` 0: run_mom[nruns][3] = {n, sum cos, sum sin}; 1..4: the Legendre table of the subscans,
+    run_mom[nruns][3 (order + 1)] = the sums of L_l, L_l cos, L_l sin, l <= order.
     ``need_runs``: False when the pointing has fewer than 2 samples per run, where the table is no smaller than
     the TOD.  Returns dict(run_pix, run_mom, seg_first, seg_nruns, nruns), or False when it has no run."""
     nt, st = P.nrows, _stream()
@@ -734,12 +736,13 @@ def _build_run_table(P, seg_start, seg_end, nseg, need_runs):
     if nruns == 0 or (need_runs and 2 * nruns > nt):
         return False
     run_pix = torch.empty(nruns, dtype=torch.int32, device=dev)
-    run_mom = torch.empty(3 * nruns, dtype=torch.float64, device=dev)
+    run_mom = torch.empty(3 * (order + 1) * nruns, dtype=torch.float64, device=dev)
     seg_first = torch.empty(max(nseg, 1), dtype=torch.int64, device=dev)
     seg_nruns = torch.empty(max(nseg, 1), dtype=torch.int32, device=dev)
-    dv.call("cm2_filter_runs_fill", dv.ptr(pixm), dv.ptr(P._cos_dev), dv.ptr(P._sin_dev), P.pol,
-            dv.ptr(seg_start), dv.ptr(seg_end), nseg, dv.ptr(runidx), dv.ptr(run_pix), dv.ptr(run_mom),
-            dv.ptr(seg_first), dv.ptr(seg_nruns), st)
+    fill, order_arg = ("cm2_filter_poly_runs_fill", (order,)) if order else ("cm2_filter_runs_fill", ())
+    dv.call(fill, dv.ptr(pixm), dv.ptr(P._cos_dev), dv.ptr(P._sin_dev), P.pol, dv.ptr(seg_start), dv.ptr(seg_end),
+            nseg, *order_arg, dv.ptr(runidx), dv.ptr(run_pix), dv.ptr(run_mom), dv.ptr(seg_first),
+            dv.ptr(seg_nruns), st)
     return dict(run_pix=run_pix, run_mom=run_mom, seg_first=seg_first, seg_nruns=seg_nruns, nruns=nruns)
 
 
@@ -768,6 +771,12 @@ def _filter_runs(P, F):
     return cache[key]
 
 
+def _seg_means(P, F, rt, x):
+    """mu_k = u_k . x / n_k of every subscan from the run table rt of _filter_runs, into rt["mu"]."""
+    dv.call("cm2_filter_seg_mean", dv.ptr(rt["run_pix"]), dv.ptr(rt["run_mom"]), dv.ptr(rt["seg_first"]),
+            dv.ptr(rt["seg_nruns"]), F.nseg, P.pol, dv.ptr(x), dv.ptr(rt["mu"]), _stream())
+
+
 class _FusedFilterA(lp.LinearOperator):
     """P^T F P as one operator.  Default: the subscan means from the run-compressed table of
     u_k = P^T 1_k (csrc/filter_runs.cu), then ONE fused gather/scatter pass over the TOD; the table
@@ -787,8 +796,7 @@ class _FusedFilterA(lp.LinearOperator):
             self._runs = _filter_runs(P, F)
         rt = self._runs
         if rt:
-            dv.call("cm2_filter_seg_mean", dv.ptr(rt["run_pix"]), dv.ptr(rt["run_mom"]), dv.ptr(rt["seg_first"]),
-                    dv.ptr(rt["seg_nruns"]), F.nseg, P.pol, dv.ptr(x), dv.ptr(rt["mu"]), _stream())
+            _seg_means(P, F, rt, x)
             dv.call("cm2_amatvec_filter_mu", dv.ptr(P._pix_dev), dv.ptr(P._cos_dev), dv.ptr(P._sin_dev), P.nrows,
                     P.pol, dv.ptr(F._seg_start), dv.ptr(F._seg_end), dv.ptr(rt["mu"]), dv.ptr(rt["tile_seg"]),
                     dv.ptr(rt["tile_flag"]), F.nseg, dv.ptr(x), dv.ptr(y), P.ncols,
@@ -813,13 +821,12 @@ def _build_poly_runs(P, F):
     nk = order + 1
     if not (1 <= order <= 4 and F._sorted and F.nseg > 0):
         return False
-    nt, st = P.nrows, _stream()
     dev = P._pix_dev.device
     ss, se = F._seg_start_host, F._seg_end_host
     W_all = torch.empty(F.nseg * nk * nk, dtype=torch.float64, device=dev)
     info = torch.empty(2 * F.nseg, dtype=torch.float64, device=dev)
     dv.call("cm2_filter_poly_gram", dv.ptr(P._pix_dev), dv.ptr(F._seg_start), dv.ptr(F._seg_end), F.nseg, order,
-            dv.ptr(W_all), dv.ptr(info), st)
+            dv.ptr(W_all), dv.ptr(info), _stream())
     info_h = dv.to_host(info).reshape(-1, 2)
     cnt, piv = info_h[:, 0], info_h[:, 1]
     alive = cnt > order
@@ -833,29 +840,11 @@ def _build_poly_runs(P, F):
     seg_end = dv.to_dev(se[ie], torch.int64)
     W = W_all.view(F.nseg, nk * nk)[dv.to_dev(ie, torch.int64)].contiguous().view(-1)
     del W_all, info
-    flags = torch.empty(max(nt, 1), dtype=torch.int32, device=dev)
-    pixm = torch.empty(max(nt, 1), dtype=torch.int32, device=dev)
-    dv.call("cm2_filter_runs_mark", dv.ptr(P._pix_dev), dv.ptr(seg_start), dv.ptr(seg_end), ne, nt,
-            dv.ptr(flags), dv.ptr(pixm), st)
-    runidx = torch.empty(max(nt, 1), dtype=torch.int32, device=dev)
-    count = torch.zeros(1, dtype=torch.int64, device=dev)
-    scratch = torch.empty(int(dv.call("cm2_scan_scratch_bytes", nt)) // 8 + 1, dtype=torch.int64, device=dev)
-    dv.call("cm2_weights_old2new", dv.ptr(flags), nt, dv.ptr(runidx), dv.ptr(count), dv.ptr(scratch), st)
-    nruns = int(count.item())
-    del flags, scratch
-    if nruns == 0 or 2 * nruns > nt:
+    rt = _build_run_table(P, seg_start, seg_end, ne, need_runs=True, order=order)
+    if not rt:
         return False
-    run_pix = torch.empty(nruns, dtype=torch.int32, device=dev)
-    run_mom = torch.empty(3 * nk * nruns, dtype=torch.float64, device=dev)
-    seg_first = torch.empty(ne, dtype=torch.int64, device=dev)
-    seg_nruns = torch.empty(ne, dtype=torch.int32, device=dev)
-    dv.call("cm2_filter_poly_runs_fill", dv.ptr(pixm), dv.ptr(P._cos_dev), dv.ptr(P._sin_dev), P.pol,
-            dv.ptr(seg_start), dv.ptr(seg_end), ne, order, dv.ptr(runidx), dv.ptr(run_pix), dv.ptr(run_mom),
-            dv.ptr(seg_first), dv.ptr(seg_nruns), st)
-    del pixm, runidx
-    tile_seg, tile_flag = _tile_tables(seg_start, seg_end, ne, nt)
-    rt = dict(nseg=ne, seg_start=seg_start, seg_end=seg_end, W=W, run_pix=run_pix, run_mom=run_mom,
-              seg_first=seg_first, seg_nruns=seg_nruns, nruns=nruns, tile_seg=tile_seg, tile_flag=tile_flag,
+    tile_seg, tile_flag = _tile_tables(seg_start, seg_end, ne, P.nrows)
+    rt.update(nseg=ne, seg_start=seg_start, seg_end=seg_end, W=W, tile_seg=tile_seg, tile_flag=tile_flag,
               coef=torch.empty(ne * nk, dtype=torch.float64, device=dev), nhard=len(ih))
     if len(ih):
         rt["hard_start"] = dv.to_dev(ss[ih], torch.int64)
@@ -867,7 +856,7 @@ def _build_poly_runs(P, F):
 class _FusedPolyFilterA(lp.LinearOperator):
     """P^T F_K P for the Legendre filter (poly_order 1..4) as one kernel: one CTA per subscan, the
     subscan's P x kept in shared memory between the moment pass and the scatter pass.  With
-    ``FILTER_POLY_RUN_TABLE`` (experimental) the well-conditioned subscans go through the single-TOD-pass
+    ``FILTER_POLY_RUN_TABLE`` (the default) the well-conditioned subscans go through the single-TOD-pass
     scheme of the offset filter instead: coefficients from a Legendre run table, then one streaming pass."""
 
     def __init__(self, P, F):
@@ -928,8 +917,7 @@ class _FusedFilterP(lp.LinearOperator):
         if not rt:
             return F._apply(P._apply(x))
         d = dv.empty_f64(P.nrows)
-        dv.call("cm2_filter_seg_mean", dv.ptr(rt["run_pix"]), dv.ptr(rt["run_mom"]), dv.ptr(rt["seg_first"]),
-                dv.ptr(rt["seg_nruns"]), F.nseg, P.pol, dv.ptr(x), dv.ptr(rt["mu"]), _stream())
+        _seg_means(P, F, rt, x)
         dv.call("cm2_pointing_filter_mu", dv.ptr(P._pix_dev), dv.ptr(P._cos_dev), dv.ptr(P._sin_dev), P.nrows, P.pol,
                 dv.ptr(F._seg_start), dv.ptr(F._seg_end), dv.ptr(rt["mu"]), dv.ptr(rt["tile_seg"]),
                 dv.ptr(rt["tile_flag"]), F.nseg, dv.ptr(x), dv.ptr(d), _stream())

@@ -256,7 +256,7 @@ int cm2_amatvec_filter_mu(const int32_t *pix, const double *cos2phi, const doubl
  * runs_mark + scan as for the offset filter, poly_runs_fill (run_mom[nruns][3*nk] = sums of L_k, L_k cos,
  * L_k sin over each run).  Apply: poly_seg_coef (coef[nseg][nk] = W S from the run table), then
  * amatvec_filter_poly_mu: y (+)= P^T (P x - polynomial) in one TOD pass; tile tables as for
- * cm2_amatvec_filter_mu.  Experimental: not selected by default (DESIGN.md section 10). */
+ * cm2_amatvec_filter_mu.  Selected by default for the well-conditioned subscans (DESIGN.md section 10). */
 int cm2_filter_poly_gram(const int32_t *pix, const int64_t *seg_start, const int64_t *seg_end,
                          int64_t nseg, int poly_order, double *W, double *info, cm2_stream_t stream);
 int cm2_filter_poly_runs_fill(const int32_t *pix_masked, const double *cos2phi, const double *sin2phi,

@@ -546,6 +546,59 @@ def filter_tables(tod, pol, ss, se):
     return F, rt
 
 
+def run_table_ref(pix, c, s, ss, se, pol):
+    """The offset run table as the header defines it: a run starts at an unflagged sample of a segment that is the
+    segment's first sample or follows a different pixel, and lasts while the pixel repeats inside the segment; runs
+    are numbered in sample order.  The cos / sin sums add the run's samples one by one from 0.0 in sample order."""
+    nt = pix.size
+    seg = np.full(nt, -1)
+    for k, (a, b) in enumerate(zip(ss, se)):
+        seg[a:b] = k
+    t = np.arange(nt)
+    first = np.where(seg >= 0, ss[np.maximum(seg, 0)], -1)
+    starts = np.flatnonzero((seg >= 0) & (pix >= 0) & ((t == first) | (np.r_[-1, pix[:-1]] != pix)))
+    change = np.r_[np.flatnonzero(pix[1:] != pix[:-1]) + 1, nt]
+    ends = np.minimum(change[np.searchsorted(change, starts, side="right")], se[seg[starts]])
+    lens = ends - starts
+    csum, ssum = np.zeros(starts.size), np.zeros(starts.size)
+    if pol > 1:
+        for i in range(int(lens.max(initial=0))):
+            m = lens > i
+            csum[m] += c[starts[m] + i]
+            ssum[m] += s[starts[m] + i]
+    mom = np.stack([lens.astype(np.float64), csum, ssum], axis=1).ravel()
+    nruns = np.bincount(seg[starts], minlength=ss.size).astype(np.int32)
+    seg_first = np.where(nruns > 0, np.searchsorted(seg[starts], np.arange(ss.size)), 0)
+    return pix[starts], mom, seg_first, nruns
+
+
+@pytest.mark.parametrize("pol", [1, 2, 3])
+def test_filter_run_table_bits(cm, pol):
+    """The offset run table of _build_run_table (cm2_filter_runs_mark, the scan, cm2_filter_runs_fill) equals its
+    host reference bit for bit, on flagged raster pointing with a fully flagged subscan, adjacent subscans and
+    subscans that cut runs."""
+    import torch
+    from cosmomap2_b200 import linearoperators as lo
+    dv = _dv()
+    nt = (1 << 20) + 1237
+    rng = np.random.default_rng(10 + pol)
+    pix, npix = ZOO["raster"](nt, rng, sm_count())
+    pix = pix.copy()
+    pix[rng.random(nt) < 0.01] = -1
+    ss, se = subscan_layout(nt, rng)
+    pix[ss[ss.size // 2]:se[ss.size // 2]] = -1
+    tod = Tod(pix, npix, seed=pol)
+    P = SimpleNamespace(_pix_dev=tod.d_pix, _cos_dev=tod.d_c, _sin_dev=tod.d_s, nrows=nt, pol=pol)
+    rt = lo._build_run_table(P, dv.to_dev(ss, torch.int64), dv.to_dev(se, torch.int64), ss.size, need_runs=True)
+    assert rt, "the run table was not built"
+    run_pix, mom, seg_first, seg_nruns = run_table_ref(pix, tod.c, tod.s, ss, se, pol)
+    assert rt["nruns"] == run_pix.size
+    assert np.array_equal(rt["run_pix"].cpu().numpy(), run_pix)
+    assert np.array_equal(rt["run_mom"].cpu().numpy().view(np.int64), mom.view(np.int64)), "run moments"
+    assert np.array_equal(rt["seg_first"].cpu().numpy()[:ss.size], seg_first)
+    assert np.array_equal(rt["seg_nruns"].cpu().numpy()[:ss.size], seg_nruns)
+
+
 @pytest.mark.parametrize("pol", [1, 2, 3])
 def test_filter_mu_trips(cm, pol):
     """cm2_filter_seg_mean + cm2_amatvec_filter_mu (time order and interleaved) and cm2_pointing_filter_mu at >= 3
